@@ -1,10 +1,12 @@
 #!/usr/bin/env python3
 """bench.py — throughput of the panGNN message-passing hot path on B200 (see DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|...] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|...] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one whole-graph training step (fused fwd + BCE loss + bwd + Adam) over the
 ``generate_graphs()`` graph of a ``--simulate_dataset`` configuration of BASELINE.json.
+Inputs and initial weights are seeded, so the same arguments give the same inputs on every run;
+``--dump-outputs DIR`` writes what the last timed step computed (``dump_outputs``).
 Prints ONE JSON line.  ``value`` = scored similarity edges per second with graph + CSR resident in
 HBM; ``e2e`` = the same step through the public API from pinned HOST buffers (H2D of the batch,
 CSR build, gcn_norm, step, loss read-back inside the timed region).  ``--impl reference`` times the
@@ -128,6 +130,36 @@ class ClockSampler:
                 "samples": len(sm), "reasons": reasons, "source": "NVML, 200 ms period"}
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_LOGITS_FULL = 12 << 20          # logits of up to this many edges are written whole (48 MB of float32)
+DUMP_LOGITS_SAMPLE = 4 << 20         # above that, a fixed sample of this many edges
+
+
+def dump_outputs(out_dir, loss, logits, model):
+    """Write what one training step hands its caller as ``out_dir/<name>.npy``: ``loss``, the per-edge ``logits``,
+    and every parameter after the optimiser step (``param.<name>``) with the gradient it was updated from
+    (``grad.<name>``).  Two builds run with the same arguments can so be compared output for output.  Logits of
+    more than DUMP_LOGITS_FULL edges are cut to a seeded sample; ``logits_index`` then holds the sampled edges'
+    positions (float64, exact)."""
+    arrays = {"loss": loss.detach().float().cpu().numpy()}
+    z = logits.detach().float().cpu().numpy()
+    if z.size > DUMP_LOGITS_FULL:
+        idx = np.sort(np.random.default_rng(0).choice(z.size, DUMP_LOGITS_SAMPLE, replace=False))
+        arrays["logits"], arrays["logits_index"] = z[idx], idx.astype(np.float64)
+    else:
+        arrays["logits"] = z
+    for name, p in model.named_parameters():
+        arrays[f"param.{name}"] = p.detach().float().cpu().numpy()
+        if p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad.detach().float().cpu().numpy()
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
+
+
 def agg_bytes(E, N, F):
     """Algorithmic bytes of one aggregation launch (SURVEY.md §8d / DESIGN.md): per edge 4 (col) +
     4 (val) + 4F (gathered row), per node 4F (output row) + 8 (rowptr)."""
@@ -137,7 +169,9 @@ def agg_bytes(E, N, F):
 # ------------------------------------------------------------------------------------------------
 # CPU arm (oracle port of the reference model) — also the `cpu_baseline` leg of the GPU arm
 # ------------------------------------------------------------------------------------------------
-def cpu_arm(workload, steps, warmup, budget_s=45.0):
+def cpu_arm(workload, steps, warmup, budget_s=None):
+    """``steps`` timed whole-graph steps after ``warmup``; with ``budget_s`` (the cpu_baseline leg of the GPU arm) each
+    loop stops early once it has taken that many seconds, and ``steps`` of the result says how many were timed."""
     from types import SimpleNamespace
     from oracle import preprocess as op
     from oracle.model import AlternateGCN as OracleGCN, Flags, bce_with_logits
@@ -178,14 +212,14 @@ def cpu_arm(workload, steps, warmup, budget_s=45.0):
     t0 = time.perf_counter()
     for _ in range(warmup):
         step()
-        if time.perf_counter() - t0 > budget_s:
+        if budget_s is not None and time.perf_counter() - t0 > budget_s:
             break
     times = []
     for _ in range(steps):
         t1 = time.perf_counter()
         step()
         times.append(time.perf_counter() - t1)
-        if sum(times) > budget_s:
+        if budget_s is not None and sum(times) > budget_s:
             break
     dt = float(np.median(times))
     sample = (f"--simulate_dataset {n_s} {G} {f} {frags} {shuf} with the workload's flags: N={N}, "
@@ -268,12 +302,16 @@ def gpu_arm(a):
                     p.grad.copy_(flat[off:off + p.numel()].view_as(p))
                     off += p.numel()
 
+    step_out = {}
+
     def step(g):
         opt.zero_grad(set_to_none=False)
         loss, logits = model.forward_loss(g, pw)
         loss.backward()
         allreduce_grads()
         opt.step()
+        if a.dump_outputs:
+            step_out["loss"], step_out["logits"] = loss.detach(), logits
         return loss
 
     def barrier():
@@ -306,6 +344,8 @@ def gpu_arm(a):
     launches = ops.LAUNCHES["count"] - l0
     clk = clocks.stop() if rank == 0 else None
     value = E * world * a.steps / (ms * 1e-3)
+    if a.dump_outputs:                                      # here, before the legs below train the model further
+        dump_outputs(a.dump_outputs, step_out["loss"], step_out["logits"], model)
 
     if a.profile:
         a.no_cpu = True
@@ -428,7 +468,7 @@ def gpu_arm(a):
             setup.reset()
             for k, v in wl["flags"].items():
                 setattr(setup.args, k, v)
-    cpu, _ = cpu_arm(a.workload, steps=3, warmup=1) if (world == 1 and not a.no_cpu) else (None, None)
+    cpu, _ = cpu_arm(a.workload, steps=3, warmup=1, budget_s=45.0) if (world == 1 and not a.no_cpu) else (None, None)
     line = {
         "metric": "train_edges_per_s", "value": value, "unit": "edges/s", "n_gpus": world,
         "steps": a.steps, "warmup": a.warmup, "ms_per_step": ms / a.steps, "higher_is_better": True,
@@ -799,7 +839,7 @@ def reference_arm(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    cpu, E = cpu_arm(a.workload, steps=max(1, min(a.steps, 5)), warmup=max(1, min(a.warmup, 2)))
+    cpu, E = cpu_arm(a.workload, steps=a.steps, warmup=max(1, min(a.warmup, 2)))
     wl = WORKLOADS[a.workload]
     line = {"impl": "reference", "metric": "train_edges_per_s", "value": cpu["value"], "unit": "edges/s",
             "n_gpus": int(os.environ.get("WORLD_SIZE", "1")), "steps": cpu["steps"], "warmup": a.warmup,
@@ -838,7 +878,13 @@ if __name__ == "__main__":
                     help="N > 1: generate the main workload's hit table with the device Philox generator too")
     ap.add_argument("--profile", action="store_true",
                     help="ncu mode: warm-up + timed steps + aggregation loop only (no e2e / inference / CPU legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="single GPU: write the loss, logits, parameters and gradients of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: the single-GPU path only (--impl ours, one process)")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         reference_arm(a)
