@@ -413,6 +413,40 @@ int pangnn_simulate_edges(uint64_t seed, int32_t n, int32_t G, int32_t q_lo, int
                           int64_t num_fwd_rows, const int32_t *new_of_old, int32_t new_first_genome,
                           int32_t *q, int32_t *t, double *bits, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Exact ranking metrics: ROC AUC, average precision and the Youden threshold (the reference computes them with
+ * torchmetrics BinaryAUROC / BinaryAveragePrecision every epoch, pangnn.py:27-30,220-222,262-268,279-326, and with
+ * sklearn roc_auc_score / average_precision_score / roc_curve at test time, src/plot.py:103-107,131).
+ * A "run" is one distinct score with its positive and negative counts; runs are int64 rows (key, pos, neg) in
+ * DECREASING score order, key = the score's 32-bit order key (-0.0 and +0.0 share one).
+ *   pangnn_metric_runs:   runs of (scores [n] fp32, labels [n] of label_kind) — key pass, pangnn_sort_pairs_u64 on
+ *                         32 key bits, compaction — or, with runs_in != NULL, of n input runs in any order (equal
+ *                         keys are merged, counts summed; scores / labels ignored).  runs_out has room for n rows.
+ *                         info [6] (device, written): runs, P, N, 0, 0, flags (PANGNN_METRIC_*; the caller raises).
+ *                         hist (device, optional) [65536]: number of runs per top 16 key bits.  n < 2^32.
+ *   pangnn_metric_reduce: over runs with params [5] (device) = (runs, P, N, TP_0, FP_0): P, N the global class
+ *                         counts, (TP_0, FP_0) the counts ranked ahead of these runs (0 on one device; info
+ *                         serves as params).  max_runs sizes the launch.  out [8] (device):
+ *                         [0..1] sum_k neg_k (TP_{k-1} + TP_k) as unsigned 128-bit (lo, hi)  -> AUROC = / (2 P N)
+ *                         [2..3] sum_k pos_k floor(TP_k 2^s / (TP_k + FP_k)), 128-bit, s = out[7] = 127 - bitlen(P)
+ *                                -> AP = / (P 2^s)
+ *                         [4] max_k TP_k/P - FP_k/N (fp64 bits; -inf if P or N is 0), [5] key of the first run that
+ *                         reaches it (all ones if none), [6] runs.
+ * Integer accumulation throughout: results do not depend on input order, tiling or a split of the runs.
+ * ---------------------------------------------------------------------------------------------- */
+#define PANGNN_LABEL_F32 0
+#define PANGNN_LABEL_I32 1
+#define PANGNN_LABEL_I64 2
+#define PANGNN_LABEL_U8 3
+#define PANGNN_METRIC_NAN 1        /* a score is NaN */
+#define PANGNN_METRIC_BAD_LABEL 2  /* a label is not 0 or 1 */
+size_t pangnn_metric_runs_workspace_bytes(int64_t n);
+int pangnn_metric_runs(const float *scores, const void *labels, int label_kind, const int64_t *runs_in, int64_t n,
+                       int64_t *runs_out, int64_t *info, int64_t *hist, void *ws, size_t ws_bytes, void *stream);
+size_t pangnn_metric_reduce_workspace_bytes(int64_t max_runs);
+int pangnn_metric_reduce(const int64_t *runs, int64_t max_runs, const int64_t *params, int64_t *out, void *ws,
+                         size_t ws_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

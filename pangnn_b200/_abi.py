@@ -75,6 +75,10 @@ SIGNATURES = {
     "pangnn_simulate_neg_counts": (_int, [C.c_uint64, _i32, _i64, _i32, _i32, _c_p, _c_p]),
     "pangnn_simulate_edges": (_int, [C.c_uint64, _i32, _i32, _i32, _i32, _f64, _f64, _f64, _i32, _i32, _c_p, _c_p, _c_p,
                                      _i64, _i64, _c_p, _i32, _c_p, _c_p, _c_p, _c_p]),
+    "pangnn_metric_runs_workspace_bytes": (_sz, [_i64]),
+    "pangnn_metric_runs": (_int, [_c_p, _c_p, _int, _c_p, _i64, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
+    "pangnn_metric_reduce_workspace_bytes": (_sz, [_i64]),
+    "pangnn_metric_reduce": (_int, [_c_p, _i64, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
 ABI_VERSION = 3

@@ -751,6 +751,46 @@ class DistModel:
                                           m.mlp[4].weight, m.mlp[4].bias, pg.scored.gs, pg.skip, pg.y,
                                           float(pos_weight), 1.0 / max(pg.num_edges_total, 1), dpq_out, unit_grad)
 
+    @torch.no_grad()
+    def evaluate(self, pg, threshold, pos_weight=None):
+        """Test statistics of the whole partitioned graph, identical on every rank (``train.evaluate`` of the global
+        graph, ``src/predict.py:29-55``): global confusion matrix (one all-reduce of four counts), precision /
+        recall / F1 with ``eps=0``, the global mean BCE loss when ``pos_weight`` is given, and the exact global
+        ranking metrics of the probabilities (``metrics.ranking_metrics`` over the group).  Also returns this
+        rank's ``logits`` / ``prob`` / ``pred`` (edges ``pg.scored_edge_ids``)."""
+        from .metrics import ranking_metrics
+        from .train import prf
+        m = self.model
+        next_step()
+        pq_ext, w1c, _ = self._scorer_inputs(pg, self.embed(pg))
+        logits, prob, pred = ops.edge_score_predict(pq_ext, w1c, m.mlp[0].bias, m.mlp[2].weight, m.mlp[2].bias,
+                                                    m.mlp[4].weight, m.mlp[4].bias, pg.scored.gs, pg.skip, threshold)
+        y = pg.y
+        p, yl = pred.long(), y.long()
+        tp = (p * yl).sum()
+        fp = (p * (1 - yl)).sum()
+        fn = ((1 - p) * yl).sum()
+        cnt = torch.stack((torch.full_like(tp, y.numel()) - tp - fp - fn, fp, fn, tp))
+        loss_sum = None
+        if pos_weight is not None:
+            loss_sum = torch.nn.functional.binary_cross_entropy_with_logits(
+                logits, y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device), reduction="sum")
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
+        if world > 1:
+            dist.all_reduce(cnt, group=self.group)
+            if loss_sum is not None:
+                loss_sum = loss_sum.double()
+                dist.all_reduce(loss_sum, group=self.group)
+        tn, fp, fn, tp = (int(v) for v in cnt.tolist())
+        pr, rc, f1 = prf(tn, fp, fn, tp, eps=0.0)
+        rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=pr, recall=rc, f1=f1, logits=logits, prob=prob, pred=pred)
+        if loss_sum is not None:
+            rec["loss"] = float(loss_sum) / max(pg.num_edges_total, 1)
+        rk = ranking_metrics(prob, y, self.group)
+        rec.update(auroc=rk["auroc"], average_precision=rk["average_precision"],
+                   youden_threshold=rk["youden_threshold"], num_runs=rk["num_runs"])
+        return rec
+
     def _categorical_table(self):
         return self.model.embedding.weight if getattr(self.model, "_categorical", False) else None
 

@@ -1168,6 +1168,58 @@ def segment_max_labels(q, t, score, genome_of):
     return label
 
 
+_LABEL_KINDS = {torch.float32: 0, torch.int32: 1, torch.int64: 2, torch.uint8: 3, torch.bool: 3}
+METRIC_NAN, METRIC_BAD_LABEL = 1, 2
+METRIC_HIST_BINS = 65536
+
+
+def metric_runs(scores=None, labels=None, runs=None, info=None, hist=None):
+    """Distinct-score runs for the ranking metrics (``pangnn_metric_runs``): of (fp32 ``scores``, {0,1} ``labels``),
+    or of input ``runs`` [m, 3] (merged, counts of equal keys summed).  -> int64 runs [n, 3] (key, pos, neg) in
+    decreasing score order, of which the first ``info[0]`` rows are valid.  ``info`` int64 [6] (device, written):
+    runs, P, N, 0, 0, flags; ``hist`` int64 [65536] (device, optional, written): runs per top 16 key bits."""
+    lib = _abi.load()
+    if runs is not None:
+        _need_cuda(runs, info, hist)
+        runs = runs.contiguous()
+        n, dev, kind = runs.size(0), runs.device, 0
+    else:
+        _need_cuda(scores, labels, info, hist)
+        if scores.dtype != torch.float32:
+            raise _abi.PangnnError(f"metric_runs: scores must be float32, not {scores.dtype}")
+        if labels.dtype not in _LABEL_KINDS:
+            raise _abi.PangnnError(f"metric_runs: unsupported label dtype {labels.dtype}")
+        scores, labels = scores.reshape(-1).contiguous(), labels.reshape(-1).contiguous()
+        if labels.numel() != scores.numel():
+            raise _abi.PangnnError("metric_runs: scores and labels differ in length")
+        n, dev, kind = scores.numel(), scores.device, _LABEL_KINDS[labels.dtype]
+    if n >= 1 << 32:
+        raise _abi.PangnnError(f"metric_runs: {n} scores on one device; the sort takes fewer than 2^32")
+    out = torch.empty(n, 3, dtype=torch.int64, device=dev)
+    ws = _ws(lib.pangnn_metric_runs_workspace_bytes(n), dev)
+    _abi.check(lib.pangnn_metric_runs(_p(scores), _p(labels), kind, _p(runs), n, _p(out), _p(info), _p(hist),
+                                      _p(ws), ws.numel(), _stream()), "metric_runs")
+    LAUNCHES["count"] += 4 + 3 * 4 if n else 0
+    return out
+
+
+def metric_reduce(runs, params, out=None):
+    """``pangnn_metric_reduce`` over the first ``params[0]`` rows of ``runs`` (device int64 params: runs, P, N, TP_0,
+    FP_0) -> int64 [8] (device): AUROC numerator (lo, hi), AP numerator (lo, hi), best Youden j (fp64 bits), its
+    run's key, runs, AP fixed-point shift."""
+    lib = _abi.load()
+    _need_cuda(runs, params, out)
+    runs = runs.contiguous()
+    if out is None:
+        out = torch.empty(8, dtype=torch.int64, device=runs.device)
+    R = runs.size(0)
+    ws = _ws(lib.pangnn_metric_reduce_workspace_bytes(R), runs.device)
+    _abi.check(lib.pangnn_metric_reduce(_p(runs), R, _p(params), _p(out), _p(ws), ws.numel(), _stream()),
+               "metric_reduce")
+    LAUNCHES["count"] += 4 if R else 1
+    return out
+
+
 def rows_gather_copy(src, idx, dst):
     """dst[k] = src[idx[k]] (idx int32 or None); ``dst`` may be a PEER tensor (symmetric memory)."""
     lib = _abi.load()

@@ -14,6 +14,7 @@ import torch
 
 from . import postprocessing as post
 from . import setup
+from .metrics import ranking_metrics
 from .data import DeviceLoader
 from .dataset import UnionGraphDataset
 from .gnn import AlternateGCN
@@ -61,7 +62,8 @@ def youden_threshold(prob, labels):
 
 
 def evaluate(model, graphs, threshold, pos_weight=None):
-    """Whole-batch inference as ``src/predict.py:29-55``: logits, sigmoid, threshold, confusion."""
+    """Whole-batch inference as ``src/predict.py:29-55``: logits, sigmoid, threshold, confusion; plus the ROC AUC, AP
+    and Youden threshold of the probabilities (``src/plot.py:103-107,131``; exact, ``metrics.ranking_metrics``)."""
     model.eval()
     out = []
     for g in graphs:
@@ -69,11 +71,63 @@ def evaluate(model, graphs, threshold, pos_weight=None):
         tn, fp, fn, tp = confusion(pred, g.y)
         p, r, f1 = prf(tn, fp, fn, tp, eps=0.0)
         rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=p, recall=r, f1=f1, logits=logits, prob=prob, pred=pred)
+        rk = ranking_metrics(prob, g.y)
+        rec.update(auroc=rk["auroc"], average_precision=rk["average_precision"],
+                   youden_threshold=rk["youden_threshold"])
         if pos_weight is not None:
             rec["loss"] = float(torch.nn.functional.binary_cross_entropy_with_logits(
                 logits, g.y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device)))
         out.append(rec)
     return out
+
+
+def _fmt(v):
+    return "n/a" if v is None else f"{v:.4f}"
+
+
+def log_ranking(stats):
+    for s in stats:
+        log.info(f"test: auroc {_fmt(s['auroc'])} average precision {_fmt(s['average_precision'])} "
+                 f"youden threshold {_fmt(s['youden_threshold'])}")
+
+
+def _whole_graph(dataset, graph):
+    return getattr(graph, "node_id", None) is None or graph.node_id.numel() == dataset.num_genes
+
+
+def _logit_baseline(dataset, graph, stat):
+    """Max-logit-candidate baseline labels of the scored edges (``src/predict.py:84-88``), kept in the stat."""
+    from . import preprocessing as pp
+    if "logit_baseline" not in stat:
+        genome_d = torch.as_tensor(dataset.genome_of, device=graph.edge_index.device)
+        ei = graph.edge_index
+        stat["logit_baseline"] = pp.baseline_labels(ei[0].int(), ei[1].int(), stat["logits"], genome_d)
+    return stat["logit_baseline"]
+
+
+def add_baselines(dataset, graph, stat):
+    """Precision / recall / F1 of the max-candidate baselines next to the model's (``src/predict.py:77-89``):
+    ``stat["baselines"] = {name: (p, r, f1)}`` for the whole test graph (a sub-graph batch has no baseline)."""
+    if not _whole_graph(dataset, graph):
+        return None
+    cand = {"base_labels": dataset.base_labels, "base_labels_raw": dataset.base_labels_raw,
+            "logit_baseline": _logit_baseline(dataset, graph, stat)}
+    out = {}
+    for name, lab in cand.items():
+        if lab is None or len(lab) == 0:
+            continue
+        pred = torch.as_tensor(lab, device=graph.y.device)
+        out[name] = prf(*confusion(pred, graph.y), eps=0.0)
+    stat["baselines"] = out
+    log.info("baselines (precision / recall / f1): " +
+             "; ".join(f"{k} {p:.4f} / {r:.4f} / {f:.4f}" for k, (p, r, f) in out.items()))
+    return out
+
+
+def _epoch_ranking(probs, labels):
+    if not probs:
+        return dict(auroc=None, average_precision=None)
+    return ranking_metrics(torch.cat(probs), torch.cat(labels))
 
 
 def write_groups(dataset, graph, stat, out_dir):
@@ -93,13 +147,10 @@ def write_groups(dataset, graph, stat, out_dir):
 def write_edge_table(dataset, graph, stat, out_dir):
     """``q_score_vs_logit.csv`` for the whole test graph (``src/predict.py:84-88``: the max-logit-candidate
     baseline — a segmented arg-max over the logits — and the table itself, ``src/plot.py:473-504``)."""
-    from . import preprocessing as pp
-    if getattr(graph, "node_id", None) is not None and graph.node_id.numel() != dataset.num_genes:
+    if not _whole_graph(dataset, graph):
         return None                       # a sub-graph batch: the reference has no gene mapping for those either
-    genome_d = torch.as_tensor(dataset.genome_of, device=graph.edge_index.device)
     ei = graph.edge_index
-    logit_base = pp.baseline_labels(ei[0].int(), ei[1].int(), stat["logits"], genome_d)
-    stat["logit_baseline"] = logit_base
+    logit_base = _logit_baseline(dataset, graph, stat)
     path = post.write_q_score_vs_logit(ei, graph.edge_attr, stat["logits"], graph.y, dataset.gene_str_ids_lst,
                                        dataset.base_labels or None, dataset.base_labels_raw or None, logit_base,
                                        os.path.join(out_dir, "q_score_vs_logit.csv"))
@@ -135,7 +186,9 @@ def run(args, device=None):
         stats = evaluate(model, test, threshold, pos_weight)
         for s in stats:
             log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f} loss {s.get('loss', float('nan')):.4f}")
+        log_ranking(stats)
         if stats:
+            add_baselines(dataset, test[0], stats[0])
             write_groups(dataset, test[0], stats[0], args.output)
             write_edge_table(dataset, test[0], stats[0], args.output)                 # src/predict.py:84-88
         return dict(model=model, dataset=dataset, history=history, test=stats)
@@ -161,6 +214,7 @@ def run(args, device=None):
     for epoch in range(args.epochs):                                                  # pangnn.py:167-238
         model.train()
         train_loss, cm = 0.0, [0, 0, 0, 0]
+        ep_prob, ep_y = [], []                                 # the epoch's (prob, label) pairs, on the device
         batches = train_loader.iter_ids() if stepper is not None else train_loader
         for batch in batches:
             if stepper is not None:
@@ -174,16 +228,21 @@ def run(args, device=None):
                 labels = batch.y
             train_loss += loss.item()
             prob = torch.sigmoid(logits)
+            ep_prob.append(prob.detach())
+            ep_y.append(labels.clone() if stepper is not None else labels)   # the stepper's labels are static buffers
             pred = (prob >= threshold).int()
             cm = [a + b for a, b in zip(cm, confusion(pred, labels))]
             if args.dynamic_binary_threshold:                                         # pangnn.py:229-233
                 th = youden_threshold(prob, labels)
                 threshold = th if th is not None else threshold
         val_loss, cmv = 0.0, [0, 0, 0, 0]
+        val_prob, val_y = [], []
         model.eval()
         with torch.no_grad():                                                         # pangnn.py:241-275
             for batch in val_loader:
                 logits, prob, pred = model.predict(batch, threshold)
+                val_prob.append(prob)
+                val_y.append(batch.y)
                 val_loss += float(torch.nn.functional.binary_cross_entropy_with_logits(
                     logits, batch.y, pos_weight=torch.as_tensor(pos_weight, device=logits.device)))
                 cmv = [a + b for a, b in zip(cmv, confusion(pred, batch.y))]
@@ -191,9 +250,15 @@ def run(args, device=None):
         pv, rv, f1v = prf(*cmv)
         mean_val = val_loss / max(len(val_loader), 1)
         scheduler.step(mean_val)                                                      # pangnn.py:296
+        # epoch-level ranking metrics (torchmetrics' compute() over the whole epoch, pangnn.py:279-326)
+        rk_tr, rk_val = _epoch_ranking(ep_prob, ep_y), _epoch_ranking(val_prob, val_y)
         history.append(dict(epoch=epoch, train_loss=train_loss / max(len(train_loader), 1), val_loss=mean_val,
-                            f1_train=f1, f1_val=f1v, precision_val=pv, recall_val=rv))
+                            f1_train=f1, f1_val=f1v, precision_val=pv, recall_val=rv,
+                            auroc_train=rk_tr["auroc"], ap_train=rk_tr["average_precision"],
+                            auroc_val=rk_val["auroc"], ap_val=rk_val["average_precision"]))
         log.info(f"epoch {epoch}: train loss {history[-1]['train_loss']:.4f} f1 {f1:.4f} | val loss {mean_val:.4f} f1 {f1v:.4f}")
+        log.info(f"epoch {epoch}: train auroc {_fmt(rk_tr['auroc'])} ap {_fmt(rk_tr['average_precision'])} | "
+                 f"val auroc {_fmt(rk_val['auroc'])} ap {_fmt(rk_val['average_precision'])}")
 
     os.makedirs(args.output, exist_ok=True)
     path = os.path.join(args.output, os.path.basename(args.model_args))
@@ -202,7 +267,9 @@ def run(args, device=None):
     stats = evaluate(model, test, threshold, pos_weight)                              # pangnn.py:344-346
     for s in stats:
         log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f}")
+    log_ranking(stats)
     if stats:
+        add_baselines(dataset, test[0], stats[0])
         write_groups(dataset, test[0], stats[0], args.output)
         if args.simulate_dataset:                                                     # src/predict.py:84: not args.train or simulate
             write_edge_table(dataset, test[0], stats[0], args.output)
