@@ -115,10 +115,16 @@ __device__ __forceinline__ void emit_entry(int64_t i, int32_t qi, int32_t ti, bo
         // 1 - p = (S - e_i) / S: the subtraction in fp64 (S was accumulated in fp64 from the very e_i it removes,
         // so it is exact), the quotient of the two positive numbers and the logarithm in fp32 (1e-7 relative on
         // 1 - p = 4e-7 absolute on w); an fp64 division + log10 per entry was a fifth of the kernel's instructions
-        float om = 0.f;
-        if (members > 1) om = (float)(sum - e) / (float)sum;
+        // 1 - p is not representable in fp32 near 1 (ulp 6e-8 > eps = 1e-8), so that end is taken from p itself:
+        // -10 log10(1 - p) = -10 / ln(10) log1p(-p), which rounds to the same float as the fp64 formula
+        float om = 0.f, pf = 1.f;
+        if (members > 1) {
+            om = (float)(sum - e) / (float)sum;
+            pf = (float)e / (float)sum;
+        }
         if (om <= (float)eps) wi = w_hi;                       // np.clip(1-p, eps, 1-eps)
-        else if (om >= (float)(1.0 - eps)) wi = w_lo;
+        else if (pf <= (float)eps) wi = w_lo;
+        else if (pf < 0.5f) wi = fmaf(-4.342944819032518f, log1pf(-pf), (float)pseudo);
         else wi = fmaf(-10.f, log10f(om), (float)pseudo);
     }
     w[i] = wi;
