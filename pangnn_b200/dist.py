@@ -234,15 +234,6 @@ def _sym(plan, kind, site, F, device):
     return plan.p2p.buffer(f"{kind}:{site}:{_STEP['parity']}", plan.n_ext_max, F, device)
 
 
-def _alias(buf, rows):
-    """A fresh tensor over the first ``rows`` rows of a persistent buffer that is NOT a view of it as far
-    as autograd is concerned: the buffers are reused every step, and an in-place (mark_dirty) custom
-    function on a view would rebase the history of the shared base tensor, chaining the graphs of
-    unrelated exchange sites and steps together."""
-    return torch.empty(0, dtype=buf.dtype, device=buf.device).set_(
-        buf.untyped_storage(), buf.storage_offset(), (int(rows), buf.size(1)), (buf.size(1), 1))
-
-
 class HaloGather(torch.autograd.Function):
     """x_own [n_own, F] -> x_ext [n_own + n_halo, F]; backward = transposed exchange.  ``site`` names
     the exchange (one symmetric buffer pair per site in peer-memory mode)."""
@@ -256,7 +247,7 @@ class HaloGather(torch.autograd.Function):
             ext, hdl = _sym(plan, "fwd", site, x_own.size(1), x_own.device)
             ext[:plan.n_own].copy_(x_own)
             plan.p2p_push(ext, hdl)
-            return _alias(ext, plan.n_own + plan.n_halo)
+            return ops._alias(ext, (plan.n_own + plan.n_halo, ext.size(1)))
         return torch.cat((x_own, plan.gather(x_own)), dim=0)
 
     @staticmethod
@@ -265,7 +256,8 @@ class HaloGather(torch.autograd.Function):
         if plan.n_halo == 0 and plan.world == 1:
             return d_ext, None, None
         if plan.p2p is not None and d_ext.size(1) % 4 == 0:
-            return _alias(_p2p_backward(plan, ctx.site, d_ext), plan.n_own), None, None
+            buf = _p2p_backward(plan, ctx.site, d_ext)
+            return ops._alias(buf, (plan.n_own, buf.size(1))), None, None
         d_own = d_ext[:plan.n_own].clone()
         plan.scatter_add(d_ext[plan.n_own:], d_own)
         return d_own, None, None
@@ -279,7 +271,7 @@ def _p2p_backward(plan, site, d_ext):
     if d_ext.data_ptr() != buf.data_ptr():
         buf[:n].copy_(d_ext[:n])
     plan.p2p_pull_add(buf, hdl)
-    return _alias(buf, n)
+    return ops._alias(buf, (n, buf.size(1)))
 
 
 class HaloFill(torch.autograd.Function):
@@ -601,7 +593,7 @@ def _fwd_buf(plan, site, F, device):
     """(out_full for the producing GEMM, dx_out for the consumer's backward) of an exchange site."""
     if plan.p2p is None:
         return None, None
-    return (_alias(_sym(plan, "fwd", site, F, device)[0], plan.n_own + plan.n_halo),
+    return (ops._alias(_sym(plan, "fwd", site, F, device)[0], (plan.n_own + plan.n_halo, F)),
             _sym(plan, "bwd", site, F, device)[0])
 
 
@@ -719,37 +711,32 @@ class DistModel:
         return _layer(h, m.conv_out, pg.nb, False, ELU, "nb")
 
     def _scorer_inputs(self, pg, h):
-        m, D = self.model, ops.SCORER_D
+        """-> (endpoint rows pq_ext [n_ext, 2D], the scorer's weights (w1c, b1, w2, b2, w3, b3), dpq_out)."""
+        mlp, D = self.model.mlp, ops.SCORER_D
         if args.decoder != "mlp" or h.size(1) != D:
             raise NotImplementedError("the partitioned path scores edges with the fused mlp decoder at --node_dim 64")
-        w1 = m.mlp[0].weight
-        wcat = torch.cat((w1[:, :D], w1[:, D:2 * D]), dim=0)
+        wcat, w1c = ops.split_w1(mlp[0].weight, pg.skip is not None)
         plan = pg.scored.plan
         _, dpq_out = _fwd_buf(plan, "pq", 2 * D, h.device)
         pq_ext = _linear_with_halo(h, wcat, plan, "pq")
-        w1c = w1[:, 2 * D].contiguous() if pg.skip is not None else None
-        return pq_ext, w1c, dpq_out
+        return pq_ext, (w1c, mlp[0].bias, mlp[2].weight, mlp[2].bias, mlp[4].weight, mlp[4].bias), dpq_out
 
     @torch.no_grad()
     def forward(self, pg):
         """Inference: logits of the locally scored edges (``pg.scored_edge_ids`` in the global list)."""
-        m = self.model
         next_step()
-        pq_ext, w1c, _ = self._scorer_inputs(pg, self.embed(pg))
-        return ops.edge_score_pq_fwd(pq_ext, w1c, m.mlp[0].bias, m.mlp[2].weight, m.mlp[2].bias,
-                                     m.mlp[4].weight, m.mlp[4].bias, pg.scored.gs, pg.skip)
+        pq_ext, weights, _ = self._scorer_inputs(pg, self.embed(pg))
+        return ops.edge_score_pq_fwd(pq_ext, *weights, pg.scored.gs, pg.skip)
 
     __call__ = forward
 
     def forward_loss(self, pg, pos_weight, unit_grad=True):
         """-> (this rank's share of the global mean loss, logits of the locally scored edges).  ``unit_grad``: the
         loss is back-propagated as is (``loss.backward()``, checked on the device) — pass False to scale it first."""
-        m = self.model
         next_step()                                            # exchange buffers of the other parity (see _sym)
-        pq_ext, w1c, dpq_out = self._scorer_inputs(pg, self.embed(pg))
-        return ops.EdgeScoreBCEPQFn.apply(pq_ext, w1c, m.mlp[0].bias, m.mlp[2].weight, m.mlp[2].bias,
-                                          m.mlp[4].weight, m.mlp[4].bias, pg.scored.gs, pg.skip, pg.y,
-                                          float(pos_weight), 1.0 / max(pg.num_edges_total, 1), dpq_out, unit_grad)
+        pq_ext, weights, dpq_out = self._scorer_inputs(pg, self.embed(pg))
+        return ops.EdgeScoreBCEPQFn.apply(pq_ext, *weights, pg.scored.gs, pg.skip, pg.y, float(pos_weight),
+                                          1.0 / max(pg.num_edges_total, 1), dpq_out, unit_grad)
 
     @torch.no_grad()
     def evaluate(self, pg, threshold, pos_weight=None):
@@ -760,11 +747,9 @@ class DistModel:
         rank's ``logits`` / ``prob`` / ``pred`` (edges ``pg.scored_edge_ids``)."""
         from .metrics import ranking_metrics
         from .train import prf
-        m = self.model
         next_step()
-        pq_ext, w1c, _ = self._scorer_inputs(pg, self.embed(pg))
-        logits, prob, pred = ops.edge_score_predict(pq_ext, w1c, m.mlp[0].bias, m.mlp[2].weight, m.mlp[2].bias,
-                                                    m.mlp[4].weight, m.mlp[4].bias, pg.scored.gs, pg.skip, threshold)
+        pq_ext, weights, _ = self._scorer_inputs(pg, self.embed(pg))
+        logits, prob, pred = ops.edge_score_predict(pq_ext, *weights, pg.scored.gs, pg.skip, threshold)
         y = pg.y
         p, yl = pred.long(), y.long()
         tp = (p * yl).sum()

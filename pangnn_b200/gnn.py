@@ -100,7 +100,7 @@ class AlternateGCN(nn.Module):
         if (not self._categorical and graph.x.dim() == 2 and graph.x.size(1) == 1 and self.fuse_embedding
                 and OPERATOR_LAYER["kind"] == "function"
                 and self.conv_in.out_channels % 4 == 0 and self.conv_in.out_channels <= 256):
-            # scalar node features: Linear(1, D) + conv_in collapse into one rank-2 update (ops.EmbedConvFn)
+            # scalar node features: Linear(1, D) + conv_in collapse into one rank-2 update (ops.RankOneFn)
             ei = graph.union_edge_index if args.union_edge_weights else graph.edge_index
             emb, cin = self.embedding, self.conv_in
             if self.fuse_second_aggregation and not args.base_model and cin.out_channels in ops.RANK1_AGG_WIDTHS:
@@ -185,11 +185,9 @@ class AlternateGCN(nn.Module):
             prob = torch.sigmoid(logits)
             return logits, prob, (prob >= th).to(torch.int32)
         gs = ops.graph_struct(graph.edge_index, nodes.size(0))
-        m, D = self.mlp, ops.SCORER_D
+        m = self.mlp
         skip = self._skip(graph)
-        w1 = m[0].weight
-        wcat = torch.cat((w1[:, :D], w1[:, D:2 * D]), dim=0).contiguous()
-        w1c = w1[:, 2 * D].contiguous() if skip is not None else None
+        wcat, w1c = ops.split_w1(m[0].weight, skip is not None)
         pq = ops.node_linear(nodes, wcat)
         return ops.edge_score_predict(pq, w1c, m[0].bias, m[2].weight, m[2].bias, m[4].weight, m[4].bias, gs, skip, th)
 

@@ -6,7 +6,7 @@ our tcgen05 3xTF32 kernel (``node_linear``); only shapes outside {64,128}^2 reac
 No fallback: a tensor that is not on a CUDA device raises.
 """
 import ctypes as C
-from collections import OrderedDict
+from collections import OrderedDict, namedtuple
 
 import torch
 
@@ -15,7 +15,6 @@ from . import _abi
 ACT_NONE, ACT_ELU = 0, 1
 SCORER_D = 64
 NGRADS = 64 * 64 + 64 + 64 + 1 + 64 + 64
-_G_W2, _G_B2, _G_W3, _G_B3, _G_B1, _G_W1C = 0, 4096, 4160, 4224, 4225, 4289
 
 # kernel-launch accounting for bench.py ("gpu_launches")
 LAUNCHES = {"count": 0}
@@ -37,6 +36,15 @@ def _need_cuda(*ts):
 
 def _ws(nbytes, device):
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
+
+
+def _alias(buf, shape, stride=()):
+    """A fresh tensor of ``shape`` (row-major unless ``stride`` is given) over the memory of a persistent buffer,
+    from its first element, that is NOT a view of it as far as autograd is concerned: the buffers are reused every
+    step, and an in-place (mark_dirty) custom function on a view, or an output that is a view of an input, would
+    tie the history of the shared base tensor to unrelated sites and steps."""
+    return torch.empty(0, dtype=buf.dtype, device=buf.device).set_(buf.untyped_storage(), buf.storage_offset(),
+                                                                   tuple(map(int, shape)), tuple(stride))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -732,15 +740,93 @@ def gcn_layer(x, weight, bias, edge_index, edge_weight=None, act=ACT_NONE):
 
 
 # ------------------------------------------------------------------------------------------------
-# autograd: fused edge scorer
+# fused edge scorer: one host wrapper per C entry point, the layout of its gradients, the W1 split
 # ------------------------------------------------------------------------------------------------
-def _scorer_common(h, w1, skip):
+ScorerGrads = namedtuple("ScorerGrads", "dW2 db2 dw3 db3 db1 dw1c")
+# offsets of the small gradients in grads[NGRADS] (``pangnn_edge_score_bwd``); read them through scorer_grads
+_G_W2, _G_B2, _G_W3, _G_B3, _G_B1, _G_W1C = 0, 4096, 4160, 4224, 4225, 4289
+
+
+def scorer_grads(grads):
+    """Parameter-shaped views of the scorer's small gradients ``grads`` [NGRADS] (``pangnn_edge_score_bwd``):
+    dW2 [D, D], db2 [D], dw3 [1, D], db3 [1], db1 [D], dw1c [D]."""
     D = SCORER_D
-    if h.size(1) != D or w1.size(0) != D:
+    return ScorerGrads(grads[_G_W2:_G_W2 + D * D].view(D, D), grads[_G_B2:_G_B2 + D], grads[_G_W3:_G_W3 + D].view(1, D),
+                       grads[_G_B3:_G_B3 + 1], grads[_G_B1:_G_B1 + D], grads[_G_W1C:_G_W1C + D])
+
+
+def split_w1(w1, has_skip):
+    """First scorer layer ``W1`` [D, 2D (+1)] hoisted to the nodes: -> (``wcat = [W1[:, :D] ; W1[:, D:2D]]``
+    [2D, D], so that ``pq = h wcat^T``; the skip column ``w1c`` [D], or None).  Plain differentiable torch ops."""
+    D = SCORER_D
+    wcat = torch.cat((w1[:, :D], w1[:, D:2 * D]), dim=0)
+    return wcat, (w1[:, 2 * D].contiguous() if has_skip else None)
+
+
+def _scorer_operands(pq, w1c, b1, w2, b2, w3, b3, gs, skip):
+    """-> (the ten leading arguments of every scorer entry point, as tensors that the caller holds until the launch
+    is enqueued; the edge count).  ``gs``: the scored-edge structure, or its int32 endpoints ``(src, dst)``."""
+    _need_cuda(pq)
+    src, dst = gs if isinstance(gs, tuple) else gs.endpoints32
+    return (pq.contiguous(), src, dst, skip, w1c, b1, w2.contiguous(), b2, w3.contiguous(), b3), src.numel()
+
+
+def edge_score_pq_fwd(pq, w1c, b1, w2, b2, w3, b3, gs, skip):
+    """Inference form of the scorer on pre-transformed endpoint rows ``pq`` [n_ext, 2D] (layer 1 hoisted,
+    ``split_w1``) -> logits."""
+    lib = _abi.load()
+    args, E = _scorer_operands(pq, w1c, b1, w2, b2, w3, b3, gs, skip)
+    logits = torch.empty(E, dtype=torch.float32, device=pq.device)
+    _abi.check(lib.pangnn_edge_score_fwd(*map(_p, args), E, None, 1.0, _p(logits), None, None, 0, _stream()),
+               "edge_score_fwd")
+    LAUNCHES["count"] += 1
+    return logits
+
+
+def edge_score_predict(pq, w1c, b1, w2, b2, w3, b3, gs, skip, threshold=0.5):
+    """Inference with the prediction head fused in: -> (logits, prob = sigmoid(logits), pred = prob >= threshold)
+    (``pangnn.py:220-221``, ``src/predict.py:54-55``)."""
+    lib = _abi.load()
+    args, E = _scorer_operands(pq, w1c, b1, w2, b2, w3, b3, gs, skip)
+    dev = pq.device
+    logits = torch.empty(E, dtype=torch.float32, device=dev)
+    prob = torch.empty(E, dtype=torch.float32, device=dev)
+    pred = torch.empty(E, dtype=torch.int32, device=dev)
+    _abi.check(lib.pangnn_edge_score_predict(*map(_p, args), E, float(threshold), _p(logits), _p(prob), _p(pred),
+                                             _stream()), "edge_score_predict")
+    LAUNCHES["count"] += 1
+    return logits, prob, pred
+
+
+def edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, *, y=None, pos_weight=1.0, scale=1.0, dlogits=None,
+                     logits=None, loss_sum=None, da1=None, grads=None, ws=None):
+    """Training form -> (da1 [E, D], the per-edge gradient of layer 1's pre-activation; grads [NGRADS], see
+    ``scorer_grads``).  The upstream gradient is ``dlogits`` [E], or with labels ``y`` the fused
+    BCE-with-logits(``pos_weight``) times ``scale``, which also writes ``logits`` and adds the loss sum into
+    ``loss_sum`` (float64 [1], zeroed by the caller) when they are given.  ``da1`` (at least E rows), ``grads`` and
+    the workspace ``ws`` are allocated unless given."""
+    lib = _abi.load()
+    args, E = _scorer_operands(pq, w1c, b1, w2, b2, w3, b3, gs, skip)
+    dev = pq.device
+    if da1 is None:
+        da1 = torch.empty(E, SCORER_D, dtype=torch.float32, device=dev)
+    if grads is None:
+        grads = torch.empty(NGRADS, dtype=torch.float32, device=dev)
+    if ws is None:
+        ws = _ws(lib.pangnn_edge_score_workspace_bytes(E), dev)
+    dlogits = None if dlogits is None else dlogits.contiguous()
+    y = None if y is None else y.contiguous()
+    _abi.check(lib.pangnn_edge_score_bwd(*map(_p, args), E, _p(dlogits), _p(y), float(pos_weight), float(scale),
+                                         _p(da1), _p(grads), _p(logits), _p(loss_sum), _p(ws), ws.numel(), _stream()),
+               "edge_score_bwd")
+    LAUNCHES["count"] += 2 + (loss_sum is not None)
+    return da1, grads
+
+
+def _scorer_common(h, w1, skip):
+    if h.size(1) != SCORER_D or w1.size(0) != SCORER_D:
         raise _abi.PangnnError("the fused edge scorer is built for --node_dim 64")
-    wcat = torch.cat((w1[:, :D], w1[:, D:2 * D]), dim=0).contiguous()   # [2D, D]
-    w1c = w1[:, 2 * D].contiguous() if skip is not None else None
-    return wcat, w1c
+    return split_w1(w1, skip is not None)
 
 
 def _unpack_scorer_grads(grads, da1, gs, h, wcat, skip, need_h, scale=None):
@@ -752,16 +838,13 @@ def _unpack_scorer_grads(grads, da1, gs, h, wcat, skip, need_h, scale=None):
     segment_sum_edges(gs.src, da1, N, dpq[:, :D])                                 # edges by source
     segment_sum_edges(gs.dst, da1, N, dpq[:, D:])                                 # edges by target
     dwcat = gemm_tn(dpq, h)                                                        # [2D, D]
-    dw1 = torch.cat((dwcat[:D], dwcat[D:]) + ((grads[_G_W1C:_G_W1C + D].unsqueeze(1),)
-                                               if skip is not None else ()), dim=1)
     if scale is not None:
         # upstream scalar gradient: folded into the small operands, never into an [N, *] pass
         grads, dwcat, wcat = grads * scale, dwcat * scale, wcat * scale
-        dw1 = torch.cat((dwcat[:D], dwcat[D:]) + ((grads[_G_W1C:_G_W1C + D].unsqueeze(1),)
-                                                   if skip is not None else ()), dim=1)
+    g = scorer_grads(grads)
+    dw1 = torch.cat((dwcat[:D], dwcat[D:]) + ((g.dw1c.unsqueeze(1),) if skip is not None else ()), dim=1)
     dh = node_linear(dpq, wcat, w_is_kn=True) if need_h else None
-    return (dh, dw1, grads[_G_B1:_G_B1 + D], grads[_G_W2:_G_W2 + D * D].view(D, D),
-            grads[_G_B2:_G_B2 + D], grads[_G_W3:_G_W3 + D].view(1, D), grads[_G_B3:_G_B3 + 1])
+    return dh, dw1, g.db1, g.dW2, g.db2, g.dw3, g.db3
 
 
 class EdgeScoreFn(torch.autograd.Function):
@@ -769,40 +852,20 @@ class EdgeScoreFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, h, w1, b1, w2, b2, w3, b3, gs, skip):
-        lib = _abi.load()
         wcat, w1c = _scorer_common(h, w1, skip)
-        src, dst = gs.endpoints32
-        E = gs.num_edges
         pq = node_linear(h, wcat)                                       # hoisted layer 1
-        logits = torch.empty(E, dtype=torch.float32, device=h.device)
-        _abi.check(lib.pangnn_edge_score_fwd(_p(pq), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                             _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3),
-                                             E, None, 1.0, _p(logits), None, None, 0, _stream()),
-                   "edge_score_fwd")
-        LAUNCHES["count"] += 1
+        logits = edge_score_pq_fwd(pq, w1c, b1, w2, b2, w3, b3, gs, skip)
         ctx.gs, ctx.skip = gs, skip
         ctx.save_for_backward(h, w1, b1, w2, b2, w3, b3, pq)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        lib = _abi.load()
         h, w1, b1, w2, b2, w3, b3, pq = ctx.saved_tensors
         gs, skip = ctx.gs, ctx.skip
         wcat, w1c = _scorer_common(h, w1, skip)
-        src, dst = gs.endpoints32
-        E = gs.num_edges
-        da1 = torch.empty(E, SCORER_D, dtype=torch.float32, device=h.device)
-        grads = torch.empty(NGRADS, dtype=torch.float32, device=h.device)
-        ws = _ws(lib.pangnn_edge_score_workspace_bytes(E), h.device)
-        _abi.check(lib.pangnn_edge_score_bwd(_p(pq), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                             _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3),
-                                             E, _p(dlogits.contiguous()), None, 1.0, 1.0, _p(da1),
-                                             _p(grads), None, None, _p(ws), ws.numel(), _stream()),
-                   "edge_score_bwd")
-        LAUNCHES["count"] += 2
-        out = _unpack_scorer_grads(grads, da1, gs, h, wcat, skip, ctx.needs_input_grad[0])
-        return out + (None, None)
+        da1, grads = edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, dlogits=dlogits)
+        return _unpack_scorer_grads(grads, da1, gs, h, wcat, skip, ctx.needs_input_grad[0]) + (None, None)
 
 
 class EdgeScoreBCEFn(torch.autograd.Function):
@@ -812,23 +875,13 @@ class EdgeScoreBCEFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, h, w1, b1, w2, b2, w3, b3, gs, skip, y, pos_weight):
-        lib = _abi.load()
         wcat, w1c = _scorer_common(h, w1, skip)
-        src, dst = gs.endpoints32
         E = gs.num_edges
         pq = node_linear(h, wcat)
         logits = torch.empty(E, dtype=torch.float32, device=h.device)
         loss_sum = torch.zeros(1, dtype=torch.float64, device=h.device)
-        da1 = torch.empty(E, SCORER_D, dtype=torch.float32, device=h.device)
-        grads = torch.empty(NGRADS, dtype=torch.float32, device=h.device)
-        ws = _ws(lib.pangnn_edge_score_workspace_bytes(E), h.device)
-        _abi.check(lib.pangnn_edge_score_bwd(_p(pq), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                             _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3),
-                                             E, None, _p(y.contiguous()), float(pos_weight),
-                                             1.0 / max(E, 1), _p(da1), _p(grads), _p(logits),
-                                             _p(loss_sum), _p(ws), ws.numel(), _stream()),
-                   "edge_score_bwd(fused)")
-        LAUNCHES["count"] += 3
+        da1, grads = edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, y=y, pos_weight=pos_weight,
+                                      scale=1.0 / max(E, 1), logits=logits, loss_sum=loss_sum)
         ctx.gs, ctx.skip = gs, skip
         ctx.save_for_backward(h, wcat, da1, grads)
         ctx.mark_non_differentiable(logits)
@@ -909,8 +962,7 @@ class LinearFn(torch.autograd.Function):
         else:
             # a fresh tensor object over the caller's memory (never the caller's own tensor: returning
             # an input would need mark_dirty and tie this node's history to a reused buffer)
-            y_full = torch.empty(0, dtype=torch.float32, device=x.device).set_(
-                out_full.untyped_storage(), out_full.storage_offset(), tuple(out_full.shape), tuple(out_full.stride()))
+            y_full = _alias(out_full, out_full.shape, out_full.stride())
         y = node_linear(x, weight, bias, act, out=y_full[:M], push=push)
         ctx.act, ctx.has_bias, ctx.M = act, bias is not None, M
         ctx.save_for_backward(x, weight, y if act != ACT_NONE else None)
@@ -957,11 +1009,7 @@ class AggregateFn(torch.autograd.Function):
             g, dbias = act_bwd_bias(dy, y, ctx.act)
         else:
             g, dbias = dy.contiguous(), None
-        out = None
-        if ctx.dx_out is not None:
-            b = ctx.dx_out
-            out = torch.empty(0, dtype=b.dtype, device=b.device).set_(b.untyped_storage(), b.storage_offset(),
-                                                                      (ctx.n_in, b.size(1)), (b.size(1), 1))
+        out = None if ctx.dx_out is None else _alias(ctx.dx_out, (ctx.n_in, ctx.dx_out.size(1)))
         dx = gcn_aggregate(ctx.csr_src.rowptr, ctx.csr_src.col, ctx.val_src, g, ctx.n_in, out=out)
         return dx, (dbias if ctx.has_bias else None), None, None, None, None, None, None, None
 
@@ -977,62 +1025,45 @@ class EdgeScoreBCEPQFn(torch.autograd.Function):
         # backward then skips the pass that multiplies the [n, 2D] node gradient by the incoming scalar (0.2 ms at
         # C3 on a partition) and checks the promise with an asynchronous device-side assert instead
         ctx.unit_grad = bool(unit_grad)
-        lib = _abi.load()
-        src, dst = gs.endpoints32
-        E = gs.num_edges
-        pq = pq.contiguous()
-        ctx.dpq_out = dpq_out
+        E, D, n = gs.num_edges, SCORER_D, pq.size(0)
+        weights = (w1c, b1, w2, b2, w3, b3)
         logits = torch.empty(E, dtype=torch.float32, device=pq.device)
         loss_sum = torch.zeros(1, dtype=torch.float64, device=pq.device)
-        if E > SCORER_CHUNK_EDGES["n"] and gs.src.identity_perm:
+        ctx.gs, ctx.has_skip, ctx.n_ext, ctx.dpq_out = gs, skip is not None, n, dpq_out
+        ctx.chunked = E > SCORER_CHUNK_EDGES["n"] and gs.src.identity_perm
+        if not ctx.chunked:
+            da1, grads = edge_score_train(pq, *weights, gs, skip, y=y, pos_weight=pos_weight, scale=scale,
+                                          logits=logits, loss_sum=loss_sum)
+            ctx.save_for_backward(da1, grads)
+        else:
             # ---- chunked form: one scorer launch per run of source rows, node gradients reduced right away
-            D, n = SCORER_D, pq.size(0)
+            lib = _abi.load()
             ch = scored_chunks(gs, SCORER_CHUNK_EDGES["n"])
-            if dpq_out is not None:
-                dpq = torch.empty(0, dtype=dpq_out.dtype, device=pq.device).set_(
-                    dpq_out.untyped_storage(), dpq_out.storage_offset(), (n, 2 * D), (2 * D, 1))
-            else:
-                dpq = torch.empty(n, 2 * D, dtype=torch.float32, device=pq.device)
+            dpq = (_alias(dpq_out, (n, 2 * D)) if dpq_out is not None
+                   else torch.empty(n, 2 * D, dtype=torch.float32, device=pq.device))
             dpq.zero_()                                         # rows of nodes without scored edges; Q half accumulates
             da1 = torch.empty(ch.max_edges, D, dtype=torch.float32, device=pq.device)
             tmp = torch.empty(n, D, dtype=torch.float32, device=pq.device)
             grads = torch.zeros(NGRADS, dtype=torch.float32, device=pq.device)
             gk = torch.empty(NGRADS, dtype=torch.float32, device=pq.device)
             ws = _ws(lib.pangnn_edge_score_workspace_bytes(ch.max_edges), pq.device)
-            yc, w2c, w3c = y.contiguous(), w2.contiguous(), w3.contiguous()
-            off = lambda t, c0: None if t is None else C.c_void_p(t.data_ptr() + c0 * t.element_size())
+            src, dst = gs.endpoints32
+            y = y.contiguous()
             for (r0, r1, c0, c1), csr_k in zip(ch.runs, ch.csr_dst):
-                ek = c1 - c0
-                _abi.check(lib.pangnn_edge_score_bwd(_p(pq), off(src, c0), off(dst, c0), off(skip, c0), _p(w1c), _p(b1),
-                                                     _p(w2c), _p(b2), _p(w3c), _p(b3), ek, None, off(yc, c0),
-                                                     float(pos_weight), float(scale), _p(da1), _p(gk), off(logits, c0),
-                                                     _p(loss_sum), _p(ws), ws.numel(), _stream()), "edge_score_bwd(fused, pq, chunk)")
+                edge_score_train(pq, *weights, (src[c0:c1], dst[c0:c1]), None if skip is None else skip[c0:c1],
+                                 y=y[c0:c1], pos_weight=pos_weight, scale=scale, logits=logits[c0:c1],
+                                 loss_sum=loss_sum, da1=da1, grads=gk, ws=ws)
                 grads += gk                                     # (the loss is accumulated by the kernel's own reduction)
-                # by source: the run's rows are complete inside the chunk (identity columns; the CSR's offsets are
-                # absolute edge positions, so the row base is shifted back by c0 rows)
+                # by source: the run's rows are complete inside the chunk (identity columns).  A raw call, because
+                # the CSR's offsets are absolute edge positions: the row base is shifted back by c0 rows
                 _abi.check(lib.pangnn_gcn_aggregate(_p(gs.src.rowptr[r0:]), None, None,
                                                     C.c_void_p(da1.data_ptr() - c0 * D * 4), D, r1 - r0, D, None, ACT_NONE,
                                                     _p(dpq[r0:r1]), dpq.stride(0), _stream()), "segment_sum(chunk, by source)")
                 # by destination: this chunk's share of every node's sum, accumulated in fixed chunk order
-                gcn_aggregate(csr_k.rowptr, csr_k.perm, None, da1[:ek], n, out=tmp)
+                gcn_aggregate(csr_k.rowptr, csr_k.perm, None, da1[:c1 - c0], n, out=tmp)
                 dpq[:, D:] += tmp
-                LAUNCHES["count"] += 6
-            ctx.gs, ctx.has_skip, ctx.n_ext, ctx.chunked = gs, skip is not None, n, True
+                LAUNCHES["count"] += 3                          # the raw segment sum and the two accumulations
             ctx.save_for_backward(dpq, grads)
-            ctx.mark_non_differentiable(logits)
-            return (loss_sum * scale).float().squeeze(0), logits
-        ctx.chunked = False
-        da1 = torch.empty(E, SCORER_D, dtype=torch.float32, device=pq.device)
-        grads = torch.zeros(NGRADS, dtype=torch.float32, device=pq.device)
-        ws = _ws(lib.pangnn_edge_score_workspace_bytes(E), pq.device)
-        _abi.check(lib.pangnn_edge_score_bwd(_p(pq), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                             _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3),
-                                             E, None, _p(y.contiguous()), float(pos_weight), float(scale),
-                                             _p(da1), _p(grads), _p(logits), _p(loss_sum), _p(ws),
-                                             ws.numel(), _stream()), "edge_score_bwd(fused, pq)")
-        LAUNCHES["count"] += 3
-        ctx.gs, ctx.has_skip, ctx.n_ext = gs, skip is not None, pq.size(0)
-        ctx.save_for_backward(da1, grads)
         ctx.mark_non_differentiable(logits)
         return (loss_sum * scale).float().squeeze(0), logits
 
@@ -1043,59 +1074,16 @@ class EdgeScoreBCEPQFn(torch.autograd.Function):
         if ctx.unit_grad:
             torch._assert_async(dloss == 1)                     # misuse guard, no host synchronisation
         if ctx.chunked:                                         # the forward already reduced da1 to the nodes
-            dpq, g = da1, (grads if ctx.unit_grad else grads * dloss)
-            if not ctx.unit_grad:
-                dpq = dpq * dloss if dloss.requires_grad else dpq.mul_(dloss)
-            return (dpq, g[_G_W1C:_G_W1C + D] if ctx.has_skip else None, g[_G_B1:_G_B1 + D],
-                    g[_G_W2:_G_W2 + D * D].view(D, D), g[_G_B2:_G_B2 + D], g[_G_W3:_G_W3 + D].view(1, D),
-                    g[_G_B3:_G_B3 + 1], None, None, None, None, None, None, None)
-        if ctx.dpq_out is not None:
-            b = ctx.dpq_out
-            dpq = torch.empty(0, dtype=b.dtype, device=b.device).set_(b.untyped_storage(), b.storage_offset(),
-                                                                      (n, 2 * D), (2 * D, 1))
+            dpq = da1
         else:
-            dpq = torch.empty(n, 2 * D, dtype=torch.float32, device=da1.device)
-        segment_sum_edges(gs.src, da1, n, dpq[:, :D])
-        segment_sum_edges(gs.dst, da1, n, dpq[:, D:])
-        g = grads if ctx.unit_grad else grads * dloss
+            dpq = (_alias(ctx.dpq_out, (n, 2 * D)) if ctx.dpq_out is not None
+                   else torch.empty(n, 2 * D, dtype=torch.float32, device=da1.device))
+            segment_sum_edges(gs.src, da1, n, dpq[:, :D])
+            segment_sum_edges(gs.dst, da1, n, dpq[:, D:])
+        g = scorer_grads(grads if ctx.unit_grad else grads * dloss)
         if not ctx.unit_grad:
             dpq = dpq * dloss if dloss.requires_grad else dpq.mul_(dloss)
-        return (dpq, g[_G_W1C:_G_W1C + D] if ctx.has_skip else None, g[_G_B1:_G_B1 + D],
-                g[_G_W2:_G_W2 + D * D].view(D, D), g[_G_B2:_G_B2 + D], g[_G_W3:_G_W3 + D].view(1, D),
-                g[_G_B3:_G_B3 + 1], None, None, None, None, None, None, None)
-
-
-def edge_score_pq_fwd(pq, w1c, b1, w2, b2, w3, b3, gs, skip):
-    """Inference form of the scorer on pre-transformed endpoint rows ``pq`` [n_ext, 2D] -> logits."""
-    lib = _abi.load()
-    _need_cuda(pq)
-    src, dst = gs.endpoints32
-    E = gs.num_edges
-    logits = torch.empty(E, dtype=torch.float32, device=pq.device)
-    _abi.check(lib.pangnn_edge_score_fwd(_p(pq.contiguous()), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                         _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3),
-                                         E, None, 1.0, _p(logits), None, None, 0, _stream()),
-               "edge_score_fwd(pq)")
-    LAUNCHES["count"] += 1
-    return logits
-
-
-def edge_score_predict(pq, w1c, b1, w2, b2, w3, b3, gs, skip, threshold=0.5):
-    """Inference with the prediction head fused in: -> (logits, prob = sigmoid(logits), pred = prob >= threshold)
-    (``pangnn.py:220-221``, ``src/predict.py:54-55``)."""
-    lib = _abi.load()
-    _need_cuda(pq)
-    src, dst = gs.endpoints32
-    E = gs.num_edges
-    logits = torch.empty(E, dtype=torch.float32, device=pq.device)
-    prob = torch.empty(E, dtype=torch.float32, device=pq.device)
-    pred = torch.empty(E, dtype=torch.int32, device=pq.device)
-    _abi.check(lib.pangnn_edge_score_predict(_p(pq.contiguous()), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                             _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3), E,
-                                             float(threshold), _p(logits), _p(prob), _p(pred), _stream()),
-               "edge_score_predict")
-    LAUNCHES["count"] += 1
-    return logits, prob, pred
+        return (dpq, g.dw1c if ctx.has_skip else None, g.db1, g.dW2, g.db2, g.dw3, g.db3) + (None,) * 7
 
 
 # ------------------------------------------------------------------------------------------------

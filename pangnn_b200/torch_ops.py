@@ -19,15 +19,13 @@ Operators (all tensors CUDA; structure tensors as produced by ``ops.GraphStruct`
 * ``pangnn::edge_score_bce(pq, src, dst, skip?, w1c?, b1, w2, b2, w3, b3, y, pos_weight, scale, rowptr_src,
   perm_src, rowptr_dst, perm_dst) -> (loss, logits, da1, grads)``                     fused scorer + BCE(pos_weight)
 """
-import ctypes as C
 from typing import Optional, Tuple
 
 import torch
 from torch import Tensor
 
-from . import _abi, ops
+from . import ops
 
-_p, _stream, _ws = ops._p, ops._stream, ops._ws
 D = ops.SCORER_D
 
 
@@ -148,14 +146,7 @@ gcn_propagate.register_autograd(_propagate_backward, setup_context=_propagate_se
 @torch.library.custom_op("pangnn::edge_score", mutates_args=())
 def edge_score(pq: Tensor, src: Tensor, dst: Tensor, skip: Optional[Tensor], w1c: Optional[Tensor], b1: Tensor,
                w2: Tensor, b2: Tensor, w3: Tensor, b3: Tensor) -> Tensor:
-    lib = _abi.load()
-    E = src.numel()
-    logits = torch.empty(E, dtype=torch.float32, device=pq.device)
-    _abi.check(lib.pangnn_edge_score_fwd(_p(pq.contiguous()), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                         _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3), E, None, 1.0,
-                                         _p(logits), None, None, 0, _stream()), "edge_score_fwd")
-    ops.LAUNCHES["count"] += 1
-    return logits
+    return ops.edge_score_pq_fwd(pq, w1c, b1, w2, b2, w3, b3, (src, dst), skip)
 
 
 @edge_score.register_fake
@@ -170,19 +161,10 @@ def edge_score_bce(pq: Tensor, src: Tensor, dst: Tensor, skip: Optional[Tensor],
                    ) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (sum of the per-edge losses * scale, logits, da1 [E, 64], small gradients [NGRADS]); the last two are
     what the backward consumes (the fused kernel produces every gradient in the forward pass)."""
-    lib = _abi.load()
-    E = src.numel()
-    dev = pq.device
-    logits = torch.empty(E, dtype=torch.float32, device=dev)
-    loss_sum = torch.zeros(1, dtype=torch.float64, device=dev)
-    da1 = torch.empty(E, D, dtype=torch.float32, device=dev)
-    grads = torch.zeros(ops.NGRADS, dtype=torch.float32, device=dev)
-    ws = _ws(lib.pangnn_edge_score_workspace_bytes(E), dev)
-    _abi.check(lib.pangnn_edge_score_bwd(_p(pq.contiguous()), _p(src), _p(dst), _p(skip), _p(w1c), _p(b1),
-                                         _p(w2.contiguous()), _p(b2), _p(w3.contiguous()), _p(b3), E, None,
-                                         _p(y.contiguous()), float(pos_weight), float(scale), _p(da1), _p(grads),
-                                         _p(logits), _p(loss_sum), _p(ws), ws.numel(), _stream()), "edge_score_bwd")
-    ops.LAUNCHES["count"] += 3
+    logits = torch.empty(src.numel(), dtype=torch.float32, device=pq.device)
+    loss_sum = torch.zeros(1, dtype=torch.float64, device=pq.device)
+    da1, grads = ops.edge_score_train(pq, w1c, b1, w2, b2, w3, b3, (src, dst), skip, y=y, pos_weight=pos_weight,
+                                      scale=scale, logits=logits, loss_sum=loss_sum)
     return (loss_sum * scale).float().squeeze(0), logits, da1, grads
 
 
@@ -207,11 +189,8 @@ def _score_bce_backward(ctx, dloss, _dlogits, _dda1, _dgrads):
     dp = torch.ops.pangnn.gcn_aggregate(rowptr_src, perm_src, None, da1, n, None, ops.ACT_NONE)
     dq = torch.ops.pangnn.gcn_aggregate(rowptr_dst, perm_dst, None, da1, n, None, ops.ACT_NONE)
     dpq = torch.cat((dp, dq), dim=1) * dloss
-    g = grads * dloss
-    G = ops
-    return (dpq, None, None, None, g[G._G_W1C:G._G_W1C + D] if ctx.has_skip else None, g[G._G_B1:G._G_B1 + D],
-            g[G._G_W2:G._G_W2 + D * D].view(D, D), g[G._G_B2:G._G_B2 + D], g[G._G_W3:G._G_W3 + D].view(1, D),
-            g[G._G_B3:G._G_B3 + 1]) + (None,) * 7
+    g = ops.scorer_grads(grads * dloss)
+    return (dpq, None, None, None, g.dw1c if ctx.has_skip else None, g.db1, g.dW2, g.db2, g.dw3, g.db3) + (None,) * 7
 
 
 edge_score_bce.register_autograd(_score_bce_backward, setup_context=_score_bce_setup)
@@ -239,8 +218,7 @@ def score_edges_bce(h, w1, b1, w2, b2, w3, b3, edge_index, skip, y, pos_weight):
     reduction: -> (loss, logits).  Layer 1 of the MLP is hoisted to the nodes (``pq = h [W1a ; W1b]^T``)."""
     gs = ops.graph_struct(edge_index, h.size(0))
     src, dst = gs.endpoints32
-    wcat = torch.cat((w1[:, :D], w1[:, D:2 * D]), dim=0)
-    w1c = w1[:, 2 * D].contiguous() if skip is not None else None
+    wcat, w1c = ops.split_w1(w1, skip is not None)
     P = torch.ops.pangnn
     pq = P.node_linear(h, wcat, None, ops.ACT_NONE, False)
     E = gs.num_edges

@@ -347,12 +347,12 @@ def scorer_formulas(pq, src, dst, sk, P, y, pw, scale, dz_ext, dt):
 @pytest.mark.parametrize("skip", [True, False])
 @pytest.mark.parametrize("order", ["canonical", "shuffled"])
 def test_scorer_entry_points_at_c3_vs_fp64(c3, order, skip):
-    """``edge_score_pq_fwd``, ``edge_score_predict`` and ``pangnn_edge_score_bwd`` in its fused-loss form and in its
+    """``edge_score_pq_fwd``, ``edge_score_predict`` and ``edge_score_train`` in its fused-loss form and in its
     external-``dlogits`` form, on the C3 scored edges (canonical (src, dst) order, or shuffled) with endpoint rows
     pq [N, 2D] drawn at random, against fp64 evaluations of the same formulas; the same formulas in plain fp32 are
     the yardstick of bar (b).  Only the per-edge da1 is masked near ReLU kinks; logits and parameter gradients
     never are."""
-    from pangnn_b200 import _abi, ops
+    from pangnn_b200 import ops
     D, N, E = ops.SCORER_D, c3.N, C3_EDGES
     gen = torch.Generator(device=DEV).manual_seed(11)
     src, dst, y = c3.src.long(), c3.dst.long(), c3.y
@@ -362,7 +362,6 @@ def test_scorer_entry_points_at_c3_vs_fp64(c3, order, skip):
         src, dst, y = src[perm], dst[perm], y[perm].contiguous()
         sk = sk[perm].contiguous() if skip else None
     gs = ops.GraphStruct(torch.stack((src, dst)), N)
-    s32, d32 = gs.endpoints32
     pq = torch.randn(N, 2 * D, generator=gen, device=DEV)
     sd = {k: v.to(DEV) for k, v in make_state_dict(skip_connections=True).items()}
     P = dict(w1c=sd["mlp.0.weight"][:, 2 * D].contiguous() if skip else None, b1=sd["mlp.0.bias"],
@@ -390,30 +389,21 @@ def test_scorer_entry_points_at_c3_vs_fp64(c3, order, skip):
     pred_ok = torch.equal(pred[clear], (ref["prob"] >= 0.5).to(torch.int32)[clear])
     del z_pr, prob, pred, clear
 
-    lib, p, st = _abi.load(), ops._p, ops._stream
-    ws = ops._ws(lib.pangnn_edge_score_workspace_bytes(E), DEV)
     da1 = torch.empty(E, D, device=DEV)
     grads = torch.empty(ops.NGRADS, device=DEV)
-    w = [p(P[k]) for k in ("w1c", "b1", "w2", "b2", "w3", "b3")]
     for form in ("fused loss", "external dlogits"):
         if form == "fused loss":
             logits = torch.empty(E, device=DEV)
             loss = torch.zeros(1, dtype=torch.float64, device=DEV)
-            _abi.check(lib.pangnn_edge_score_bwd(p(pq), p(s32), p(d32), p(sk), *w, E, None, p(y), pw, scale, p(da1),
-                                                 p(grads), p(logits), p(loss), p(ws), ws.numel(), st()),
-                       "edge_score_bwd(fused loss)")
+            ops.edge_score_train(*args, y=y, pos_weight=pw, scale=scale, logits=logits, loss_sum=loss, da1=da1,
+                                 grads=grads)
             r.add("logits (bwd, fused loss)", logits, ref["logits"], r32["logits"], 2e-6, elementwise=True)
             r.add("loss sum", loss, ref["loss sum"], r32["loss sum"], 2e-6)
             del logits
         else:
-            _abi.check(lib.pangnn_edge_score_bwd(p(pq), p(s32), p(d32), p(sk), *w, E, p(dz_ext), None, 1.0, 1.0,
-                                                 p(da1), p(grads), None, None, p(ws), ws.numel(), st()),
-                       "edge_score_bwd(external dlogits)")
+            ops.edge_score_train(*args, dlogits=dz_ext, da1=da1, grads=grads)
         (g64, da1_64), (g32, da1_32) = ref[form], r32[form]
-        G = ops
-        got = {"dW2": grads[G._G_W2:G._G_W2 + D * D].view(D, D), "db2": grads[G._G_B2:G._G_B2 + D],
-               "dw3": grads[G._G_W3:G._G_W3 + D], "db3": grads[G._G_B3:G._G_B3 + 1], "db1": grads[G._G_B1:G._G_B1 + D],
-               "dw1c": grads[G._G_W1C:G._G_W1C + D]}
+        got = ops.scorer_grads(grads)._asdict()
         for k in g64:
             r.add(f"{k} ({form})", got[k], g64[k], g32[k], DW2_BAR if k == "dW2" else 1e-5)
         r.add(f"da1 off kinks ({form})", da1[ok], da1_64[ok], da1_32[ok], 1e-5)

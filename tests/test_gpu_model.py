@@ -149,7 +149,7 @@ def test_scored_only_batch_is_assembled_on_the_device(golden, flags, variant):
 @pytest.mark.parametrize("case,variant", [("c2", "union_skip"), ("c2", "default"), ("c1", "base"), ("sim5", "union_n4")])
 @pytest.mark.parametrize("ones", [True, False])
 def test_fused_embedding_conv_equals_the_two_modules(golden, flags, case, variant, ones):
-    """Linear(1, D) + conv_in as one rank-2 update (ops.EmbedConvFn) against the unfused modules, for x = ones
+    """Linear(1, D) + conv_in as one rank-2 update (ops.RankOneFn) against the unfused modules, for x = ones
     (the reference's features) and for arbitrary scalar features: logits, loss and every parameter gradient."""
     g = golden(case)
     model = build_model(variant, flags)

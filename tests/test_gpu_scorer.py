@@ -151,28 +151,24 @@ def test_pair_score_backward_kernel(mode, E):
 def test_scorer_scale_accuracy_vs_fp64():
     """2e6 edges (many tiles per CTA: long tensor-core accumulation chains for dW2): every output and
     gradient of the fused kernel against an fp64 evaluation of the same formulas on the GPU."""
-    from pangnn_b200 import ops, _abi
+    from pangnn_b200 import ops
     torch.manual_seed(0)
     N, E = 200_000, 2_000_000
     pq = torch.randn(N, 2 * D, device=DEV)
     src = torch.sort(torch.randint(0, N, (E,), device=DEV)).values
     dst = torch.randint(0, N, (E,), device=DEV)
     gs = ops.GraphStruct(torch.stack((src, dst)), N)
-    s32, d32 = gs.endpoints32
     skip = torch.rand(E, device=DEV) * 80 + 1
     y = (torch.rand(E, device=DEV) < 0.2).float()
     w1c, b1, b2 = (torch.randn(D, device=DEV) * 0.1 for _ in range(3))
     b3 = torch.randn(1, device=DEV)
     w2 = torch.randn(D, D, device=DEV) / 8
     w3 = torch.randn(1, D, device=DEV) / 8
-    lib = _abi.load()
-    p, st = ops._p, ops._stream
-    logits = torch.empty(E, device=DEV); da1 = torch.empty(E, D, device=DEV)
-    grads = torch.empty(ops.NGRADS, device=DEV); loss = torch.zeros(1, dtype=torch.float64, device=DEV)
-    ws = ops._ws(lib.pangnn_edge_score_workspace_bytes(E), DEV)
+    logits = torch.empty(E, device=DEV); loss = torch.zeros(1, dtype=torch.float64, device=DEV)
     pw, scale = 4.0, 1.0 / E
-    _abi.check(lib.pangnn_edge_score_bwd(p(pq), p(s32), p(d32), p(skip), p(w1c), p(b1), p(w2), p(b2), p(w3), p(b3), E, None,
-                                         p(y), pw, scale, p(da1), p(grads), p(logits), p(loss), p(ws), ws.numel(), st()), "bwd")
+    da1, grads = ops.edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, y=y, pos_weight=pw, scale=scale,
+                                      logits=logits, loss_sum=loss)
+    g = ops.scorer_grads(grads)
     W2, W3 = w2.double(), w3.double().squeeze(0)
     a1 = pq[src, :D].double() + pq[dst, D:].double() + skip[:, None].double() * w1c.double() + b1.double()
     r1 = a1.clamp_min(0)
@@ -185,17 +181,16 @@ def test_scorer_scale_accuracy_vs_fp64():
     da2 = dz[:, None] * W3 * (a2 > 0)
     da1_ref = (da2 @ W2) * (a1 > 0)
     rel = lambda got, ref: float((got.double() - ref).abs().max() / ref.abs().max())
-    G = ops
     assert rel(logits, z) < 2e-6
     assert abs(float(loss) - float(lsum)) <= 2e-6 * abs(float(lsum))
     # entries whose pre-activation sits within fp32 noise of a ReLU kink may legitimately flip
     ok = ((a1.abs().min(dim=1).values > 1e-5) & (a2.abs().min(dim=1).values > 1e-5))
     assert rel(da1[ok], da1_ref[ok]) < 1e-5
-    assert rel(grads[G._G_W2:G._G_W2 + D * D].view(D, D), da2.t() @ r1) < 1e-5
-    assert rel(grads[G._G_B2:G._G_B2 + D], da2.sum(0)) < 1e-5
-    assert rel(grads[G._G_W3:G._G_W3 + D], (dz[:, None] * r2).sum(0)) < 1e-5
-    assert rel(grads[G._G_B1:G._G_B1 + D], da1_ref.sum(0)) < 1e-5
-    assert rel(grads[G._G_W1C:G._G_W1C + D], (da1_ref * skip[:, None].double()).sum(0)) < 1e-5
+    assert rel(g.dW2, da2.t() @ r1) < 1e-5
+    assert rel(g.db2, da2.sum(0)) < 1e-5
+    assert rel(g.dw3[0], (dz[:, None] * r2).sum(0)) < 1e-5
+    assert rel(g.db1, da1_ref.sum(0)) < 1e-5
+    assert rel(g.dw1c, (da1_ref * skip[:, None].double()).sum(0)) < 1e-5
 
 
 @pytest.mark.parametrize("skew", [False, True])
@@ -237,3 +232,50 @@ def test_chunked_scorer_equals_the_single_launch(skew):
     assert abs(float(l0) - float(l1)) <= 1e-6 * abs(float(l0))
     for a, b in zip(g0, g1):
         assert rel_err(b.cpu().numpy(), a.cpu().numpy()) < 1e-5
+
+
+def test_scorer_launch_counts():
+    """Kernel launches each scorer path adds to ``ops.LAUNCHES`` (bench.py reports the total as ``gpu_launches``),
+    on a small graph in canonical (src, dst) order whose structures and chunks are built beforehand."""
+    from pangnn_b200 import ops
+    N, E, chunk = 1000, 20_000, 7000
+    h, ei, P, sk, y = make(N, E, True, 3)
+    order = torch.argsort(ei[0] * N + ei[1], stable=True)
+    ei, sk, y = ei[:, order].contiguous().to(DEV), sk[order].to(DEV), y[order].to(DEV)
+    gs = ops.GraphStruct(ei, N)
+    runs = len(ops.scored_chunks(gs, chunk).runs)
+    gs.endpoints32
+    assert gs.src.identity_perm and runs > 1
+    hd = h.to(DEV).requires_grad_(True)
+    Pd = {k: v.to(DEV).requires_grad_(True) for k, v in P.items()}
+    wcat, w1c = ops.split_w1(Pd["w1"].detach(), True)
+    pq = ops.node_linear(hd.detach(), wcat)
+    weights = (w1c,) + tuple(Pd[k].detach() for k in NAMES[1:])
+    counts = {}
+
+    def count(name, fn):
+        n0 = ops.LAUNCHES["count"]
+        out = fn()
+        counts[name] = ops.LAUNCHES["count"] - n0
+        return out
+
+    z = count("EdgeScoreFn", lambda: ops.EdgeScoreFn.apply(hd, *[Pd[k] for k in NAMES], gs, sk))
+    count("EdgeScoreFn backward", z.sum().backward)
+    loss, _ = count("EdgeScoreBCEFn", lambda: ops.EdgeScoreBCEFn.apply(hd, *[Pd[k] for k in NAMES], gs, sk, y, 2.0))
+    count("EdgeScoreBCEFn backward", loss.backward)
+    for name, limit in (("EdgeScoreBCEPQFn", 1 << 30), ("EdgeScoreBCEPQFn chunked", chunk)):
+        old = ops.SCORER_CHUNK_EDGES["n"]
+        ops.SCORER_CHUNK_EDGES["n"] = limit
+        try:
+            leaves = [t.clone().requires_grad_(True) for t in (pq,) + weights]
+            loss, _ = count(name, lambda: ops.EdgeScoreBCEPQFn.apply(*leaves, gs, sk, y, 2.0, 1.0 / E))
+        finally:
+            ops.SCORER_CHUNK_EDGES["n"] = old
+        count(name + " backward", loss.backward)
+    count("edge_score_pq_fwd", lambda: ops.edge_score_pq_fwd(pq, *weights, gs, sk))
+    count("edge_score_predict", lambda: ops.edge_score_predict(pq, *weights, gs, sk))
+    assert counts == {"EdgeScoreFn": 2, "EdgeScoreFn backward": 7,
+                      "EdgeScoreBCEFn": 4, "EdgeScoreBCEFn backward": 5,
+                      "EdgeScoreBCEPQFn": 3, "EdgeScoreBCEPQFn backward": 2,
+                      "EdgeScoreBCEPQFn chunked": 7 * runs, "EdgeScoreBCEPQFn chunked backward": 0,
+                      "edge_score_pq_fwd": 1, "edge_score_predict": 1}, counts

@@ -14,23 +14,19 @@ src = torch.sort(torch.randint(0, N, (E,), device=dev)).values
 dst = ((src // 100_000 + 1) % 10) * 100_000 + torch.randint(0, 100_000, (E,), device=dev)
 ei = torch.stack((src, dst))
 gs = ops.GraphStruct(ei, N)
-s32, d32 = gs.endpoints32
 skip = torch.rand(E, device=dev) * 80 + 1
 y = (torch.rand(E, device=dev) < 0.2).float()
 w1c, b1, b2, b3 = (torch.randn(D, device=dev) * 0.1 for _ in range(3)).__iter__().__next__(), torch.randn(D, device=dev) * .1, torch.randn(D, device=dev) * .1, torch.randn(1, device=dev)
 w2 = torch.randn(D, D, device=dev) / 8
 w3 = torch.randn(1, D, device=dev) / 8
-lib = _abi.load()
-p, st = ops._p, ops._stream
 logits = torch.empty(E, device=dev); da1 = torch.empty(E, D, device=dev)
 grads = torch.empty(ops.NGRADS, device=dev); loss = torch.zeros(1, dtype=torch.float64, device=dev)
-ws = ops._ws(lib.pangnn_edge_score_workspace_bytes(E), dev)
+ws = ops._ws(_abi.load().pangnn_edge_score_workspace_bytes(E), dev)
 def train():
-    _abi.check(lib.pangnn_edge_score_bwd(p(pq), p(s32), p(d32), p(skip), p(w1c), p(b1), p(w2), p(b2), p(w3), p(b3), E, None, p(y),
-                                         4.0, 1.0 / E, p(da1), p(grads), p(logits), p(loss), p(ws), ws.numel(), st()), "bwd")
+    ops.edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, y=y, pos_weight=4.0, scale=1.0 / E, logits=logits,
+                         loss_sum=loss, da1=da1, grads=grads, ws=ws)
 def infer():
-    _abi.check(lib.pangnn_edge_score_fwd(p(pq), p(s32), p(d32), p(skip), p(w1c), p(b1), p(w2), p(b2), p(w3), p(b3), E, None,
-                                         1.0, p(logits), None, None, 0, st()), "fwd")
+    ops.edge_score_pq_fwd(pq, w1c, b1, w2, b2, w3, b3, gs, skip)
 def timeit(f, reps=10):
     for _ in range(3): f()
     torch.cuda.synchronize()
@@ -70,8 +66,7 @@ def fp64_ref():
 loss.zero_(); train(); torch.cuda.synchronize()
 z, lsum, dW2, gb2, gw3, gb1, gw1c = fp64_ref()
 rel = lambda got, ref: float((got.double() - ref).abs().max() / ref.abs().max())
-G = ops
+g = ops.scorer_grads(grads)
 print(json.dumps({"err_logits": rel(logits, z), "err_loss": abs(float(loss) - float(lsum)) / abs(float(lsum)),
-                  "err_dW2": rel(grads[G._G_W2:G._G_W2 + D * D].view(D, D), dW2), "err_db2": rel(grads[G._G_B2:G._G_B2 + D], gb2),
-                  "err_dw3": rel(grads[G._G_W3:G._G_W3 + D], gw3), "err_db1": rel(grads[G._G_B1:G._G_B1 + D], gb1),
-                  "err_dw1c": rel(grads[G._G_W1C:G._G_W1C + D], gw1c)}))
+                  "err_dW2": rel(g.dW2, dW2), "err_db2": rel(g.db2, gb2), "err_dw3": rel(g.dw3[0], gw3),
+                  "err_db1": rel(g.db1, gb1), "err_dw1c": rel(g.dw1c, gw1c)}))

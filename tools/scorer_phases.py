@@ -19,13 +19,12 @@ y = (torch.rand(E, device=dev) < 0.2).float()
 w1c, b1, b2, b3 = (torch.randn(D, device=dev) * .1 for _ in range(3)).__next__(), torch.randn(D, device=dev) * .1, torch.randn(D, device=dev) * .1, torch.randn(1, device=dev)
 w2, w3 = torch.randn(D, D, device=dev) / 8, torch.randn(1, D, device=dev) / 8
 lib = _abi.load()
-p, st = ops._p, ops._stream
 logits = torch.empty(E, device=dev); da1 = torch.empty(E, D, device=dev)
 grads = torch.empty(ops.NGRADS, device=dev); loss = torch.zeros(1, dtype=torch.float64, device=dev)
 ws = ops._ws(lib.pangnn_edge_score_workspace_bytes(E), dev)
 def train():
-    _abi.check(lib.pangnn_edge_score_bwd(p(pq), p(s32), p(d32), p(skip), p(w1c), p(b1), p(w2), p(b2), p(w3), p(b3), E, None, p(y),
-                                         4.0, 1.0 / E, p(da1), p(grads), p(logits), p(loss), p(ws), ws.numel(), st()), "bwd")
+    ops.edge_score_train(pq, w1c, b1, w2, b2, w3, b3, (s32, d32), skip, y=y, pos_weight=4.0, scale=1.0 / E,
+                         logits=logits, loss_sum=loss, da1=da1, grads=grads, ws=ws)
 prof = lib.pangnn_debug_scorer_prof
 buf = (ctypes.c_ulonglong * 16)()
 for _ in range(2): train()
