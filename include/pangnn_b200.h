@@ -447,6 +447,29 @@ size_t pangnn_metric_reduce_workspace_bytes(int64_t max_runs);
 int pangnn_metric_reduce(const int64_t *runs, int64_t max_runs, const int64_t *params, int64_t *out, void *ws,
                          size_t ws_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * ROC and precision-recall curve points over runs (replaces sklearn roc_curve / precision_recall_curve at
+ * src/plot.py:103-107,131 of the reference, and the data behind its TensorBoard PR curve).
+ *   params [5] (device): as pangnn_metric_reduce.  bound [3] (device): (pos, neg) of the run that follows the last
+ *   of these runs in the whole curve, and PANGNN_CURVE_FIRST (these runs start the curve) | PANGNN_CURVE_FOLLOWED
+ *   (a run follows them); (0, 0, PANGNN_CURVE_FIRST) on one device.
+ *   mode: PANGNN_CURVE_ALL keeps every run; otherwise run k is kept if it is the first or the last of the curve, or
+ *   PANGNN_CURVE_ROC: (pos_{k+1}, neg_{k+1}) != (pos_k, neg_k)   (sklearn roc_curve drop_intermediate)
+ *   PANGNN_CURVE_PR:  pos_k != 0 or pos_{k+1} != 0               (sklearn precision_recall_curve drop_intermediate)
+ *   Kept runs in order: thresholds [c] fp32 (the run's score, +0.0 for the zeros), tp [c] = TP_0 + TP_k,
+ *   fp [c] = FP_0 + FP_k (int64); each output has room for max_runs points.  count [3] (device, written): kept
+ *   points, positives and negatives of the runs.  Deterministic, no atomics.
+ * ---------------------------------------------------------------------------------------------- */
+#define PANGNN_CURVE_ALL 0
+#define PANGNN_CURVE_ROC 1
+#define PANGNN_CURVE_PR 2
+#define PANGNN_CURVE_FIRST 1     /* bound[2]: these runs start the curve */
+#define PANGNN_CURVE_FOLLOWED 2  /* bound[2]: a run follows the last of them */
+size_t pangnn_metric_curve_workspace_bytes(int64_t max_runs);
+int pangnn_metric_curve(const int64_t *runs, int64_t max_runs, const int64_t *params, const int64_t *bound, int mode,
+                        float *thresholds, int64_t *tp, int64_t *fp, int64_t *count, void *ws, size_t ws_bytes,
+                        void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -79,6 +79,8 @@ SIGNATURES = {
     "pangnn_metric_runs": (_int, [_c_p, _c_p, _int, _c_p, _i64, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
     "pangnn_metric_reduce_workspace_bytes": (_sz, [_i64]),
     "pangnn_metric_reduce": (_int, [_c_p, _i64, _c_p, _c_p, _c_p, _sz, _c_p]),
+    "pangnn_metric_curve_workspace_bytes": (_sz, [_i64]),
+    "pangnn_metric_curve": (_int, [_c_p, _i64, _c_p, _c_p, _int, _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
 ABI_VERSION = 3

@@ -18,6 +18,10 @@
 //                128-bit AUROC numerator  sum_k neg_k (TP_{k-1} + TP_k),  the 128-bit AP numerator
 //                sum_k pos_k floor(TP_k 2^s / (TP_k + FP_k)) with s = 127 - bitlen(P), and the Youden arg-max
 //                (fp64 TP_k/P - FP_k/N, earliest run = smallest key on ties); one fixed final reduction.
+//   curve        (pangnn_metric_curve) over runs with the same params: per-tile (kept, pos, neg) sums -> the tile
+//                scan -> emit, which recomputes the cumulative counts and writes each kept run's (score, TP, FP) at
+//                its compacted position.  A run's keep decision (sklearn roc_curve / precision_recall_curve
+//                drop_intermediate) needs only the next run: read from `runs`, or from `bound` after the last run.
 // Integer sums are exact, so the result does not depend on tiles, input order or the rank split.
 #include "common.cuh"
 
@@ -456,6 +460,118 @@ reduce_final_kernel(const Partial *__restrict__ part, uint32_t nb, const int64_t
     }
 }
 
+// ---- curve points over runs ----------------------------------------------------------------------------------
+// bound: [0] pos, [1] neg of the run that follows the last of these runs, [2] PANGNN_CURVE_* flags.
+// The thread's kMItems runs and which of them are kept: run i is kept if it is the first run of the curve, the last
+// one, or passes the mode's rule against run i+1 (read across the thread's and the tile's edge from `runs`, and from
+// `bound` after the last run).
+struct CurveItems {
+    u64 key[kMItems], pos[kMItems], neg[kMItems];
+    uint32_t keep;                                             // bit r: item r is kept
+};
+
+__device__ __forceinline__ bool curve_rule(int mode, u64 pos, u64 neg, u64 npos, u64 nneg) {
+    if (mode == PANGNN_CURVE_ROC) return pos != npos || neg != nneg;
+    if (mode == PANGNN_CURVE_PR) return pos != 0 || npos != 0;
+    return true;
+}
+
+__device__ __forceinline__ void curve_items(const int64_t *__restrict__ runs, int64_t R, int64_t i0,
+                                            const int64_t *__restrict__ bound, int mode, CurveItems &it) {
+    const int64_t flags = bound[2];
+    it.keep = 0;
+#pragma unroll
+    for (int r = 0; r < kMItems; ++r) {
+        const int64_t i = i0 + r;
+        it.key[r] = 0; it.pos[r] = 0; it.neg[r] = 0;
+        if (i < R) {
+            it.key[r] = (u64)runs[3 * i];
+            it.pos[r] = (u64)runs[3 * i + 1];
+            it.neg[r] = (u64)runs[3 * i + 2];
+        }
+    }
+    u64 npos, nneg;                                            // run i0 + kMItems
+    bool has_next;
+    {
+        const int64_t i = i0 + kMItems;
+        has_next = i < R || (flags & PANGNN_CURVE_FOLLOWED);
+        npos = i < R ? (u64)runs[3 * i + 1] : (u64)bound[0];
+        nneg = i < R ? (u64)runs[3 * i + 2] : (u64)bound[1];
+    }
+#pragma unroll
+    for (int r = kMItems - 1; r >= 0; --r) {
+        const int64_t i = i0 + r;
+        if (i < R) {
+            const bool first = i == 0 && (flags & PANGNN_CURVE_FIRST);
+            if (i + 1 == R) {                                  // the next run is the bound's, if any
+                has_next = (flags & PANGNN_CURVE_FOLLOWED) != 0;
+                npos = (u64)bound[0];
+                nneg = (u64)bound[1];
+            }
+            if (first || !has_next || curve_rule(mode, it.pos[r], it.neg[r], npos, nneg)) it.keep |= 1u << r;
+        }
+        npos = it.pos[r];
+        nneg = it.neg[r];
+        has_next = true;
+    }
+}
+
+// Per tile: [0] kept runs, [1] positives, [2] negatives.  Layout tstat[3][nb].
+__global__ void __launch_bounds__(kMThreads)
+curve_tile_stats_kernel(const int64_t *__restrict__ runs, const int64_t *__restrict__ params,
+                        const int64_t *__restrict__ bound, int mode, u64 *__restrict__ tstat, uint32_t nb) {
+    const int64_t R = params[0];
+    const int64_t i0 = (int64_t)blockIdx.x * kMTile + (int64_t)threadIdx.x * kMItems;
+    CurveItems it;
+    curve_items(runs, R, i0, bound, mode, it);
+    Tri sum = {(u64)__popc(it.keep), 0, 0};
+#pragma unroll
+    for (int r = 0; r < kMItems; ++r) sum = tri_add(sum, {0ull, it.pos[r], it.neg[r]});
+    Tri total;
+    block_exscan3<kMThreads>(sum, total);
+    if (threadIdx.x == 0) {
+        tstat[blockIdx.x] = total.a;
+        tstat[(size_t)nb + blockIdx.x] = total.b;
+        tstat[2 * (size_t)nb + blockIdx.x] = total.c;
+    }
+}
+
+// Inverse of score_key: the fp32 score of a key (+0.0 for the folded zeros).
+__device__ __forceinline__ float key_score(u64 key) {
+    const uint32_t asc = ~(uint32_t)key;
+    return __uint_as_float((asc & 0x80000000u) ? (asc & 0x7fffffffu) : ~asc);
+}
+
+// Kept run i -> thr[c] (its score), tp[c] = TP_0 + TP_i, fp[c] = FP_0 + FP_i, c = kept runs before it.
+__global__ void __launch_bounds__(kMThreads)
+curve_emit_kernel(const int64_t *__restrict__ runs, const int64_t *__restrict__ params,
+                  const int64_t *__restrict__ bound, int mode, const u64 *__restrict__ toff, uint32_t nb,
+                  float *__restrict__ thr, int64_t *__restrict__ tp_out, int64_t *__restrict__ fp_out) {
+    const int64_t R = params[0];
+    const int64_t i0 = (int64_t)blockIdx.x * kMTile + (int64_t)threadIdx.x * kMItems;
+    CurveItems it;
+    curve_items(runs, R, i0, bound, mode, it);
+    Tri sum = {(u64)__popc(it.keep), 0, 0};
+#pragma unroll
+    for (int r = 0; r < kMItems; ++r) sum = tri_add(sum, {0ull, it.pos[r], it.neg[r]});
+    Tri total;
+    const Tri ex = block_exscan3<kMThreads>(sum, total);
+    u64 c = toff[blockIdx.x] + ex.a;
+    u64 tp = (u64)params[3] + toff[(size_t)nb + blockIdx.x] + ex.b;
+    u64 fp = (u64)params[4] + toff[2 * (size_t)nb + blockIdx.x] + ex.c;
+#pragma unroll
+    for (int r = 0; r < kMItems; ++r) {
+        tp += it.pos[r];
+        fp += it.neg[r];
+        if ((it.keep >> r) & 1u) {
+            thr[c] = key_score(it.key[r]);
+            tp_out[c] = (int64_t)tp;
+            fp_out[c] = (int64_t)fp;
+            ++c;
+        }
+    }
+}
+
 uint32_t tiles(int64_t n) { return (uint32_t)((n + kMTile - 1) / kMTile); }
 
 size_t runs_ws_bytes(int64_t n) {
@@ -472,6 +588,8 @@ size_t reduce_ws_bytes(int64_t max_runs) {
     const size_t nb = tiles(max_runs);
     return 2 * align_up(3 * nb * sizeof(u64), 256) + align_up(nb * sizeof(Partial), 256) + 1024;
 }
+
+size_t curve_ws_bytes(int64_t max_runs) { return 2 * align_up(3 * (size_t)tiles(max_runs) * sizeof(u64), 256) + 1024; }
 
 }  // namespace
 }  // namespace pangnn
@@ -549,6 +667,32 @@ int pangnn_metric_reduce(const int64_t *runs, int64_t max_runs, const int64_t *p
     }
     reduce_final_kernel<<<1, kMThreads, 0, st>>>(part, nb, params, out);
     PANGNN_CHECK_LAUNCH("reduce_final");
+    return PANGNN_OK;
+}
+
+size_t pangnn_metric_curve_workspace_bytes(int64_t max_runs) { return curve_ws_bytes(max_runs < 0 ? 0 : max_runs); }
+
+int pangnn_metric_curve(const int64_t *runs, int64_t max_runs, const int64_t *params, const int64_t *bound, int mode,
+                        float *thresholds, int64_t *tp, int64_t *fp, int64_t *count, void *ws, size_t ws_bytes,
+                        void *stream) {
+    PANGNN_REQUIRE(params && bound && count && max_runs >= 0, "bad arguments");
+    PANGNN_REQUIRE(mode >= PANGNN_CURVE_ALL && mode <= PANGNN_CURVE_PR, "bad curve mode");
+    PANGNN_REQUIRE(max_runs == 0 || (runs && thresholds && tp && fp && ws), "null pointer");
+    if (ws_bytes < curve_ws_bytes(max_runs)) {
+        set_error("metric_curve: workspace too small (%zu < %zu)", ws_bytes, curve_ws_bytes(max_runs));
+        return PANGNN_EWORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const uint32_t nb = tiles(max_runs);
+    if (nb == 0) return check_cuda(cudaMemsetAsync(count, 0, 3 * sizeof(int64_t), st), "memset(count)");
+    Workspace w(ws, ws_bytes);
+    u64 *tstat = w.take<u64>(3 * (size_t)nb), *toff = w.take<u64>(3 * (size_t)nb);
+    curve_tile_stats_kernel<<<nb, kMThreads, 0, st>>>(runs, params, bound, mode, tstat, nb);
+    PANGNN_CHECK_LAUNCH("curve_tile_stats");
+    tile_scan_kernel<<<1, kScanThreads1, 0, st>>>(tstat, nb, 0, toff, count);
+    PANGNN_CHECK_LAUNCH("curve_tile_scan");
+    curve_emit_kernel<<<nb, kMThreads, 0, st>>>(runs, params, bound, mode, toff, nb, thresholds, tp, fp);
+    PANGNN_CHECK_LAUNCH("curve_emit");
     return PANGNN_OK;
 }
 

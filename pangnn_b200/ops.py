@@ -1208,6 +1208,34 @@ def metric_reduce(runs, params, out=None):
     return out
 
 
+CURVE_ALL, CURVE_ROC, CURVE_PR = 0, 1, 2
+CURVE_FIRST, CURVE_FOLLOWED = 1, 2
+
+
+def metric_curve(runs, params, bound, mode, out=None):
+    """``pangnn_metric_curve`` over the first ``params[0]`` rows of ``runs`` (device int64 params: runs, P, N, TP_0,
+    FP_0; ``bound`` int64 [3]: (pos, neg) of the run after the last one, ``CURVE_FIRST | CURVE_FOLLOWED`` flags) with
+    ``mode`` ``CURVE_ALL`` / ``CURVE_ROC`` / ``CURVE_PR`` -> (thresholds fp32 [R], TP int64 [R], FP int64 [R],
+    count int64 [3]) on the device: the first ``count[0]`` points are the kept runs; ``count[1:3]`` = (pos, neg) of
+    the runs.  ``out`` = the same four tensors, preallocated."""
+    lib = _abi.load()
+    _need_cuda(runs, params, bound)
+    runs = runs.contiguous()
+    R, dev = runs.size(0), runs.device
+    if out is None:
+        out = (torch.empty(R, dtype=torch.float32, device=dev), torch.empty(R, dtype=torch.int64, device=dev),
+               torch.empty(R, dtype=torch.int64, device=dev), torch.empty(3, dtype=torch.int64, device=dev))
+    thr, tp, fp, count = out
+    _need_cuda(thr, tp, fp, count)
+    if min(thr.numel(), tp.numel(), fp.numel()) < R or count.numel() < 3:
+        raise _abi.PangnnError(f"metric_curve: outputs need room for {R} points and count for 3")
+    ws = _ws(lib.pangnn_metric_curve_workspace_bytes(R), dev)
+    _abi.check(lib.pangnn_metric_curve(_p(runs), R, _p(params), _p(bound), int(mode), _p(thr), _p(tp), _p(fp),
+                                       _p(count), _p(ws), ws.numel(), _stream()), "metric_curve")
+    LAUNCHES["count"] += 3 if R else 1
+    return out
+
+
 def rows_gather_copy(src, idx, dst):
     """dst[k] = src[idx[k]] (idx int32 or None); ``dst`` may be a PEER tensor (symmetric memory)."""
     lib = _abi.load()

@@ -10,11 +10,12 @@ numbers they would show are logged and returned.
 import os
 import time
 
+import numpy as np
 import torch
 
 from . import postprocessing as post
 from . import setup
-from .metrics import ranking_metrics
+from .metrics import precision_recall_curve, ranking_metrics, roc_curve
 from .data import DeviceLoader
 from .dataset import UnionGraphDataset
 from .gnn import AlternateGCN
@@ -144,6 +145,29 @@ def write_groups(dataset, graph, stat, out_dir):
     return path
 
 
+def write_curves(graph, stat, out_dir):
+    """``roc_curve.csv`` (threshold,fpr,tpr) and ``precision_recall_curve.csv`` (threshold,precision,recall; the final
+    (1, 0) point has no threshold) of the test probabilities, thinned as sklearn's ``drop_intermediate=True``: the
+    data of the reference's ROC and PR figures (``src/plot.py:103-107,131``).  Floats are written round-trip exact."""
+    roc = roc_curve(stat["prob"], graph.y)
+    if roc is None:
+        return None
+    pr = precision_recall_curve(stat["prob"], graph.y, drop_intermediate=True)
+    os.makedirs(out_dir, exist_ok=True)
+    paths = os.path.join(out_dir, "roc_curve.csv"), os.path.join(out_dir, "precision_recall_curve.csv")
+    fpr, tpr, th = roc
+    np.savetxt(paths[0], torch.stack((th, fpr, tpr), 1).cpu().numpy(), fmt="%.17g", delimiter=",",
+               header="threshold,fpr,tpr", comments="")
+    precision, recall, th = pr
+    with open(paths[1], "w") as f:
+        f.write("threshold,precision,recall\n")
+        np.savetxt(f, torch.stack((th.double(), precision[:-1], recall[:-1]), 1).cpu().numpy(), fmt="%.17g",
+                   delimiter=",")
+        f.write(f",{float(precision[-1]):.17g},{float(recall[-1]):.17g}\n")
+    log.info(f"Wrote '{paths[0]}' ({fpr.numel()} points) and '{paths[1]}' ({precision.numel()} points)")
+    return paths
+
+
 def write_edge_table(dataset, graph, stat, out_dir):
     """``q_score_vs_logit.csv`` for the whole test graph (``src/predict.py:84-88``: the max-logit-candidate
     baseline — a segmented arg-max over the logits — and the table itself, ``src/plot.py:473-504``)."""
@@ -190,6 +214,7 @@ def run(args, device=None):
         if stats:
             add_baselines(dataset, test[0], stats[0])
             write_groups(dataset, test[0], stats[0], args.output)
+            write_curves(test[0], stats[0], args.output)                              # src/plot.py:103-107,131
             write_edge_table(dataset, test[0], stats[0], args.output)                 # src/predict.py:84-88
         return dict(model=model, dataset=dataset, history=history, test=stats)
 
@@ -271,6 +296,7 @@ def run(args, device=None):
     if stats:
         add_baselines(dataset, test[0], stats[0])
         write_groups(dataset, test[0], stats[0], args.output)
+        write_curves(test[0], stats[0], args.output)                                  # src/plot.py:103-107,131
         if args.simulate_dataset:                                                     # src/predict.py:84: not args.train or simulate
             write_edge_table(dataset, test[0], stats[0], args.output)
     return dict(model=model, dataset=dataset, history=history, test=stats, model_path=path)

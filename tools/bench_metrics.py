@@ -1,8 +1,12 @@
 """Ranking metrics (``pangnn_b200.metrics.ranking_metrics``) on the B200: whole call, sort share, post-sort share,
-algorithmic bytes, peak extra memory, sklearn on the host for comparison, and the multi-GPU merge.
+algorithmic bytes, peak extra memory, sklearn on the host for comparison, and the multi-GPU merge.  With ``--curves``:
+``roc_curve`` / ``precision_recall_curve`` instead: whole calls, the share of the curve kernels
+(``pangnn_metric_curve`` timed alone on the same runs), curve lengths with and without thinning, and sklearn's
+``roc_curve`` / ``precision_recall_curve`` on the host for the same input.
 
     python tools/bench_metrics.py --out profiles/metrics_1gpu.json
     python tools/bench_metrics.py --gpus 2 --out profiles/metrics_2gpu.json
+    python tools/bench_metrics.py --curves --out profiles/curves_1gpu.json
 
 Inputs are model-shaped: sigmoid of a bimodal logit (positives N(4, 3), negatives N(-4, 3)) at the positive fraction
 of C3 (18 %) and of C5 (1 %), with 2 % of the scores saturated at 1.0f (ties).  E >= 1e7 exceeds the L2 (8 + 4 B per
@@ -113,6 +117,77 @@ def sklearn_rows(sizes):
     return rows
 
 
+def curve_rows(sizes, reps):
+    """Whole calls of the four curve variants, ``metric_runs`` and ``metric_curve`` alone (per mode) on the same
+    input, curve lengths, and the curve pass's algorithmic bytes: two reads of 24 B per run (tile statistics, emit)
+    and 20 B per kept point (fp32 threshold, int64 TP and FP)."""
+    from pangnn_b200 import ops
+    from pangnn_b200.metrics import precision_recall_curve, roc_curve
+    dev = torch.device("cuda:0")
+    calls = {"roc_thinned": lambda s, y: roc_curve(s, y),
+             "roc_all": lambda s, y: roc_curve(s, y, drop_intermediate=False),
+             "pr_all": lambda s, y: precision_recall_curve(s, y),
+             "pr_thinned": lambda s, y: precision_recall_curve(s, y, drop_intermediate=True)}
+    modes = {"all": ops.CURVE_ALL, "roc": ops.CURVE_ROC, "pr": ops.CURVE_PR}
+    rows = []
+    for name, frac in FRACTIONS.items():
+        for E in sizes:
+            s, y = scores(E, frac, dev)
+            reps_e = max(3, reps // max(1, E // 10_000_000))
+            row = dict(workload=name, pos_fraction=frac, E=E)
+            for k, fn in calls.items():
+                row[f"{k}_len"] = fn(s, y)[0].numel()
+                row[f"{k}_ms"] = timed(lambda: fn(s, y), reps_e)
+            info = torch.zeros(6, dtype=torch.int64, device=dev)
+            row["metric_runs_ms"] = timed(lambda: ops.metric_runs(s, y, info=info), reps_e)
+            runs = ops.metric_runs(s, y, info=info)
+            R = int(info[0])
+            bound = torch.tensor([0, 0, ops.CURVE_FIRST], dtype=torch.int64, device=dev)
+            out = (torch.empty(runs.size(0), dtype=torch.float32, device=dev),
+                   torch.empty(runs.size(0), dtype=torch.int64, device=dev),
+                   torch.empty(runs.size(0), dtype=torch.int64, device=dev), torch.empty(3, dtype=torch.int64, device=dev))
+            row["runs"] = R
+            for k, mode in modes.items():
+                t = timed(lambda: ops.metric_curve(runs, info, bound, mode, out=out), reps_e)
+                kept = int(out[3][0])
+                row[f"curve_kernel_{k}_ms"] = t
+                row[f"curve_kernel_{k}_kept"] = kept
+                row[f"curve_kernel_{k}_GBps"] = (48 * R + 20 * kept) / (t * 1e6)
+            row["curve_kernel_share_of_roc_thinned"] = row["curve_kernel_roc_ms"] / row["roc_thinned_ms"]
+            row["curve_kernel_share_of_pr_all"] = row["curve_kernel_all_ms"] / row["pr_all_ms"]
+            row["curve_kernel_roc_vs_metric_runs"] = row["curve_kernel_roc_ms"] / row["metric_runs_ms"]
+            rows.append(row)
+            print(json.dumps(row), flush=True)
+            del s, y, runs, out
+            torch.cuda.empty_cache()
+    return rows
+
+
+def sklearn_curve_rows(sizes):
+    """sklearn on the host (including the device-to-host copy of the scores) and bit-equality with the device."""
+    import numpy as np
+    from sklearn.metrics import precision_recall_curve as sk_pr, roc_curve as sk_roc
+    from pangnn_b200.metrics import precision_recall_curve, roc_curve
+    rows = []
+    for E in sizes:
+        s, y = scores(E, FRACTIONS["C3"], torch.device("cuda:0"))
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        sh, yh = s.cpu().numpy(), y.cpu().numpy()
+        roc = sk_roc(yh, sh)
+        t_roc = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        sh, yh = s.cpu().numpy(), y.cpu().numpy()
+        pr = sk_pr(yh, sh)
+        t_pr = time.perf_counter() - t0
+        same = all(a.dtype == b.cpu().numpy().dtype and np.array_equal(a, b.cpu().numpy())
+                   for a, b in zip(roc + pr, roc_curve(s, y) + precision_recall_curve(s, y)))
+        rows.append(dict(E=E, sklearn_roc_curve_incl_d2h_ms=t_roc * 1e3, sklearn_pr_curve_incl_d2h_ms=t_pr * 1e3,
+                         bit_equal_to_device=same))
+        print(json.dumps(rows[-1]), flush=True)
+    return rows
+
+
 def _dist_worker(rank, world, init_file, sizes, reps, out_path):
     import torch.distributed as dist
     torch.cuda.set_device(rank)
@@ -150,12 +225,16 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--curves", action="store_true", help="time roc_curve / precision_recall_curve (one GPU)")
     a = ap.parse_args()
     from pangnn_b200 import build
     if not build.is_current():
         raise SystemExit("the CUDA library is not built or is stale: run `python -m pangnn_b200.build`")
     res = dict(gpu=gpu_info())
-    if a.gpus == 1:
+    if a.curves:
+        res["curves"] = curve_rows([1_000_000, 10_000_000, 100_000_000], a.reps)
+        res["sklearn_curves_host"] = sklearn_curve_rows([1_000_000, 10_000_000])
+    elif a.gpus == 1:
         res["one_gpu"] = one_gpu([1_000_000, 10_000_000, 100_000_000], a.reps)
         res["sklearn_host"] = sklearn_rows([1_000_000, 10_000_000])
     else:
