@@ -686,15 +686,17 @@ size_t pangnn_act_bwd_bias_workspace_bytes(int64_t num_rows, int32_t feat) {
 
 int pangnn_act_bwd_bias(const float *dy, const float *yv, int64_t num_rows, int32_t feat, int act,
                         float *g, float *dbias, void *ws, size_t ws_bytes, void *stream) {
-    PANGNN_REQUIRE(dy && dbias && ws, "null pointer");
-    PANGNN_REQUIRE(act == PANGNN_ACT_NONE || yv, "activation output required");
+    PANGNN_REQUIRE(dbias && ws, "null pointer");
     PANGNN_REQUIRE(feat > 0 && feat % 4 == 0 && feat <= 1024, "feat must be a multiple of 4, <= 1024");
     if (ws_bytes < pangnn_act_bwd_bias_workspace_bytes(num_rows, feat)) {
         set_error("act_bwd_bias: workspace too small");
         return PANGNN_EWORKSPACE;
     }
     cudaStream_t st = (cudaStream_t)stream;
+    // zero rows: the inputs are empty tensors, whose data pointer is NULL
     if (num_rows == 0) return check_cuda(cudaMemsetAsync(dbias, 0, feat * sizeof(float), st), "memset");
+    PANGNN_REQUIRE(dy, "null pointer");
+    PANGNN_REQUIRE(act == PANGNN_ACT_NONE || yv, "activation output required");
     const int64_t nb = act_blocks(num_rows);
     const int fq = feat / 4;
     const int TY = 256 / fq;

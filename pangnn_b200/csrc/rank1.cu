@@ -310,15 +310,17 @@ size_t pangnn_rank1_bwd_workspace_bytes(int64_t num_rows, int32_t feat) {
 
 int pangnn_rank1_bwd(const float *dy, const float *yv, const float *a, const float *c, int64_t num_rows, int32_t feat,
                      int act, float *sums, void *ws, size_t ws_bytes, void *stream) {
-    PANGNN_REQUIRE(dy && a && c && sums && ws, "null pointer");
-    PANGNN_REQUIRE(act == PANGNN_ACT_NONE || yv, "activation output required");
+    PANGNN_REQUIRE(sums && ws, "null pointer");
     PANGNN_REQUIRE(feat > 0 && feat % 4 == 0 && feat <= 256, "feat must be a multiple of 4, <= 256");
     if (ws_bytes < pangnn_rank1_bwd_workspace_bytes(num_rows, feat)) {
         set_error("rank1_bwd: workspace too small");
         return PANGNN_EWORKSPACE;
     }
     cudaStream_t st = (cudaStream_t)stream;
+    // zero rows: the inputs are empty tensors, whose data pointer is NULL
     if (num_rows == 0) return check_cuda(cudaMemsetAsync(sums, 0, 3 * feat * sizeof(float), st), "memset");
+    PANGNN_REQUIRE(dy && a && c, "null pointer");
+    PANGNN_REQUIRE(act == PANGNN_ACT_NONE || yv, "activation output required");
     const int64_t nb = r1_blocks(num_rows);
     const int fq = feat / 4;
     const int TY = 256 / fq;

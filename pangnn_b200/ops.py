@@ -315,10 +315,18 @@ def scored_chunks(gs, max_edges):
     return ent["chunks"]
 
 
+def _rows16(t):
+    """``t`` as dense rows from a 16-byte aligned base (the row kernels read float4 at ``base + r * F``)."""
+    if t is None:
+        return None
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 def act_bwd_bias(dy, y, act, need_g=True):
     """-> (g = dy * act'(y), dbias = column sums of g)."""
     lib = _abi.load()
-    dy = dy.contiguous()
+    dy, y = _rows16(dy), _rows16(y)
     rows, F = dy.shape
     g = torch.empty_like(dy) if (need_g and act != ACT_NONE) else None
     dbias = torch.empty(F, dtype=torch.float32, device=dy.device)
@@ -331,10 +339,12 @@ def act_bwd_bias(dy, y, act, need_g=True):
 
 def gemm_tn(a, b):
     """``a.t() @ b`` for tall-skinny operands ([N,M], [N,K], M,K in {64,128}) with our deterministic
-    streaming kernel; other shapes go to the library GEMM."""
+    streaming kernel; other shapes and layouts (row strides or bases that are not 16-byte aligned) go to the
+    library GEMM."""
     M, K = a.size(1), b.size(1)
     if (M not in (64, 128) or K not in (64, 128) or a.stride(1) != 1 or b.stride(1) != 1
-            or a.stride(0) % 4 or b.stride(0) % 4 or a.dtype != torch.float32):
+            or a.stride(0) % 4 or b.stride(0) % 4 or a.data_ptr() % 16 or b.data_ptr() % 16
+            or a.dtype != torch.float32):
         return torch.mm(a.t(), b)
     lib = _abi.load()
     N = a.size(0)
