@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define PANGNN_ABI_VERSION 3
+#define PANGNN_ABI_VERSION 4
 
 #define PANGNN_OK 0
 #define PANGNN_EINVAL (-1)    /* bad argument (null pointer, unsupported width, ...) */
@@ -115,18 +115,6 @@ int pangnn_gcn_norm_apply(const int64_t *rowptr, const int32_t *col, const uint3
 int pangnn_gcn_aggregate(const int64_t *rowptr, const int32_t *col, const float *val, const float *x,
                          int64_t ldx, int32_t num_rows, int32_t feat, const float *bias, int act,
                          float *y, int64_t ldy, void *stream);
-
-/* Aggregation over the whole-graph UNION list [sim ; band(n)] (a11, src/dataset.py:373-381) with the band kept
- * implicit (SURVEY §8b pangnn_band_aggregate; band definition src/dataset.py:351-366: i -> j for j in
- * [i-n, i+n] ∩ [0,N) incl. j = i, edge weight 1):  Y[i,:] = act( sum_{sim e in row i} val_e X[col_e,:]
- * + sum_j dis[i] dis[j] X[j,:] + bias ).  rowptr/col/val = CSR of the SIM edges only with val normalised by the
- * union graph's degrees (pangnn_gcn_norm_apply with the union `dis`); the band rows are a sliding window of
- * consecutive rows of X held in registers.  Summation order = the union CSR's (ascending column, sim before band
- * on equal columns): bit-identical to pangnn_gcn_aggregate over pangnn_csr_merge_band.  The band is symmetric,
- * so the same call on the by-source CSR is the backward.  feat in {32,64,128}, n in 1..3, X has num_rows rows. */
-int pangnn_band_aggregate(const int64_t *rowptr, const int32_t *col, const float *val, const float *dis,
-                          int32_t n, const float *x, int64_t ldx, int32_t num_rows, int32_t feat,
-                          const float *bias, int act, float *y, int64_t ldy, void *stream);
 
 /* ELU backward fused with the bias gradient: g = dy * (y > 0 ? 1 : y + 1), dbias_partial[b,:] =
  * column sums of block b's rows (deterministic two-stage reduce; final sum by the caller or by
@@ -235,18 +223,6 @@ int pangnn_csr_spmv2(const int64_t *rowptr, const int32_t *col, const float *val
                      float *ax, float *a1, void *stream);
 int pangnn_rank1_affine_act(const float *a, const float *c, const float *u, const float *v, const float *bias,
                             int64_t num_rows, int32_t feat, int act, float *y, int64_t ldy, void *stream);
-/* The convolution AFTER the folded layer: Z = A2_hat H1 with H1 = act(a u^T + c v^T + bias) rebuilt per edge
- * from the two scalars of its source instead of gathering F-wide rows (feat in {32, 64, 128}); `a`, `c` are
- * indexed by column id, (rowptr, col, val) is the normalised by-destination CSR of the second graph.
- * Backward: sums [3, feat] = sum_r dz[r,:] * sum_{e in row r} val_e (1, a_s, c_s) act'(pre_s)  =  (db, du, dv). */
-int pangnn_rank1_aggregate(const int64_t *rowptr, const int32_t *col, const float *val, const float *a, const float *c,
-                           const float *u, const float *v, const float *bias, int32_t num_rows, int32_t feat, int act,
-                           float *y, int64_t ldy, void *stream);
-size_t pangnn_rank1_aggregate_bwd_workspace_bytes(int64_t num_rows, int32_t feat);
-int pangnn_rank1_aggregate_bwd(const int64_t *rowptr, const int32_t *col, const float *val, const float *a,
-                               const float *c, const float *u, const float *v, const float *bias, int32_t num_rows,
-                               int32_t feat, int act, const float *dz, int64_t lddz, float *sums, void *ws,
-                               size_t ws_bytes, void *stream);
 size_t pangnn_rank1_bwd_workspace_bytes(int64_t num_rows, int32_t feat);
 int pangnn_rank1_bwd(const float *dy, const float *y, const float *a, const float *c, int64_t num_rows, int32_t feat,
                      int act, float *sums, void *ws, size_t ws_bytes, void *stream);

@@ -24,7 +24,6 @@ SIGNATURES = {
     "pangnn_gcn_norm": (_int, [_c_p, _c_p, _c_p, _c_p, _i32, _c_p, _c_p, _c_p]),
     "pangnn_gcn_norm_apply": (_int, [_c_p, _c_p, _c_p, _c_p, _c_p, _i32, _int, _c_p, _c_p]),
     "pangnn_gcn_aggregate": (_int, [_c_p, _c_p, _c_p, _c_p, _i64, _i32, _i32, _c_p, _int, _c_p, _i64, _c_p]),
-    "pangnn_band_aggregate": (_int, [_c_p, _c_p, _c_p, _c_p, _i32, _c_p, _i64, _i32, _i32, _c_p, _int, _c_p, _i64, _c_p]),
     "pangnn_act_bwd_bias": (_int, [_c_p, _c_p, _i64, _i32, _int, _c_p, _c_p, _c_p, _sz, _c_p]),
     "pangnn_act_bwd_bias_workspace_bytes": (_sz, [_i64, _i32]),
     "pangnn_gemm_tn_workspace_bytes": (_sz, [_i64, _i32, _i32]),
@@ -45,10 +44,6 @@ SIGNATURES = {
     "pangnn_csr_merge_band": (_int, [_c_p, _c_p, _c_p, _i64, _i64, _i32, _int, _c_p, _c_p, _c_p, _c_p]),
     "pangnn_csr_spmv2": (_int, [_c_p, _c_p, _c_p, _c_p, _i32, _c_p, _c_p, _c_p]),
     "pangnn_rank1_affine_act": (_int, [_c_p, _c_p, _c_p, _c_p, _c_p, _i64, _i32, _int, _c_p, _i64, _c_p]),
-    "pangnn_rank1_aggregate": (_int, [_c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _i32, _i32, _int, _c_p, _i64, _c_p]),
-    "pangnn_rank1_aggregate_bwd_workspace_bytes": (_sz, [_i64, _i32]),
-    "pangnn_rank1_aggregate_bwd": (_int, [_c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _i32, _i32, _int, _c_p, _i64,
-                                          _c_p, _c_p, _sz, _c_p]),
     "pangnn_rank1_bwd_workspace_bytes": (_sz, [_i64, _i32]),
     "pangnn_rank1_bwd": (_int, [_c_p, _c_p, _c_p, _c_p, _i64, _i32, _int, _c_p, _c_p, _sz, _c_p]),
     "pangnn_parse_hits_tsv_workspace_bytes": (_sz, [_i64]),
@@ -83,7 +78,7 @@ SIGNATURES = {
     "pangnn_metric_curve": (_int, [_c_p, _i64, _c_p, _c_p, _int, _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
 }
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 _lib = None
 
 

@@ -9,7 +9,6 @@
 // A row of F floats is fetched as F/4 float4 lanes, so a warp keeps 32/(F/4) edges in flight per
 // load instruction and UNROLL independent instructions before the first FMA.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace pangnn {
 
@@ -166,14 +165,6 @@ __device__ __forceinline__ void rv_store(float *p, const float (&r)[VEC]) {
     else { *reinterpret_cast<float4 *>(p) = make_float4(r[0], r[1], r[2], r[3]); }
 }
 
-template <int VEC>
-__device__ __forceinline__ void rv_load_smem(float (&r)[VEC], const float *p) {
-    const typename RowVec<VEC>::T t = *reinterpret_cast<const typename RowVec<VEC>::T *>(p);
-    if constexpr (VEC == 1) { r[0] = t; }
-    else if constexpr (VEC == 2) { r[0] = t.x; r[1] = t.y; }
-    else { r[0] = t.x; r[1] = t.y; r[2] = t.z; r[3] = t.w; }
-}
-
 constexpr int kRowsPerWarp = 32;
 
 // IDENT: col == identity and val == ones (the CSR's entries ARE consecutive rows of x): the sorted-segment sum of
@@ -272,187 +263,6 @@ gcn_aggregate_stream_kernel(const int64_t *__restrict__ rowptr, const int32_t *_
         }
     }
     while (cur < nrows) close_row();                          // last row and trailing empty rows
-}
-
-// ------------------------------------------------------------------------------------------------
-// Union graph [sim ; band(n)] (src/dataset.py:351-381) WITHOUT the band edges in memory.  The band
-// of a destination row i is the 2n+1 rows i-n .. i+n of X itself, weight dis[i] * dis[j] (its edge
-// weight is 1): for a warp that walks 32 consecutive rows these are a sliding window of consecutive
-// rows — one new coalesced row load per destination row, kept in registers — instead of 2n+1 (col,
-// val) pairs and 2n+1 gathered rows through L2 per row (41 % of the C3 union edges).  Only the sim
-// edges are streamed from their CSR, with the UNION graph's normalisation.
-// Summation order = the union CSR's (ascending column, sim edge before the band edge of the same
-// column), so the result is bit-identical to gcn_aggregate_stream_kernel over pangnn_csr_merge_band's
-// CSR: band terms are slipped in before the first sim edge whose column passes them (a warp-uniform
-// test per gather group; on simulated graphs — sim edges only between genomes — once per row).
-// ------------------------------------------------------------------------------------------------
-template <int BYTES>
-__device__ __forceinline__ void cp_async_row(void *smem_dst, const void *gsrc) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;"
-                 :: "r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc), "n"(BYTES) : "memory");
-}
-
-template <int VEC, int UNROLL, int MINB, int NB>
-__global__ void __launch_bounds__(256, MINB)
-gcn_aggregate_band_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
-                          const float *__restrict__ val, const float *__restrict__ dis,
-                          const float *__restrict__ x, int32_t ldx, int32_t num_rows,
-                          const float *__restrict__ bias, int act, float *__restrict__ y, int32_t ldy) {
-    constexpr int W = 2 * NB + 1;
-    constexpr int RING = 12;                                  // rows of X resident per warp
-    constexpr int LEAD = RING - W;                            // row loads that may still be in flight at a band use
-    constexpr int F = 32 * VEC;
-    // per warp: a ring of RING consecutive rows of X (slot = (row - (r0 - NB)) % RING), filled by cp.async one row
-    // per closed destination row, LEAD rows ahead of the row's first use; a lane only ever reads the bytes it
-    // fetched itself, so no warp synchronisation is involved
-    __shared__ __align__(16) float s_ring[8][RING][F];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int64_t r0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * kRowsPerWarp;
-    if (r0 >= num_rows) return;
-    const int nrows = (int)min((int64_t)kRowsPerWarp, (int64_t)num_rows - r0);
-    const int64_t e_begin = rowptr[r0];
-    const int my_end = (int)(rowptr[r0 + min(lane, nrows - 1) + 1] - e_begin);
-    const int n_edges = __shfl_sync(0xffffffffu, my_end, nrows - 1);
-    col += e_begin;
-    val += e_begin;
-    float *ring = &s_ring[wib][0][lane * VEC];                // this lane's columns of slot 0; slot stride F
-    const float *xl = x + lane * VEC;
-    y += r0 * (int64_t)ldy + lane * VEC;
-    if (bias) bias += lane * VEC;
-    // dis of the chunk's band range r0 - NB .. r0 + 31 + NB: lane l holds entries l and 32 + l (0 outside the graph:
-    // that band edge does not exist)
-    float d0 = 0.f, d1 = 0.f;
-    {
-        const int64_t j0 = r0 - NB + lane, j1 = j0 + 32;
-        if (j0 >= 0 && j0 < num_rows) d0 = __ldg(dis + j0);
-        if (lane < 2 * NB && j1 < num_rows) d1 = __ldg(dis + j1);
-    }
-
-    // row `rel` of the band range (graph row r0 - NB + rel) into ring slot `slot`; one cp.async group per call
-    auto fetch = [&](int rel, int slot) {
-        const int64_t j = r0 - NB + rel;
-        if (rel < nrows + 2 * NB) {
-            if (j >= 0 && j < num_rows) {
-                cp_async_row<4 * VEC>(ring + slot * F, xl + j * ldx);
-            } else {
-#pragma unroll
-                for (int q = 0; q < VEC; ++q) ring[slot * F + q] = 0.f;
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-#pragma unroll
-    for (int rel = 0; rel < RING; ++rel) fetch(rel, rel);
-
-    int cur = 0;
-    int slot0 = 0;                                            // ring slot of band term 0 of the open row
-    int cur_end = __shfl_sync(0xffffffffu, my_end, 0);
-    int bpos = 0;                                             // band terms of the open row already added
-    int band_lo = (int)r0 - NB;                               // column of band term 0 of the open row
-    float vk;                                                 // lane k < W: weight of band term k of the open row
-    auto open_row = [&]() {
-        const int rel = cur + lane;
-        const float a = __shfl_sync(0xffffffffu, d0, rel & 31), b = __shfl_sync(0xffffffffu, d1, rel & 31);
-        const float dk = rel < 32 ? a : b;
-        vk = dk * __shfl_sync(0xffffffffu, dk, NB);           // (dis[src] * 1) * dis[dst], as gcn_val_kernel
-    };
-    open_row();
-    float acc[VEC];
-#pragma unroll
-    for (int k = 0; k < VEC; ++k) acc[k] = 0.f;
-
-    auto band_upto = [&](int upto) {                          // add band terms [bpos, upto), warp-uniform
-        asm volatile("cp.async.wait_group %0;" :: "n"(LEAD) : "memory");
-#pragma unroll
-        for (int k = 0; k < W; ++k) {
-            if (k >= bpos && k < upto) {
-                int slot = slot0 + k;
-                slot -= slot >= RING ? RING : 0;
-                const float v = __shfl_sync(0xffffffffu, vk, k);
-                float w[VEC];
-                rv_load_smem<VEC>(w, ring + slot * F);
-#pragma unroll
-                for (int q = 0; q < VEC; ++q) acc[q] = fmaf(v, w[q], acc[q]);
-            }
-        }
-        bpos = max(bpos, upto);
-    };
-    auto close_row = [&]() {
-        band_upto(W);
-        float o[VEC];
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) o[k] = 0.f;
-        if (bias) rv_load<VEC>(o, bias);
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) {
-            o[k] += acc[k];
-            if (act == PANGNN_ACT_ELU) o[k] = elu1(o[k]);
-            acc[k] = 0.f;
-        }
-        rv_store<VEC>(y + (int64_t)cur * ldy, o);
-        fetch(cur + RING, slot0);                             // the slot of band term 0 takes the row RING further on
-        ++cur;
-        ++band_lo;
-        slot0 = slot0 + 1 == RING ? 0 : slot0 + 1;
-        bpos = 0;
-        cur_end = __shfl_sync(0xffffffffu, my_end, cur & 31);
-        open_row();
-    };
-
-    int32_t c_nxt = 0;
-    float v_nxt = 0.f;
-    if (lane < n_edges) {
-        c_nxt = col[lane];
-        v_nxt = val[lane];
-    }
-    for (int base = 0; base < n_edges; base += 32) {
-        const int32_t c = c_nxt;
-        const float v = v_nxt;
-        const int nb = base + 32 + lane;
-        if (nb < n_edges) {
-            c_nxt = col[nb];
-            v_nxt = val[nb];
-        }
-        const int cnt = min(32, n_edges - base);
-        for (int j0 = 0; j0 < cnt; j0 += UNROLL) {
-            float r[UNROLL][VEC];
-            float vv[UNROLL];
-            int32_t cc[UNROLL];
-#pragma unroll
-            for (int u = 0; u < UNROLL; ++u) {
-                const int j = j0 + u;
-                cc[u] = __shfl_sync(0xffffffffu, c, j & 31);
-                vv[u] = __shfl_sync(0xffffffffu, v, j & 31);
-                if (j < cnt) {
-                    rv_load<VEC>(r[u], xl + (int64_t)cc[u] * ldx);
-                } else {
-#pragma unroll
-                    for (int k = 0; k < VEC; ++k) r[u][k] = 0.f;
-                }
-            }
-            const int e0 = base + j0;
-            // whole group inside the open row and no pending band column below its largest column
-            if (e0 + UNROLL <= cur_end && (bpos >= W || cc[UNROLL - 1] <= band_lo + bpos)) {
-#pragma unroll
-                for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-                    for (int k = 0; k < VEC; ++k) acc[k] = fmaf(vv[u], r[u][k], acc[k]);
-            } else {
-#pragma unroll
-                for (int u = 0; u < UNROLL; ++u) {
-                    if (e0 + u < n_edges) {                   // warp-uniform
-                        while (e0 + u >= cur_end) close_row();
-                        const int upto = min(max(cc[u] - band_lo, 0), W);     // band columns < this column
-                        if (upto > bpos) band_upto(upto);
-#pragma unroll
-                        for (int k = 0; k < VEC; ++k) acc[k] = fmaf(vv[u], r[u][k], acc[k]);
-                    }
-                }
-            }
-        }
-    }
-    while (cur < nrows) close_row();
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
 // Wide rows (F > 128): one warp per row, loop over 128-float column panels.
@@ -639,39 +449,6 @@ int pangnn_gcn_aggregate(const int64_t *rowptr, const int32_t *col, const float 
                                                           bias, act, y, ldy);
 #undef LAUNCH
     PANGNN_CHECK_LAUNCH("gcn_aggregate");
-    return PANGNN_OK;
-}
-
-int pangnn_band_aggregate(const int64_t *rowptr, const int32_t *col, const float *val, const float *dis,
-                          int32_t n, const float *x, int64_t ldx, int32_t num_rows, int32_t feat,
-                          const float *bias, int act, float *y, int64_t ldy, void *stream) {
-    if (num_rows == 0) return PANGNN_OK;
-    PANGNN_REQUIRE(rowptr && dis && x && y, "null pointer");
-    PANGNN_REQUIRE(feat == 32 || feat == 64 || feat == 128, "feat must be 32, 64 or 128");
-    PANGNN_REQUIRE(n >= 1 && n <= 3, "band half-width must be 1..3 (wider bands: merge them into the CSR)");
-    PANGNN_REQUIRE(ldx % 4 == 0 && ldy % 4 == 0 && ldx >= feat && ldy >= feat && ldx < (1 << 30) && ldy < (1 << 30),
-                   "bad row stride");
-    PANGNN_REQUIRE(((uintptr_t)x % 16 == 0) && ((uintptr_t)y % 16 == 0) && (!bias || (uintptr_t)bias % 16 == 0),
-                   "pointers must be 16-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t warps = ((int64_t)num_rows + kRowsPerWarp - 1) / kRowsPerWarp;
-    const unsigned blocks = (unsigned)((warps * 32 + 255) / 256);
-#define BLAUNCH(VEC, UNR, MINB, NB)                                                                  \
-    gcn_aggregate_band_kernel<VEC, UNR, MINB, NB><<<blocks, 256, 0, st>>>(                           \
-        rowptr, col, val, dis, x, (int32_t)ldx, num_rows, bias, act, y, (int32_t)ldy)
-#define BLAUNCH_N(VEC, UNR, MINB)                                                                    \
-    switch (n) {                                                                                     \
-    case 1: BLAUNCH(VEC, UNR, MINB, 1); break;                                                       \
-    case 2: BLAUNCH(VEC, UNR, MINB, 2); break;                                                       \
-    default: BLAUNCH(VEC, UNR, MINB, 3); break;                                                      \
-    }
-    static const int variant = getenv("PANGNN_BAND_VARIANT") ? atoi(getenv("PANGNN_BAND_VARIANT")) : 0;   // tuning aid
-    if (feat == 128) { if (variant == 1) { BLAUNCH_N(4, 4, 3) } else { BLAUNCH_N(4, 4, 4) } }
-    else if (feat == 64) { if (variant == 1) { BLAUNCH_N(2, 4, 4) } else { BLAUNCH_N(2, 4, 5) } }
-    else { BLAUNCH_N(1, 4, 5) }
-#undef BLAUNCH_N
-#undef BLAUNCH
-    PANGNN_CHECK_LAUNCH("band_aggregate");
     return PANGNN_OK;
 }
 

@@ -110,165 +110,6 @@ rank1_bwd_kernel(const float *__restrict__ dy, const float *__restrict__ yv, con
     }
 }
 
-// ------------------------------------------------------------------------------------------------
-// The convolution AFTER the folded first layer aggregates H1 = act(a u^T + c v^T + b) — rows that are a
-// function of two scalars per node.  Z = A2_hat H1 is therefore computed WITHOUT gathering feature rows:
-// per edge the kernel fetches (a, c) of the source (8 bytes instead of 4 F), rebuilds the row in registers
-// (2 FMA + one ex2 per element) and accumulates.  The gather of [N, F] rows, the dominant cost of a
-// normalised aggregation (L2 -> SM fabric bound), becomes MUFU work: F ex2 per edge.
-// Warp = 32 consecutive rows, lanes = VEC consecutive features each (F = 32 VEC); (col, val, a, c) of the next
-// 32 edges are prefetched lane-parallel and broadcast with shuffles; rows are closed in order.
-// Backward: dL/d(u, v, b) = sum_r dZ[r,:] * sum_{e in row r} val_e (a_s, c_s, 1) act'(pre_s) — the same walk,
-// three accumulators per feature, one read of dZ per ROW; per-block partials, fixed-order reduction.
-// ------------------------------------------------------------------------------------------------
-constexpr int kR1RowsPerWarp = 32;
-constexpr int kR1Unroll = 4;                 // edges per inner step: independent FMA / ex2 chains
-
-template <int VEC>
-__device__ __forceinline__ void ldvec(float (&r)[VEC], const float *p) {
-    if constexpr (VEC == 1) { r[0] = __ldg(p); }
-    else if constexpr (VEC == 2) { const float2 t = __ldg(reinterpret_cast<const float2 *>(p)); r[0] = t.x; r[1] = t.y; }
-    else { const float4 t = __ldg(reinterpret_cast<const float4 *>(p)); r[0] = t.x; r[1] = t.y; r[2] = t.z; r[3] = t.w; }
-}
-
-template <int VEC>
-__device__ __forceinline__ void stvec(float *p, const float (&r)[VEC]) {
-    if constexpr (VEC == 1) { *p = r[0]; }
-    else if constexpr (VEC == 2) { *reinterpret_cast<float2 *>(p) = make_float2(r[0], r[1]); }
-    else { *reinterpret_cast<float4 *>(p) = make_float4(r[0], r[1], r[2], r[3]); }
-}
-
-// BWD == false: y[r,:] = sum_e val_e act(a_s u + c_s v + b)
-// BWD == true : partial[block] = sum over the block's rows of t[r,:] * sum_e val_e (1, a_s, c_s) act'(a_s u + c_s v + b)
-template <int VEC, bool BWD>
-__global__ void __launch_bounds__(256)
-rank1_aggregate_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
-                       const float *__restrict__ val, const float *__restrict__ a, const float *__restrict__ c,
-                       const float *__restrict__ u, const float *__restrict__ v, const float *__restrict__ bias,
-                       int32_t num_rows, int act, float *__restrict__ y, int64_t ldy,
-                       const float *__restrict__ t, int64_t ldt, float *__restrict__ partial) {
-    constexpr int F = 32 * VEC;
-    __shared__ float red[BWD ? 8 * 3 * F : 1];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t r0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * kR1RowsPerWarp;
-    float s0[VEC], s1[VEC], s2[VEC];                         // BWD: running column sums of this warp
-#pragma unroll
-    for (int k = 0; k < VEC; ++k) s0[k] = s1[k] = s2[k] = 0.f;
-    if (r0 < num_rows) {
-        const int nrows = (int)min((int64_t)kR1RowsPerWarp, (int64_t)num_rows - r0);
-        const int64_t e_begin = rowptr[r0];
-        const int my_end = (int)(rowptr[r0 + min(lane, nrows - 1) + 1] - e_begin);
-        const int n_edges = __shfl_sync(0xffffffffu, my_end, nrows - 1);
-        col += e_begin;
-        val += e_begin;
-        float uu[VEC], vv[VEC], bb[VEC];
-        ldvec<VEC>(uu, u + lane * VEC);
-        ldvec<VEC>(vv, v + lane * VEC);
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) bb[k] = 0.f;
-        if (bias) ldvec<VEC>(bb, bias + lane * VEC);
-        int cur = 0;
-        int cur_end = __shfl_sync(0xffffffffu, my_end, 0);
-        float q0[VEC], q1[VEC], q2[VEC];
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) q0[k] = q1[k] = q2[k] = 0.f;
-
-        auto close_row = [&]() {
-            if constexpr (!BWD) {
-                stvec<VEC>(y + (r0 + cur) * ldy + lane * VEC, q0);
-            } else {
-                float tt[VEC];
-                ldvec<VEC>(tt, t + (r0 + cur) * ldt + lane * VEC);
-#pragma unroll
-                for (int k = 0; k < VEC; ++k) {
-                    s0[k] = fmaf(tt[k], q0[k], s0[k]);
-                    s1[k] = fmaf(tt[k], q1[k], s1[k]);
-                    s2[k] = fmaf(tt[k], q2[k], s2[k]);
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < VEC; ++k) q0[k] = q1[k] = q2[k] = 0.f;
-            ++cur;
-            cur_end = __shfl_sync(0xffffffffu, my_end, cur & 31);
-        };
-
-        auto edge = [&](float we, float as, float cs, int k) {
-            const float pre = fmaf(as, uu[k], fmaf(cs, vv[k], bb[k]));
-            if constexpr (!BWD) {
-                const float h = (act == PANGNN_ACT_ELU && pre <= 0.f) ? __expf(pre) - 1.f : pre;
-                q0[k] = fmaf(we, h, q0[k]);
-            } else {
-                const float d = (act == PANGNN_ACT_ELU && pre <= 0.f) ? __expf(pre) : 1.f;
-                const float wd = we * d;
-                q0[k] += wd;
-                q1[k] = fmaf(as, wd, q1[k]);
-                q2[k] = fmaf(cs, wd, q2[k]);
-            }
-        };
-
-        float w_n = 0.f, a_n = 0.f, c_n = 0.f;
-        if (lane < n_edges) {
-            const int32_t s = col[lane];
-            w_n = val[lane]; a_n = a[s]; c_n = c[s];
-        }
-        for (int base = 0; base < n_edges; base += 32) {
-            const float w_c = w_n, a_c = a_n, c_c = c_n;
-            const int nb = base + 32 + lane;
-            if (nb < n_edges) {                                 // prefetch the next 32 edges, lane-parallel
-                const int32_t s = col[nb];
-                w_n = val[nb]; a_n = a[s]; c_n = c[s];
-            }
-            const int cnt = min(32, n_edges - base);
-            for (int j0 = 0; j0 < cnt; j0 += kR1Unroll) {
-                float we[kR1Unroll], as[kR1Unroll], cs[kR1Unroll];
-#pragma unroll
-                for (int q = 0; q < kR1Unroll; ++q) {
-                    we[q] = __shfl_sync(0xffffffffu, w_c, (j0 + q) & 31);
-                    as[q] = __shfl_sync(0xffffffffu, a_c, (j0 + q) & 31);
-                    cs[q] = __shfl_sync(0xffffffffu, c_c, (j0 + q) & 31);
-                }
-                const int e0 = base + j0;
-                if (e0 + kR1Unroll <= cur_end) {                // whole group inside the open row: independent chains
-#pragma unroll
-                    for (int q = 0; q < kR1Unroll; ++q)
-#pragma unroll
-                        for (int k = 0; k < VEC; ++k) edge(we[q], as[q], cs[q], k);
-                } else {
-#pragma unroll
-                    for (int q = 0; q < kR1Unroll; ++q) {
-                        if (e0 + q < n_edges) {                 // warp-uniform
-                            while (e0 + q >= cur_end) close_row();   // rows ending before this edge (incl. empty ones)
-#pragma unroll
-                            for (int k = 0; k < VEC; ++k) edge(we[q], as[q], cs[q], k);
-                        }
-                    }
-                }
-            }
-        }
-        while (cur < nrows) close_row();
-    }
-    if constexpr (BWD) {
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) {
-            red[(warp * 3 + 0) * F + lane * VEC + k] = s0[k];
-            red[(warp * 3 + 1) * F + lane * VEC + k] = s1[k];
-            red[(warp * 3 + 2) * F + lane * VEC + k] = s2[k];
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < 3 * F; i += blockDim.x) {
-            float s = 0.f;
-#pragma unroll
-            for (int w = 0; w < 8; ++w) s += red[w * 3 * F + i];
-            partial[(int64_t)blockIdx.x * 3 * F + i] = s;
-        }
-    }
-}
-
-static int64_t r1_agg_blocks(int64_t num_rows) {
-    const int64_t warps = (num_rows + kR1RowsPerWarp - 1) / kR1RowsPerWarp;
-    return (warps * 32 + 255) / 256;
-}
-
 static int64_t r1_blocks(int64_t num_rows) {
     const int64_t nchunks = (num_rows + kR1RowsPerChunk - 1) / kR1RowsPerChunk;
     return nchunks < 1 ? 1 : (nchunks < kR1MaxBlocks ? nchunks : kR1MaxBlocks);
@@ -328,57 +169,6 @@ int pangnn_rank1_bwd(const float *dy, const float *yv, const float *a, const flo
     rank1_bwd_kernel<<<(unsigned)nb, 256, (size_t)TY * 3 * fq * sizeof(float4), st>>>(dy, yv, a, c, num_rows, feat, act,
                                                                                      partial);
     PANGNN_CHECK_LAUNCH("rank1_bwd");
-    return reduce_partials(partial, nb, 3 * feat, 3 * feat, sums, st);
-}
-
-int pangnn_rank1_aggregate(const int64_t *rowptr, const int32_t *col, const float *val, const float *a, const float *c,
-                           const float *u, const float *v, const float *bias, int32_t num_rows, int32_t feat, int act,
-                           float *y, int64_t ldy, void *stream) {
-    if (num_rows <= 0) return PANGNN_OK;
-    PANGNN_REQUIRE(rowptr && a && c && u && v && y, "null pointer");       // col / val may be NULL without edges
-    PANGNN_REQUIRE(feat == 32 || feat == 64 || feat == 128, "feat must be 32, 64 or 128");
-    PANGNN_REQUIRE(ldy % 4 == 0 && ldy >= feat && (uintptr_t)y % 16 == 0 && (uintptr_t)u % 16 == 0 &&
-                       (uintptr_t)v % 16 == 0 && (!bias || (uintptr_t)bias % 16 == 0), "alignment");
-    cudaStream_t st = (cudaStream_t)stream;
-    const unsigned blocks = (unsigned)r1_agg_blocks(num_rows);
-#define R1LAUNCH(VEC)                                                                                          \
-    rank1_aggregate_kernel<VEC, false><<<blocks, 256, 0, st>>>(rowptr, col, val, a, c, u, v, bias, num_rows, act, y, \
-                                                               ldy, nullptr, 0, nullptr)
-    if (feat == 128) R1LAUNCH(4);
-    else if (feat == 64) R1LAUNCH(2);
-    else R1LAUNCH(1);
-#undef R1LAUNCH
-    PANGNN_CHECK_LAUNCH("rank1_aggregate");
-    return PANGNN_OK;
-}
-
-size_t pangnn_rank1_aggregate_bwd_workspace_bytes(int64_t num_rows, int32_t feat) {
-    return (size_t)r1_agg_blocks(num_rows) * 3 * feat * sizeof(float) + 256;
-}
-
-int pangnn_rank1_aggregate_bwd(const int64_t *rowptr, const int32_t *col, const float *val, const float *a,
-                               const float *c, const float *u, const float *v, const float *bias, int32_t num_rows,
-                               int32_t feat, int act, const float *dz, int64_t lddz, float *sums, void *ws,
-                               size_t ws_bytes, void *stream) {
-    PANGNN_REQUIRE(rowptr && a && c && u && v && sums && ws, "null pointer");
-    PANGNN_REQUIRE(feat == 32 || feat == 64 || feat == 128, "feat must be 32, 64 or 128");
-    if (ws_bytes < pangnn_rank1_aggregate_bwd_workspace_bytes(num_rows, feat)) {
-        set_error("rank1_aggregate_bwd: workspace too small");
-        return PANGNN_EWORKSPACE;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    if (num_rows <= 0) return check_cuda(cudaMemsetAsync(sums, 0, 3 * feat * sizeof(float), st), "memset");
-    PANGNN_REQUIRE(dz && lddz % 4 == 0 && lddz >= feat && (uintptr_t)dz % 16 == 0, "dz alignment");
-    const int64_t nb = r1_agg_blocks(num_rows);
-    float *partial = static_cast<float *>(ws);
-#define R1LAUNCH(VEC)                                                                                          \
-    rank1_aggregate_kernel<VEC, true><<<(unsigned)nb, 256, 0, st>>>(rowptr, col, val, a, c, u, v, bias, num_rows, act, \
-                                                                    nullptr, 0, dz, lddz, partial)
-    if (feat == 128) R1LAUNCH(4);
-    else if (feat == 64) R1LAUNCH(2);
-    else R1LAUNCH(1);
-#undef R1LAUNCH
-    PANGNN_CHECK_LAUNCH("rank1_aggregate_bwd");
     return reduce_partials(partial, nb, 3 * feat, 3 * feat, sums, st);
 }
 

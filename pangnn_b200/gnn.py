@@ -89,10 +89,6 @@ class AlternateGCN(nn.Module):
         self.epoch = 0
         self._categorical = bool(categorical_nodes)
         self.fuse_embedding = True        # Linear(1, D) + conv_in as one rank-2 update when x is [N, 1]
-        # ... and the next convolution's aggregation rebuilt from two scalars per source instead of gathered
-        # (ops.RankOneAggFn).  Measured on B200 at C3: F ex2 per edge is MUFU/issue-bound at the same 1.1 ms as the
-        # L2-bound gather it replaces, and its backward is slower (1.64 vs 1.28 ms) -> off by default.
-        self.fuse_second_aggregation = False
 
     # -- node embeddings after the convolutions (src/gnn.py:125-166) ------------------------------
     def embed(self, graph):
@@ -103,15 +99,6 @@ class AlternateGCN(nn.Module):
             # scalar node features: Linear(1, D) + conv_in collapse into one rank-2 update (ops.RankOneFn)
             ei = graph.union_edge_index if args.union_edge_weights else graph.edge_index
             emb, cin = self.embedding, self.conv_in
-            if self.fuse_second_aggregation and not args.base_model and cin.out_channels in ops.RANK1_AGG_WIDTHS:
-                # ... and the NEXT convolution aggregates those rows rebuilt from two scalars per source
-                # (ops.RankOneAggFn), then applies its own weight: A (H W^T) = (A H) W^T
-                nxt = self.conv_hidden if args.union_edge_weights else self.conv_out
-                ei2, w2 = (ei, graph.edge_attr) if args.union_edge_weights else (graph.neighbour_edge_index, None)
-                z = ops.embed_conv_aggregate(graph.x, emb.weight, emb.bias, cin.lin.weight, cin.bias, ei,
-                                             graph.edge_attr, ELU, ei2, w2)
-                nodes = ops.linear(z, nxt.lin.weight, nxt.bias, ELU)
-                return self._embed_tail(graph, nodes, done=1)
             nodes = ops.embed_conv(graph.x, emb.weight, emb.bias, cin.lin.weight, cin.bias, ei, graph.edge_attr, ELU)
             return self._embed_tail(graph, nodes)
         if self._categorical:
@@ -129,17 +116,16 @@ class AlternateGCN(nn.Module):
         nodes = self.conv_in(node_embeddings, ei, graph.edge_attr, _act=ELU)
         return self._embed_tail(graph, nodes)
 
-    def _embed_tail(self, graph, nodes, done=0):
-        """The layers after ``conv_in`` + ELU (``src/gnn.py:131-166``); ``done`` = how many of them the caller
-        has already applied."""
+    def _embed_tail(self, graph, nodes):
+        """The layers after ``conv_in`` + ELU (``src/gnn.py:131-166``)."""
         ELU = ops.ACT_ELU
         if args.union_edge_weights:
-            for _ in range(max(args.neighbours - 2, 1) - done):
+            for _ in range(max(args.neighbours - 2, 1)):
                 nodes = self.conv_hidden(nodes, graph.union_edge_index, graph.edge_attr, _act=ELU)
             nodes = self.conv_out(nodes, graph.union_edge_index, None, _act=ELU)
         elif args.base_model:
             nodes = self.activation_fct(self.linear_out(nodes))
-        elif not done:
+        else:
             nodes = self.conv_out(nodes, graph.neighbour_edge_index, None, _act=ELU)
         return nodes
 

@@ -215,43 +215,9 @@ def gcn_aggregate(rowptr, col, val, x, num_rows, bias=None, act=ACT_NONE, out=No
     return out
 
 
-def band_aggregate(csr, val, dis, n, x, bias=None, act=ACT_NONE, out=None):
-    """Aggregation over the union list ``[sim ; band(n)]`` with the band implicit (``pangnn_band_aggregate``):
-    ``csr`` / ``val`` = the SIM edges with the union graph's normalisation, ``dis`` = the union graph's
-    ``deg^-1/2``.  Bit-identical to ``gcn_aggregate`` over ``csr_merge_band(csr, n)``."""
-    lib = _abi.load()
-    _need_cuda(x)
-    F, rows = x.size(1), csr.num_rows
-    if x.dtype != torch.float32 or x.dim() != 2 or x.stride(1) != 1 or x.size(0) != rows:
-        raise _abi.PangnnError("x must be a float32 [num_rows, F] tensor with unit column stride")
-    if out is None:
-        out = torch.empty(rows, F, dtype=torch.float32, device=x.device)
-    _abi.check(lib.pangnn_band_aggregate(_p(csr.rowptr), _p(csr.col), _p(val), _p(dis), int(n), _p(x), x.stride(0),
-                                         rows, F, _p(bias), act, _p(out), out.stride(0), _stream()), "band_aggregate")
-    LAUNCHES["count"] += 1
-    return out
-
-
-# Implicit-band aggregation for whole-graph union structures.  OFF by default — measured on B200 (C3 union graph,
-# tools/bench_band.py): F=128 1.31-1.37 ms vs 1.13 ms for the merged CSR, F=64 0.83 vs 0.73 ms.  The merged kernel
-# already serves 6 of the 7 band rows of a destination from L1 (consecutive rows re-touch the same lines), and the
-# ring of band rows in shared memory takes 48 KB per CTA out of that same L1.  Kept: bit-identical, tested.
-BAND_AGG = {"enabled": False}
-
-
 def aggregate(gs, ent, x, by_dst, bias=None, act=ACT_NONE, out=None):
     """``A_hat x`` (``by_dst``) or ``A_hat^T x`` over the structure ``gs`` with the normalisation ``ent`` (=
-    ``gs.norm(weight, need_src=not by_dst)``).  Whole-graph union structures (``graph_struct_union``) take the
-    implicit-band kernel: only the sim edges are gathered."""
-    band = gs.band
-    if (band is not None and BAND_AGG["enabled"] and 1 <= band[1] <= 3 and x.size(1) in (32, 64, 128)
-            and x.size(0) == gs.num_nodes and x.stride(0) % 4 == 0):
-        sim, n = band
-        key = "band_dst" if by_dst else "band_src"
-        val = ent.get(key)
-        if val is None:
-            val = ent[key] = gcn_norm_apply(sim.dst if by_dst else sim.src, ent["w"], ent["dis"])
-        return band_aggregate(sim.dst if by_dst else sim.src, val, ent["dis"], n, x, bias, act, out)
+    ``gs.norm(weight, need_src=not by_dst)``)."""
     csr = gs.dst if by_dst else gs.src
     return gcn_aggregate(csr.rowptr, csr.col, ent["dst" if by_dst else "src"], x, gs.num_nodes, bias, act, out)
 
@@ -407,7 +373,6 @@ class GraphStruct:
     """Both CSR orientations of one ``edge_index`` plus int32 endpoint copies; gcn_norm values are
     cached per weight tensor.  The reference recomputes gcn_norm on every GCNConv call
     (``cached=False``); here structure and norm are built once per distinct (edge_index, weight)."""
-    band = None                                       # (sim GraphStruct, n) for a whole-graph union list [sim ; band(n)]
 
     def __init__(self, edge_index, num_nodes):
         self.edge_index = edge_index                  # keeps the storage alive (cache key safety)
@@ -476,6 +441,7 @@ class GraphStruct:
         ent = self._norm.get(key)
         if ent is None:
             dis, val_dst = gcn_norm(self.dst, weight)
+            # "w" keeps the weight tensor alive: the key holds its address (as _rank1_cached does for x)
             ent = {"w": weight, "dis": dis, "dst": val_dst, "src": None}
             self._norm[key] = ent
             while len(self._norm) > 4:
@@ -506,7 +472,6 @@ def graph_struct_union(union_edge_index, num_nodes, sim, n):
         gs._dst = csr_merge_band(sim.dst, n)
         gs._src = csr_merge_band(sim.src, n)
         gs._ends, gs._norm, gs._ready = None, OrderedDict(), None
-        gs.band = (sim, int(n))
         assert gs._dst.num_edges == gs.num_edges
         _STRUCTS[key] = gs
         while len(_STRUCTS) > _STRUCT_CAP:
@@ -661,49 +626,6 @@ class RankOneFn(torch.autograd.Function):
         return None, None, dw_e, db_e, dW, (db if ctx.has_bias else None), None
 
 
-RANK1_AGG_WIDTHS = (32, 64, 128)
-
-
-class RankOneAggFn(torch.autograd.Function):
-    """``Z = A2_hat act(a u^T + c v^T + b)``: the aggregation of the convolution that FOLLOWS the folded first
-    layer, with the rows rebuilt per edge from the two scalars (a, c) of the source instead of gathered
-    (``rank1.cu``: 8 bytes per edge instead of 4 F; F ex2 per edge).  ``csr2`` / ``val2``: normalised
-    by-destination CSR of that convolution's graph; ``a``, ``c`` are indexed by its column ids."""
-
-    @staticmethod
-    def forward(ctx, a, c, w_e, b_e, weight, bias, act, csr2, val2, n_out):
-        lib = _abi.load()
-        F = weight.size(0)
-        w_e1 = w_e.reshape(-1)
-        u, v = torch.mv(weight, w_e1), torch.mv(weight, b_e)
-        z = torch.empty(n_out, F, dtype=torch.float32, device=a.device)
-        _abi.check(lib.pangnn_rank1_aggregate(_p(csr2.rowptr), _p(csr2.col), _p(val2), _p(a), _p(c), _p(u), _p(v),
-                                              _p(bias), n_out, F, act, _p(z), z.stride(0), _stream()),
-                   "rank1_aggregate")
-        LAUNCHES["count"] += 1
-        ctx.act, ctx.has_bias, ctx.csr2, ctx.n_out = act, bias is not None, csr2, n_out
-        ctx.save_for_backward(a, c, val2, u, v, bias, w_e1, b_e, weight)
-        return z
-
-    @staticmethod
-    def backward(ctx, dz):
-        lib = _abi.load()
-        a, c, val2, u, v, bias, w_e1, b_e, weight = ctx.saved_tensors
-        csr2, F = ctx.csr2, weight.size(0)
-        dz = dz.contiguous()
-        sums = torch.empty(3, F, dtype=torch.float32, device=dz.device)
-        ws = _ws(lib.pangnn_rank1_aggregate_bwd_workspace_bytes(ctx.n_out, F), dz.device)
-        _abi.check(lib.pangnn_rank1_aggregate_bwd(_p(csr2.rowptr), _p(csr2.col), _p(val2), _p(a), _p(c), _p(u), _p(v),
-                                                  _p(bias), ctx.n_out, F, ctx.act, _p(dz), dz.stride(0), _p(sums),
-                                                  _p(ws), ws.numel(), _stream()), "rank1_aggregate_bwd")
-        LAUNCHES["count"] += 2
-        db, du, dv = sums[0], sums[1], sums[2]
-        dW = torch.addr(torch.outer(du, w_e1), dv, b_e)
-        dw_e = torch.mv(weight.t(), du).unsqueeze(1)
-        db_e = torch.mv(weight.t(), dv)
-        return None, None, dw_e, db_e, dW, (db if ctx.has_bias else None), None, None, None, None
-
-
 def _rank1_cached(gs, edge_weight, x):
     ent = gs.norm(edge_weight, need_src=False)
     key = ("rank1", x.data_ptr(), x._version)
@@ -713,21 +635,6 @@ def _rank1_cached(gs, edge_weight, x):
             del ent[k]
         ac = ent[key] = rank1_vectors(gs.dst, ent["dst"], x) + (x,)     # x kept alive: the key holds its address
     return ac[0], ac[1]
-
-
-def embed_conv_aggregate(x, w_e, b_e, weight, bias, edge_index, edge_weight, act, edge_index2, edge_weight2):
-    """``A2_hat act(GCNConv_1(Linear(1, D)(x)))``: embedding, first convolution (+activation) over
-    ``(edge_index, edge_weight)`` and the AGGREGATION of the next convolution over ``(edge_index2,
-    edge_weight2)`` without ever materialising an [N, F] activation (``RankOneAggFn``).  The caller applies the
-    next convolution's weight and bias (``linear``): ``A2_hat (H1 W2^T) = (A2_hat H1) W2^T``."""
-    _need_cuda(x, weight, edge_index, edge_index2)
-    if x.requires_grad:
-        raise _abi.PangnnError("embed_conv_aggregate: node features are data, not parameters")
-    N = x.size(0)
-    a, c = _rank1_cached(graph_struct(edge_index, N), edge_weight, x)
-    gs2 = graph_struct(edge_index2, N)
-    ent2 = gs2.norm(edge_weight2, need_src=False)
-    return RankOneAggFn.apply(a, c, w_e, b_e, weight, bias, act, gs2.dst, ent2["dst"], N)
 
 
 def embed_conv(x, w_e, b_e, weight, bias, edge_index, edge_weight=None, act=ACT_NONE):

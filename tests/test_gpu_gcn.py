@@ -175,45 +175,6 @@ def test_rank1_first_layer_at_bench_scale():
         assert float((a - r).abs().max()) < 1e-4 * float(r.abs().max())
 
 
-@pytest.mark.parametrize("N,E,n", [(1, 0, 1), (3, 4, 3), (31, 0, 2), (33, 200, 3), (1000, 12000, 1), (5000, 60000, 2),
-                                   (70_001, 800_000, 3)])
-@pytest.mark.parametrize("F", [32, 64, 128])
-def test_band_aggregate_is_bit_identical_to_the_merged_union_csr(N, E, n, F):
-    """pangnn_band_aggregate (SURVEY §8b; band of src/dataset.py:351-366 kept implicit) == pangnn_gcn_aggregate over the
-    merged union CSR, bit for bit, in both orientations: sim edges near / on the band (interleaved summation order),
-    duplicates, rows without sim edges, graph ends, N not a multiple of the 32-row chunk; with bias + ELU."""
-    from pangnn_b200 import ops
-    g = torch.Generator().manual_seed(N + 7 * E + n + F)
-    ei = torch.randint(0, N, (2, E), generator=g)
-    if E >= 10:
-        k = E // 4
-        ei[1, :k] = (ei[0, :k] + torch.randint(-n - 2, n + 3, (k,), generator=g)).clamp(0, N - 1)   # near the band
-        ei[:, k: k + E // 10] = ei[:, : E // 10]                                                  # duplicates
-        ei[:, ei[0] % 97 == 5] = 0                                                                # rows without sim edges
-    key = ei[0] * N + ei[1]
-    ei = ei[:, torch.argsort(key, stable=True)].contiguous().to(DEV)
-    w = (torch.rand(E, generator=g) * 80 + 1).to(DEV)
-    sim = ops.GraphStruct(ei, N)
-    union = ops.union_index(ei, N, n)
-    gs = ops.graph_struct_union(union, N, sim, n)
-    wu = ops.union_weights(w, union.size(1))
-    x = torch.randn(N, F, generator=g).to(DEV)
-    bias = torch.randn(F, generator=g).to(DEV)
-    ent = gs.norm(wu, need_src=True)
-    ops.BAND_AGG["enabled"] = True
-    try:
-        for by_dst in (True, False):
-            csr = gs.dst if by_dst else gs.src
-            for b, act in ((None, ops.ACT_NONE), (bias, ops.ACT_ELU)):
-                ref = ops.gcn_aggregate(csr.rowptr, csr.col, ent["dst" if by_dst else "src"], x, N, b, act)
-                got = ops.aggregate(gs, ent, x, by_dst, b, act)
-                assert ("band_dst" if by_dst else "band_src") in ent          # the implicit-band kernel ran
-                assert torch.equal(got, ref)
-    finally:
-        ops.BAND_AGG["enabled"] = False
-        ops.clear_cache()
-
-
 @pytest.mark.parametrize("F", [32, 64, 128])
 def test_identity_segment_sum_equals_the_gathered_one(F):
     """col == NULL in pangnn_gcn_aggregate (rows of x already in CSR order, the scorer's per-edge gradients of a

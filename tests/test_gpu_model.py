@@ -158,19 +158,19 @@ def test_fused_embedding_conv_equals_the_two_modules(golden, flags, case, varian
         graph.x = torch.randn(graph.x.shape, generator=torch.Generator().manual_seed(3)).to(DEV)
     pw = float(g[f"model/{variant}/pos_weight"])
     out = {}
-    for fused in (True, "agg", False):
-        model.fuse_embedding, model.fuse_second_aggregation = bool(fused), fused == "agg"
+    for fused in (True, False):
+        model.fuse_embedding = fused
         model.zero_grad()
         loss, logits = model.forward_loss(graph, pw)
         loss.backward()
         out[fused] = (loss.item(), logits.cpu().numpy(), {k: p.grad.cpu().numpy().copy() for k, p in model.named_parameters()
                                                           if p.grad is not None})
-    for fused in (True, "agg"):
-        assert abs(out[fused][0] - out[False][0]) <= 2e-6 * abs(out[False][0])
-        assert rel_err(out[fused][1], out[False][1]) < 5e-6
-        assert sorted(out[fused][2]) == sorted(out[False][2])
-        for k, v in out[False][2].items():
-            assert rel_err(out[fused][2][k], v) < 2e-5, (fused, k)
+    fused, ref = out[True], out[False]
+    assert abs(fused[0] - ref[0]) <= 2e-6 * abs(ref[0])
+    assert rel_err(fused[1], ref[1]) < 5e-6
+    assert sorted(fused[2]) == sorted(ref[2])
+    for k, v in ref[2].items():
+        assert rel_err(fused[2][k], v) < 2e-5, k
 
 
 @pytest.mark.parametrize("variant", ["union_skip", "default"])

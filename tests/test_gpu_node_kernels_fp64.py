@@ -2,8 +2,7 @@
 
 Whole-model tests (``test_gpu_c3_fp64.py``) say that a step is wrong, not which kernel broke at which shape.  Each
 test here calls one kernel at the shapes where its schedule changes -- the persistent block cap, the ``kFlush``
-chain cut of ``gemm_tn``, the tile ring of ``node_linear``, the row-closing walk of ``rank1_aggregate`` -- and
-compares it with plain torch fp64 written from the definition (dense products, ``index_add_`` over the edge list).
+chain cut of ``gemm_tn``, the tile ring of ``node_linear`` -- and compares it with plain torch fp64 written from the definition (dense products, ``index_add_`` over the edge list).
 Where a kernel has to be isolated from its fp32 inputs (the CSR values), the reference takes those same fp32 inputs
 promoted to fp64.  The halo kernels see only device pointers, so their peer buffers are plain device tensors here.
 
@@ -30,7 +29,6 @@ SHAPES = [(64, 64), (128, 64), (64, 128), (128, 128)]
 # Bars (measured on one B200 in profiles/r06_node_kernels_fp64.log; the figures are in DESIGN.md section 2)
 COL_REL = 1e-6                                 # column sums: |got - ref| <= COL_REL * sum_r |term_r|
 SCALE_REL = 1e-5                               # the project's scale-relative bar
-AGG_REL = 4e-7                                 # rank1_aggregate: __expf(pre) - 1 per edge, fp32 row accumulation
 NL_SCALE, NL_ABS = 2e-6, 2e-7                  # node_linear: 3xTF32 + ex2.approx ELU
 # gemm_tn: the tensor core truncates when it adds into its fp32 accumulator, so the error drifts one way along a
 # chain (16 tiles = 192 tcgen05.mma) where cuBLAS rounds to nearest; one-signed operands show it most.  Measured on
@@ -261,75 +259,6 @@ def test_rank1_bwd_column_sums(N, F):
     t.check()
 
 
-def _agg_graph(name, g):
-    if name == "empty_rows":                     # empty rows at the start, middle and end of 32-row chunks
-        d = [3] * 96
-        for r in (0, 15, 31, 32, 33, 47, 63, 64, 65, 66, 95):
-            d[r] = 0
-        return d
-    if name == "long_rows":                      # rows longer than a 32-edge prefetch batch
-        return [40, 70, 33, 100, 5, 0, 64, 65] * 4 + [37] * 9
-    if name == "group_ends":                     # rows ending inside a group of 4 edges
-        return [1, 2, 3, 5, 6, 7, 9, 10, 11, 13] * 10
-    if name == "31_32_33":
-        return [31, 32, 33, 0, 33, 31, 32, 1] * 8 + [33]
-    if name == "ragged":
-        d = torch.randint(0, 13, (1007,), generator=g, device=DEV)
-        return d * (torch.rand(1007, generator=g, device=DEV) > 0.25)
-    if name == "random":
-        return torch.randint(0, 41, (20_011,), generator=g, device=DEV)
-    return {"one_row": [5], "one_empty_row": [0], "edgeless": [0] * 70}[name]
-
-
-AGG_GRAPHS = ["empty_rows", "long_rows", "group_ends", "31_32_33", "ragged", "random", "one_row", "one_empty_row",
-              "edgeless"]
-
-
-@pytest.mark.parametrize("F", [32, 64, 128])
-@pytest.mark.parametrize("graph", AGG_GRAPHS)
-def test_rank1_aggregate_matches_fp64(graph, F):
-    """Z = A2 act(a u^T + c v^T + b) and its three weighted column sums, on graphs aimed at the warp's row-closing
-    walk (32 rows per warp, 32-edge prefetch batches, groups of 4 edges)."""
-    o = ops()
-    g = gen("rank1_agg", graph, F)
-    rowptr, col, val, rows = csr_of(_agg_graph(graph, g), g)
-    N, E, ldz = rowptr.numel() - 1, col.numel(), F + 4
-    a = torch.rand(N, generator=g, device=DEV) * 1.5
-    c = torch.rand(N, generator=g, device=DEV) + 0.2
-    u, v = torch.randn(F, generator=g, device=DEV) * 0.5, torch.randn(F, generator=g, device=DEV) * 0.5
-    b = torch.randn(F, generator=g, device=DEV) * 0.2
-    dz = torch.randn(N, F, generator=g, device=DEV)
-    s = col.long()
-    as64, cs64, val64 = a.double()[s][:, None], c.double()[s][:, None], val.double()[:, None]
-    pre = as64 * u.double() + cs64 * v.double() + b.double()
-    t = Table(f"rank1_aggregate, {graph}: N = {N}, E = {E}, F = {F}", ["err/bar", "scale err"])
-    for act in (o.ACT_NONE, o.ACT_ELU):
-        elu = act == o.ACT_ELU
-        buf = nan_fill(N, ldz)
-        fill = bits(buf).clone()
-        check(lib().pangnn_rank1_aggregate(ptr(rowptr), ptr(col), ptr(val), ptr(a), ptr(c), ptr(u), ptr(v), ptr(b),
-                                           N, F, act, ptr(buf), ldz, o._stream()), "rank1_aggregate")
-        h = torch.where(pre > 0, pre, torch.expm1(pre)) if elu else pre
-        ref = row_sum64(rows, N, val64 * h)
-        bar = AGG_REL * row_sum64(rows, N, val64.abs() * (h.abs() + 1))
-        r = ratio((buf[:, :F].double() - ref).abs(), bar)
-        pad_ok = torch.equal(bits(buf)[:, F:], fill[:, F:])
-        name = f"act {'elu' if elu else 'none'}"
-        t.add(f"{name}: z", r, scale_err(buf[:, :F], ref), ok=r <= 1.0 and pad_ok,
-              why=f"z error {r:.2f} x bar" if pad_ok else "padding of a row written")
-        # backward: sum_r dz[r] * sum_e val_e (1, a_s, c_s) act'(pre_e)
-        sums = torch.full((3, F), float("nan"), device=DEV)
-        ws = o._ws(lib().pangnn_rank1_aggregate_bwd_workspace_bytes(N, F), DEV)
-        check(lib().pangnn_rank1_aggregate_bwd(ptr(rowptr), ptr(col), ptr(val), ptr(a), ptr(c), ptr(u), ptr(v),
-                                               ptr(b), N, F, act, ptr(dz), dz.stride(0), ptr(sums), ptr(ws),
-                                               ws.numel(), o._stream()), "rank1_aggregate_bwd")
-        wd = val64 * (torch.where(pre > 0, 1.0, torch.exp(pre)) if elu else torch.ones_like(pre))
-        term0 = dz.double()[rows] * wd
-        for k, term in enumerate((term0, term0 * as64, term0 * cs64)):
-            _col_bar(t, f"{name}: {('db', 'du', 'dv')[k]}", sums[k], term.sum(0), term.abs().sum(0))
-    t.check()
-
-
 def _random_graph(N, E, g):
     src = torch.randint(0, N, (E,), generator=g, device=DEV)
     dst = torch.randint(0, N, (E,), generator=g, device=DEV)
@@ -347,37 +276,30 @@ def _conv64(gs, weight, h):
 
 @pytest.mark.parametrize("F", [32, 64, 128])
 @pytest.mark.parametrize("x_kind", ["ones", "scalar"])
-def test_rank1_autograd_matches_fp64_unfused(x_kind, F):
-    """RankOneFn (embed_conv) and RankOneAggFn (embed_conv_aggregate): output and dw_e, db_e, dW, db against fp64
-    autograd of the unfused Linear(1, D) -> GCNConv (-> A2 aggregation)."""
+def test_embed_conv_autograd_matches_fp64_unfused(x_kind, F):
+    """RankOneFn (embed_conv): output and dw_e, db_e, dW, db against fp64 autograd of the unfused
+    Linear(1, D) -> GCNConv."""
     o = ops()
     g = gen("rank1_autograd", x_kind, F)
     N, E, D = 20_000, 200_000, 64
     ei, w = _random_graph(N, E, g)
-    ei2, w2 = _random_graph(N, E // 2, g)
     x = torch.ones(N, 1, device=DEV) if x_kind == "ones" else torch.randn(N, 1, generator=g, device=DEV)
     params = [torch.randn(*s, generator=g, device=DEV) * 0.3 for s in ((D, 1), (D,), (F, D), (F,))]
     dy = torch.randn(N, F, generator=g, device=DEV)
     t = Table(f"rank-1 autograd, x {x_kind}, N = {N}, F = {F}", ["scale err"])
     try:
-        for fused in ("RankOneFn", "RankOneAggFn"):
-            ps = [p.clone().requires_grad_(True) for p in params]
-            if fused == "RankOneFn":
-                out = o.embed_conv(x, *ps, ei, w, o.ACT_ELU)
-            else:
-                out = o.embed_conv_aggregate(x, *ps, ei, w, o.ACT_ELU, ei2, w2)
-            out.backward(dy)
-            p64 = [p.double().requires_grad_(True) for p in params]
-            w_e, b_e, W, b = p64
-            e0 = x.double() @ w_e.t() + b_e
-            ref = tnf.elu(_conv64(o.graph_struct(ei, N), w, e0 @ W.t()) + b)
-            if fused == "RankOneAggFn":
-                ref = _conv64(o.graph_struct(ei2, N), w2, ref)
-            ref.backward(dy.double())
-            for name, got, r in zip(("out", "dw_e", "db_e", "dW", "db"), [out] + [p.grad for p in ps],
-                                    [ref] + [p.grad for p in p64]):
-                e = scale_err(got.detach(), r.detach())
-                t.add(f"{fused}: {name}", e, ok=e <= SCALE_REL, why=f"{name} {e:.2e}")
+        ps = [p.clone().requires_grad_(True) for p in params]
+        out = o.embed_conv(x, *ps, ei, w, o.ACT_ELU)
+        out.backward(dy)
+        p64 = [p.double().requires_grad_(True) for p in params]
+        w_e, b_e, W, b = p64
+        e0 = x.double() @ w_e.t() + b_e
+        ref = tnf.elu(_conv64(o.graph_struct(ei, N), w, e0 @ W.t()) + b)
+        ref.backward(dy.double())
+        for name, got, r in zip(("out", "dw_e", "db_e", "dW", "db"), [out] + [p.grad for p in ps],
+                                [ref] + [p.grad for p in p64]):
+            e = scale_err(got.detach(), r.detach())
+            t.add(f"RankOneFn: {name}", e, ok=e <= SCALE_REL, why=f"{name} {e:.2e}")
     finally:
         o.clear_cache()
     t.check()
