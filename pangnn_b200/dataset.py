@@ -126,17 +126,22 @@ class UnionGraphDataset:
         if self.calculate_baseline:
             genome_d = torch.as_tensor(self.genome_of, device=dev)
             self.base_labels = pp.baseline_labels(src, dst, w, genome_d).tolist()
-            # raw baseline: scan the raw table incl. self hits (src/helper.py:470-475)
-            q, t, b = (torch.as_tensor(a, device=dev) for a in self.raw_hits)
-            qs, ts, bs = ops.hits_sort_unique(q, t, b, N)
-            if not args.include_trivial:
-                keep = self._trivial_keep(qs, ts, genome_d)
-                qs, ts, bs = qs[keep], ts[keep], bs[keep]
-            raw = pp.baseline_labels(qs, ts, bs, genome_d)
-            key_raw = qs.long() * N + ts.long()
-            key = src.long() * N + dst.long()
-            self.base_labels_raw = raw[torch.searchsorted(key_raw, key)].tolist()
+            self.base_labels_raw = self.raw_baseline_labels(self.raw_hits, src, dst, genome_d, N).tolist()
         return g
+
+    @classmethod
+    def raw_baseline_labels(cls, raw_hits, src, dst, genome_d, num_genes):
+        """Raw baseline of the edges ``(src, dst)``: the max-candidate labels of the raw hit table incl. self hits
+        (``src/helper.py:470-475``) after the same sort, dedupe and trivial-case filter as the graph.  Every
+        (query, target genome) segment of the queries in ``src`` must be complete in ``raw_hits``."""
+        q, t, b = (torch.as_tensor(a, device=src.device) for a in raw_hits)
+        qs, ts, bs = ops.hits_sort_unique(q, t, b, num_genes)
+        if not args.include_trivial:
+            keep = cls._trivial_keep(qs, ts, genome_d)
+            qs, ts, bs = qs[keep], ts[keep], bs[keep]
+        raw = pp.baseline_labels(qs, ts, bs, genome_d)
+        key_raw = qs.long() * num_genes + ts.long()
+        return raw[torch.searchsorted(key_raw, src.long() * num_genes + dst.long())]
 
     @staticmethod
     def _trivial_keep(q, t, genome_of):

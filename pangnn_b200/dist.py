@@ -416,17 +416,22 @@ class PartitionedGraph:
         self.conv = LocalGraph(conv_ei, *b, anchor="dst", edge_weight=conv_w, group=group)
         self.nb = LocalGraph(nb_ei, *b, anchor="dst", group=group) if nb_ei is not None else None
         self.scored = LocalGraph(scored_ei, *b, anchor="src", group=group)
-        m, o = self.scored.edge_mask, self.scored.edge_order
-        pick = (lambda t: t[m][o].contiguous()) if o is not None else (lambda t: t[m].contiguous())
-        self.y = pick(y)
-        self.skip = pick(scored_w).float() if args.skip_connections else None
-        self.scored_edge_ids = pick(torch.arange(m.numel(), device=m.device))
+        m = self.scored.edge_mask
+        self.y = self.pick(y)
+        self.skip = self.pick(scored_w).float() if args.skip_connections else None
+        self.scored_edge_ids = self.pick(torch.arange(m.numel(), device=m.device))
         cnt = torch.tensor([float(self.y.numel()), float(self.y.sum().item())], dtype=torch.float64,
                            device=self.y.device)
         if world > 1:
             dist.all_reduce(cnt, group=group)
         self.num_edges_total = int(cnt[0].item())
         self.class_balance = float((cnt[0] - cnt[1]) / cnt[1])                    # src/dataset.py:346
+
+    def pick(self, t):
+        """Per-edge tensor of the scored list given to the constructor -> the rows of this rank's scored edges, in
+        their local order (the order of ``y``, ``skip`` and the logits)."""
+        m, o = self.scored.edge_mask, self.scored.edge_order
+        return t[m][o].contiguous() if o is not None else t[m].contiguous()
 
     # -- host round trip of the rank's local batch (bench.py's end-to-end leg) ----------------------
     _LOCALS = ("conv", "nb", "scored")
@@ -530,15 +535,21 @@ class PartitionedGraph:
 
     @classmethod
     def from_simulation(cls, n, G, frac_pos, frags, shuf, rank, world, device, seed=0, group=None,
-                        device_generator=False):
+                        device_generator=False, keep_hits=False):
         """Partition-local build for ``--simulate_dataset`` graphs: the rank generates the hits of its
         own genomes plus one boundary genome on each side (their candidate sets are complete, and
         every edge INTO an owned node starts there), normalises them on its own device and keeps
-        what it needs.  No data-path communication besides the halo plans."""
+        what it needs.  No data-path communication besides the halo plans.
+
+        ``keep_hits`` (host generator only) also keeps what the per-edge output table needs: ``hits``, the
+        generated raw hit table ``(q, t, bits)`` as host arrays — every (query, target genome) segment of an owned
+        query is complete in it — and ``scored_w``, the Q-scores of the rank's scored edges."""
         from . import preprocessing as pp
         from .simulate import simulate_hits, simulate_hits_device
         if args.include_trivial and world > 1:
             raise NotImplementedError("--include_trivial joins every genome pair: the +-1 genome slab is not enough")
+        if keep_hits and device_generator:
+            raise NotImplementedError("keep_hits keeps the host generator's hit table")
         # whole genomes per rank when G divides evenly, otherwise a plain contiguous id split (C4: 20 genomes on 8
         # GPUs, SURVEY §8e); either way the rank generates every genome its id range touches, +- 1
         bounds = balanced_bounds(n * G, world, genome_size=n)
@@ -567,6 +578,7 @@ class PartitionedGraph:
                               score_means=tuple(args.simulated_score_means))
             src, dst, w, y = pp.normalize_sim_scores(s["q"], s["t"], s["bits"], s["genome_of"], s["group_of"],
                                                      num_nodes=N, device=device)
+            hits = (s["q"], s["t"], s["bits"]) if keep_hits else None
             del s
         sim_ei = torch.stack((src.long(), dst.long()))
         lo, hi = bounds[rank], bounds[rank + 1]
@@ -583,7 +595,10 @@ class PartitionedGraph:
         else:
             conv_ei, conv_w = sim_ei, w
             nb_ei = None if args.base_model else band
-        return cls(bounds, rank, world, x_own, conv_ei, conv_w, nb_ei, sim_ei, w, y, group)
+        pg = cls(bounds, rank, world, x_own, conv_ei, conv_w, nb_ei, sim_ei, w, y, group)
+        if keep_hits:
+            pg.hits, pg.scored_w = hits, pg.pick(w)
+        return pg
 
 
 # ------------------------------------------------------------------------------------------------

@@ -42,12 +42,15 @@ Q_SCORE_VS_LOGIT_COLUMNS = ("source_int_id", "target_int_id", "source_str_id", "
 
 
 def write_q_score_vs_logit(edge_index, edge_attr, logits, labels, gene_lst=None, base_labels=None, base_labels_raw=None,
-                           logit_baseline=None, path="q_score_vs_logit.csv"):
+                           logit_baseline=None, path="q_score_vs_logit.csv", header=True, append=False):
     """The reference's only per-edge output table (``src/plot.py:473-504``, written from ``src/predict.py:88``):
     one row per SCORED edge, keyed by (source, target), with the input Q-score (``edge_attr[:E]`` — the literal
     slice of ``src/plot.py:456``), the output logit, the label and the three max-candidate baselines.  Same
     columns, order, dtypes (score / logit float64, homolog int64) and text format as ``DataFrame.to_csv(index=False)``.
-    Tensors may live on the device; one D2H copy per column, rows formatted by pandas' C writer."""
+    Tensors may live on the device; one D2H copy per column, rows formatted by pandas' C writer.
+
+    A table can be written in consecutive pieces: the first call with ``header=True``, the others with
+    ``header=False, append=True``; the file is byte for byte the one a single call on the whole table writes."""
     import numpy as np
     import pandas as pd
 
@@ -71,5 +74,6 @@ def write_q_score_vs_logit(edge_index, edge_attr, logits, labels, gene_lst=None,
     for name, v in (("q_score_baseline", base_labels), ("raw_baseline", base_labels_raw), ("logit_baseline", logit_baseline)):
         cols[name] = host(v, np.int64) if v is not None else np.full(E, -1, dtype=np.int64)
     os.makedirs(os.path.dirname(path) or ".", exist_ok=True)
-    pd.DataFrame(cols)[list(Q_SCORE_VS_LOGIT_COLUMNS)].to_csv(path, index=False)
+    pd.DataFrame(cols)[list(Q_SCORE_VS_LOGIT_COLUMNS)].to_csv(path, index=False, header=header,
+                                                              mode="a" if append else "w")
     return path

@@ -152,7 +152,12 @@ def write_curves(graph, stat, out_dir):
     roc = roc_curve(stat["prob"], graph.y)
     if roc is None:
         return None
-    pr = precision_recall_curve(stat["prob"], graph.y, drop_intermediate=True)
+    return write_curve_files(roc, precision_recall_curve(stat["prob"], graph.y, drop_intermediate=True), out_dir)
+
+
+def write_curve_files(roc, pr, out_dir):
+    """The two files of ``write_curves`` from the arrays of ``metrics.roc_curve`` / ``metrics.precision_recall_curve``
+    (``drop_intermediate=True``)."""
     os.makedirs(out_dir, exist_ok=True)
     paths = os.path.join(out_dir, "roc_curve.csv"), os.path.join(out_dir, "precision_recall_curve.csv")
     fpr, tpr, th = roc
@@ -183,7 +188,14 @@ def write_edge_table(dataset, graph, stat, out_dir):
 
 
 def run(args, device=None):
-    """The reference's main flow.  Returns a dict with the model, per-epoch history and test statistics."""
+    """The reference's main flow.  Returns a dict with the model, per-epoch history and test statistics.
+
+    With a default process group initialised (``main`` under ``torchrun``) every rank runs the genome-partitioned
+    driver, ``pangnn_b200.dist_train.run_partitioned``; in a group of one rank the reference's sub-graph training
+    (``--train`` without ``--whole_graph_training``) has nothing to partition and runs the loop below."""
+    from . import dist_train
+    if dist_train.partitioned(args):
+        return dist_train.run_partitioned(args, device)
     device = torch.device(device if device is not None else "cuda")
     torch.manual_seed(args.seed)
     t0 = time.time()
@@ -303,8 +315,23 @@ def run(args, device=None):
 
 
 def main(argv=None):
+    """``pangnn.py``.  Under ``torchrun --nproc-per-node N`` (``WORLD_SIZE`` > 1) each process joins an NCCL group
+    from the environment on the GPU ``LOCAL_RANK`` and runs the genome-partitioned driver; the group is destroyed on
+    exit, also on an error."""
     args = setup.parse(argv)
-    return run(args)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world <= 1:
+        return run(args)
+    import torch.distributed as dist
+    from .dist_train import check_partition_flags
+    check_partition_flags(args, world)                        # every rank refuses alike, before any device work
+    device = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
+    torch.cuda.set_device(device)
+    dist.init_process_group("nccl", init_method="env://", device_id=device)
+    try:
+        return run(args, device)
+    finally:
+        dist.destroy_process_group()
 
 
 if __name__ == "__main__":
