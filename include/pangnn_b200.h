@@ -195,6 +195,37 @@ int pangnn_rows_scatter_add(const float *src, int64_t ld_src, const int32_t *idx
                             int64_t ld_dst, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Data-parallel gradient average over NVLink PEER memory (new; the all-reduce DDP runs behind
+ * accelerator.backward, pangnn.py:207).  Every rank of a group of `world` ranks calls push, then reduce, on
+ * its stream, the same number of times; both are legal inside a CUDA-graph capture and correct on replay.
+ *   grads [count] / numels [count]: host arrays of this rank's gradient tensors (fp32, dense, any size and
+ *     alignment; a NULL entry packs zeros and is not written back).  The pointers travel BY VALUE in the
+ *     kernel parameters (count <= PANGNN_GRAD_REDUCE_MAX_TENSORS), so no pointer table lives in device memory.
+ *   bucket: this rank's symmetric buffer of 2 * half_floats floats (two halves), half_floats >=
+ *     pangnn_grad_bucket_floats(numels, count); peer_buckets [world]: every rank's bucket, mapped here.
+ *   signal: this rank's symmetric int32 [world] array; peer_signals [world]: every rank's, mapped here.
+ *   ctrl: this rank's int32 [4] in ordinary device memory, zeroed once together with `signal` before the
+ *     first call: {epoch e, push ticket, reduce ticket, status}.
+ *   push:   pack the gradients into half e & 1 of `bucket`; the last CTA then stores e + 1 into
+ *           peer_signals[p][rank] of every p (release, system scope).
+ *   reduce: wait until signal[0 .. world) >= e + 1 (acquire, %globaltimer budget timeout_ns), then
+ *           grad = (b_0 + b_1 + ... + b_{world-1}) * fp32(1 / world), the sum strictly in rank order over
+ *           half e & 1 of every peer bucket; the last CTA stores e + 1 into ctrl[0].  On expiry the kernel
+ *           stores 1 + (the first rank whose signal is missing) into ctrl[3] and returns without writing.
+ * Two halves need one signal per call: a rank that writes half h at call k + 2 has seen every peer's call k + 1
+ * signal, which each peer sends only after its call-k reads.  Epoch and parity live in device memory and the
+ * signals only grow, so eager calls and replays of different graphs interleave in any order.
+ * ---------------------------------------------------------------------------------------------- */
+#define PANGNN_GRAD_REDUCE_MAX_TENSORS 32
+#define PANGNN_GRAD_REDUCE_MAX_RANKS 8
+int64_t pangnn_grad_bucket_floats(const int64_t *numels, int32_t count);
+int pangnn_grad_push(float *const *grads, const int64_t *numels, int32_t count, float *bucket, int64_t half_floats,
+                     int32_t *const *peer_signals, int32_t world, int32_t rank, int32_t *ctrl, void *stream);
+int pangnn_grad_reduce(float *const *grads, const int64_t *numels, int32_t count, const float *const *peer_buckets,
+                       int64_t half_floats, const int32_t *signal, int32_t world, int32_t rank, int32_t *ctrl,
+                       int64_t timeout_ns, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Whole-graph neighbour band (SURVEY §8 a8; replaces the Python double loop of src/dataset.py:351-366):
  * edges i -> j, j in [i-n, i+n] ∩ [0, N), self loop included, in the reference's loop order.
  * pangnn_neighbour_band_edges is host arithmetic: (2n+1) N - n (n+1) for N > n.  out_src / out_dst are

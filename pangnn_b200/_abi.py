@@ -38,6 +38,9 @@ SIGNATURES = {
                                      _c_p, _c_p, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),
     "pangnn_rows_gather_copy": (_int, [_c_p, _i64, _c_p, _i64, _i32, _c_p, _i64, _c_p]),
     "pangnn_rows_scatter_add": (_int, [_c_p, _i64, _c_p, _i64, _i32, _c_p, _i64, _c_p]),
+    "pangnn_grad_bucket_floats": (_i64, [_c_p, _i32]),
+    "pangnn_grad_push": (_int, [_c_p, _c_p, _i32, _c_p, _i64, _c_p, _i32, _i32, _c_p, _c_p]),
+    "pangnn_grad_reduce": (_int, [_c_p, _c_p, _i32, _c_p, _i64, _c_p, _i32, _i32, _c_p, _i64, _c_p]),
     "pangnn_edges_sorted": (_int, [_c_p, _i64, _i32, _c_p, _c_p]),
     "pangnn_csr_from_sorted": (_int, [_c_p, _i64, _i32, _c_p, _c_p, _c_p, _c_p]),
     "pangnn_csr_transpose": (_int, [_c_p, _c_p, _c_p, _i64, _i32, _c_p, _c_p, _c_p, _c_p, _sz, _c_p]),

@@ -169,26 +169,36 @@ class DeviceLoader:
         return (self._ids.size + self.batch_size - 1) // self.batch_size
 
     def __iter__(self):
-        import numpy as np
-        order = list(range(self._ids.size))
-        if self.shuffle:
-            self._rng.shuffle(order)
-        order = self._ids[np.asarray(order, dtype=np.int64)] if order else self._ids[:0]
-        order_dev = torch.from_numpy(order).to(self.device)
-        for i in range(0, len(order), self.batch_size):
-            yield self.packed.collate(order[i:i + self.batch_size], order_dev[i:i + self.batch_size])
+        return self.batches()
 
-    def iter_ids(self):
+    def batches(self, shard=None, pad=True):
+        """``__iter__`` with the ``shard`` / ``pad`` options of ``iter_ids``."""
+        for packed, ids, ids_dev in self.iter_ids(shard, pad):
+            yield packed.collate(ids, ids_dev)
+
+    def iter_ids(self, shard=None, pad=True):
         """The same batches as ``__iter__`` as ``(packed, ids, ids_dev)`` — for a consumer that collates into its own
-        buffers (``pangnn_b200.graphs.GraphedBatchStep.step_ids``)."""
+        buffers (``pangnn_b200.graphs.GraphedBatchStep.step_ids``).
+
+        ``shard=(rank, world)``: this rank's part of the epoch's batch list, which is the same on every rank of a
+        group with the same seed: batches ``rank, rank + world, ...``.  With ``pad`` the list is first padded to a
+        multiple of ``world`` by repeating whole batches from its start (Accelerate's ``even_batches``), so every
+        rank takes the same number of steps."""
         import numpy as np
         order = list(range(self._ids.size))
         if self.shuffle:
             self._rng.shuffle(order)
         order = self._ids[np.asarray(order, dtype=np.int64)] if order else self._ids[:0]
         order_dev = torch.from_numpy(order).to(self.device)
-        for i in range(0, len(order), self.batch_size):
+        starts = list(range(0, len(order), self.batch_size))
+        if shard is not None:
+            rank, world = shard
+            if pad and starts:
+                starts += [starts[i % len(starts)] for i in range(-len(starts) % world)]
+            starts = starts[rank::world]
+        for i in starts:
             yield self.packed, order[i:i + self.batch_size], order_dev[i:i + self.batch_size]
+
 
 
 _PREP_STREAMS = {}

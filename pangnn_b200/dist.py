@@ -92,6 +92,75 @@ class P2P:
 
 
 # ------------------------------------------------------------------------------------------------
+# data-parallel gradient average
+# ------------------------------------------------------------------------------------------------
+class GradReducer:
+    """``reducer()`` replaces every gradient of ``params`` by its mean over the ranks of ``group``: the all-reduce
+    DDP runs behind ``accelerator.backward`` (``pangnn.py:207``) in data-parallel training.  Call it between
+    ``loss.backward()`` and ``optimizer.step()``, eagerly or inside a CUDA-graph capture, the same number of times
+    on every rank.  A gradient that is None stays None.
+
+    The bucket is laid out from ``params``, which must be the same list on every rank (which parameters receive a
+    gradient depends on the flags alone).  Over NVLink peer memory (``P2P``) the reduction is ``ops.grad_push`` +
+    ``ops.grad_reduce``: every rank packs its gradients into its own symmetric bucket and sums every peer's in rank
+    order, so the result is bitwise the same on every rank.  Otherwise (``PANGNN_P2P=0``, no symmetric memory,
+    gloo) it is one flat ``dist.all_reduce`` times ``1 / W``.  In a group of one rank it does nothing."""
+
+    def __init__(self, params, group=None, timeout_s=120.0):
+        self.params, self.group, self.timeout_s = [p for p in params if p.requires_grad], group, float(timeout_s)
+        self.numels = [p.numel() for p in self.params]
+        init = dist.is_available() and dist.is_initialized()
+        self.world = dist.get_world_size(group) if init else 1
+        self.rank = dist.get_rank(group) if init else 0
+        self.scale = float(torch.tensor(1.0 / self.world, dtype=torch.float32))          # fp32(1 / W)
+        self.p2p = None
+        if self.world > 1 and self.params and self.params[0].is_cuda and len(self.params) <= ops.GRAD_REDUCE_MAX_TENSORS \
+                and self.world <= ops.GRAD_REDUCE_MAX_RANKS:
+            self.p2p = P2P.get(group)
+        if self.p2p is not None:
+            dev = self.params[0].device
+            self.half = ops.grad_bucket_floats(self.numels)
+            self.bucket, hb = self.p2p.buffer("grad_bucket", 2, self.half, dev)
+            sig, hs = self.p2p.buffer("grad_signal", 1, ops.GRAD_REDUCE_MAX_RANKS, dev)
+            sig.zero_()
+            self.signal = sig.view(torch.int32)
+            self.ctrl = torch.zeros(4, dtype=torch.int32, device=dev)              # epoch, two tickets, status
+            peers = range(self.world)
+            self.peer_buckets = [self.p2p.peer(hb, p, 2, self.half).data_ptr() if p != self.rank else
+                                 self.bucket.data_ptr() for p in peers]
+            self.peer_signals = [self.p2p.peer(hs, p, 1, ops.GRAD_REDUCE_MAX_RANKS).data_ptr() if p != self.rank else
+                                 sig.data_ptr() for p in peers]
+            hs.barrier()                                        # every rank's zeroed signals before any push
+
+    def __call__(self):
+        if self.world == 1:
+            return
+        grads = [p.grad for p in self.params]
+        if self.p2p is not None:
+            ops.grad_push(grads, self.numels, self.bucket, self.half, self.peer_signals, self.rank, self.ctrl)
+            ops.grad_reduce(grads, self.numels, self.peer_buckets, self.half, self.signal, self.rank, self.ctrl,
+                            self.timeout_s)
+            return
+        flat = torch.cat([(g if g is not None else torch.zeros_like(p)).reshape(-1) for p, g in zip(self.params, grads)])
+        dist.all_reduce(flat, group=self.group)
+        flat.mul_(self.scale)
+        off = 0
+        for g, n in zip(grads, self.numels):
+            if g is not None:
+                g.copy_(flat[off:off + n].view_as(g))
+            off += n
+
+    def check(self):
+        """Raise if a peer-memory reduction gave up waiting (reads the status word: one host synchronisation, so
+        call it where the host waits anyway, e.g. once per epoch)."""
+        if self.p2p is not None:
+            st = int(self.ctrl[3].item())
+            if st:
+                raise RuntimeError(f"rank {self.rank}: the gradient average timed out after {self.timeout_s:g} s "
+                                   f"waiting for rank {st - 1}")
+
+
+# ------------------------------------------------------------------------------------------------
 # halo plans
 # ------------------------------------------------------------------------------------------------
 class HaloPlan:

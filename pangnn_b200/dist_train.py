@@ -33,9 +33,19 @@ def check_partition_flags(args, world):
     """Raise ``ValueError`` when the flags ask for something the partitioned driver at ``world`` ranks cannot do.
     Depends on the flags and ``world`` alone, so every rank refuses alike, before any device work."""
     bad = []
+    if getattr(args, "data_parallel", False):
+        if args.whole_graph_training:
+            bad.append("--data_parallel replicates the model over sub-graph batches and --whole_graph_training "
+                       "partitions the graph: choose one")
+        if not args.train:
+            bad.append("--data_parallel needs --train (inference runs on the genome partition)")
+        if bad:
+            raise ValueError(f"pangnn.py on {world} GPU(s): " + "; ".join(bad))
+        if _trains_replicated(args):
+            return                          # the replicas run the one-GPU model code: every flag of the one-GPU loop
     if world > 1 and args.train and not args.whole_graph_training:
-        bad.append("--train needs --whole_graph_training: the partitioned path trains on the whole graph (the "
-                   "reference's -b sub-graph batches would need data-parallel training)")
+        bad.append("--train needs --whole_graph_training (partition the graph by genome and train on the whole graph) "
+                   "or --data_parallel (replicate the model and shard the reference's -b sub-graph batches)")
     if world > 1 and args.include_trivial and args.simulate_dataset:
         bad.append("--include_trivial with --simulate_dataset joins every genome pair, but a rank generates only "
                    "its own genomes and one on each side")
@@ -54,6 +64,20 @@ def partitioned(args):
     if not (dist.is_available() and dist.is_initialized()):
         return False
     return dist.get_world_size() > 1 or not args.train or args.whole_graph_training
+
+
+def _trains_replicated(args):
+    """``--train --data_parallel`` trains replicas unless ``-m`` names an existing model file, which the reference
+    restores for inference instead (``pangnn.py:125-144``): that inference runs on the genome partition, under its
+    flag checks."""
+    return (bool(getattr(args, "data_parallel", False)) and args.train and not args.whole_graph_training
+            and not os.path.exists(args.model_args))
+
+
+def data_parallel(args):
+    """Whether ``train.run`` takes the data-parallel driver: a default process group is initialised and the flags
+    ask for replicated training (``_trains_replicated``)."""
+    return _trains_replicated(args) and dist.is_available() and dist.is_initialized()
 
 
 @contextlib.contextmanager
@@ -271,3 +295,121 @@ def _outputs(args, pg, stat, t, N, rank, world, edge_table):
     dt = time.perf_counter() - t0
     log.debug(f"outputs written in {dt:.3f} s")
     return dt
+
+
+# ------------------------------------------------------------------------------------------------
+# data-parallel sub-graph training
+# ------------------------------------------------------------------------------------------------
+def run_data_parallel(args, device=None):
+    """``train.run`` with ``--train --data_parallel`` on the ranks of the default process group: DDP under
+    ``accelerate launch`` as the reference has it (``pangnn.py:25,122,155,207``).
+
+    Every rank builds the same dataset and model from ``args.seed`` (the parameters are broadcast from rank 0), takes
+    batches ``rank, rank + W, ...`` of the epoch's ``-b`` sub-graph batch list (padded to a multiple of ``W`` from its
+    start, Accelerate's ``even_batches``; validation unpadded) and averages the gradients over the ranks between
+    backward and the optimizer step (``dist.GradReducer``), eagerly or inside the ``--cuda_graphs`` step.  ``-b`` is
+    the batch per rank; the loss is each rank's own batch mean.  The epoch's statistics are global: one all-reduce of
+    the loss sums, step and batch counts and confusion counts, and the ranking metrics over the group; the scheduler
+    steps on the global validation loss, so the ranks stay identical.  ``--dynamic_binary_threshold`` takes the
+    Youden threshold of each step's ``W`` batches together (the one-GPU loop takes it per batch).  Every rank tests
+    the model; rank 0 logs and writes ``model.pkl`` and the test outputs as ``train.run`` does."""
+    rank, world = dist.get_rank(), dist.get_world_size()
+    check_partition_flags(args, world)
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    with _info_on_rank0(rank):
+        return _run_data_parallel(args, device, rank, world)
+
+
+def _run_data_parallel(args, device, rank, world):
+    from .data import DeviceLoader
+    from .graphs import GraphedBatchStep
+    from .train import build_dataset_and_model, save_test_and_write
+    dataset, model = build_dataset_and_model(args, device)
+    for p in model.parameters():
+        dist.broadcast(p.data, 0)
+    reducer = pdist.GradReducer(list(model.parameters()))
+    pos_weight = float(dataset.class_balance) if dataset.class_balance else 1.0       # pangnn.py:98
+    threshold = args.binary_threshold
+    history = []
+    test = [g.to(device) for g in dataset.test]
+    loader = lambda graphs, seed: (DeviceLoader(graphs, batch_size=args.batch_size, shuffle=True, device=device,
+                                                seed=seed) if graphs else None)
+    train_loader, val_loader = loader(dataset.train, args.seed), loader(dataset.val, args.seed + 1)
+    stepper = None
+    if args.cuda_graphs:
+        optimizer = torch.optim.Adam(model.parameters(), lr=torch.tensor(0.001, device=device), capturable=True)
+        stepper = GraphedBatchStep(model, optimizer, pos_weight, reduce_grads=reducer)
+    else:
+        optimizer = torch.optim.Adam(model.parameters(), lr=0.001)                    # pangnn.py:88
+    scheduler = torch.optim.lr_scheduler.ReduceLROnPlateau(optimizer, mode="min", patience=10, factor=0.6)
+    shard = (rank, world)
+    dist.barrier()                                     # dataset build skew never counts against the reduction's wait
+
+    for epoch in range(args.epochs):                                                  # pangnn.py:167-238
+        t_ep = time.perf_counter()
+        model.train()
+        # [train loss sum, steps, train tn fp fn tp, val tn fp fn tp, val loss sum, val batches]
+        red = torch.zeros(12, dtype=torch.float64, device=device)
+        ep_prob, ep_y = [], []
+        n_batches = len(train_loader) if train_loader is not None else 0
+        for i, (packed, ids, ids_dev) in enumerate(train_loader.iter_ids(shard) if train_loader is not None else ()):
+            if stepper is not None:
+                loss, logits = stepper.step_ids(packed, ids, ids_dev)
+                labels = stepper.last_y.clone()                  # the stepper's labels are static buffers
+            else:
+                batch = packed.collate(ids, ids_dev)
+                optimizer.zero_grad()
+                loss, logits = model.forward_loss(batch, pos_weight)
+                loss.backward()
+                reducer()
+                optimizer.step()
+                labels = batch.y
+            prob = torch.sigmoid(logits.detach())
+            if i * world + rank < n_batches:     # not a repeat of the even-batches padding (Accelerate's
+                red[0] += loss.detach().double()  # gather_for_metrics drops those too): the epoch's statistics
+                red[1] += 1
+                ep_prob.append(prob)
+                ep_y.append(labels)
+                red[2:6] += _counts(prob >= threshold, labels).double()
+            if args.dynamic_binary_threshold:                                         # pangnn.py:229-233
+                # the step's W batches together (a padding repeat included: every rank joins every step's call)
+                th = ranking_metrics(prob, labels)["youden_threshold"]
+                threshold = th if th is not None else threshold
+        t_val = time.perf_counter()
+        model.eval()
+        val_prob, val_y = [], []
+        with torch.no_grad():                                                         # pangnn.py:241-275
+            for batch in (val_loader.batches(shard, pad=False) if val_loader is not None else ()):
+                logits, prob, pred = model.predict(batch, threshold)
+                val_prob.append(prob)
+                val_y.append(batch.y)
+                red[10] += torch.nn.functional.binary_cross_entropy_with_logits(
+                    logits, batch.y, pos_weight=torch.as_tensor(pos_weight, device=logits.device)).double()
+                red[11] += 1
+                red[6:10] += _counts(pred, batch.y).double()
+        dist.all_reduce(red)
+        reducer.check()
+        red = red.tolist()
+        cm, cmv = [int(v) for v in red[2:6]], [int(v) for v in red[6:10]]
+        p, r, f1 = prf(*cm)
+        pv, rv, f1v = prf(*cmv)
+        mean_val = red[10] / max(int(red[11]), 1)
+        scheduler.step(mean_val)                                                      # pangnn.py:296
+        cat = lambda v: torch.cat(v) if v else torch.zeros(0, device=device)
+        rk_tr = ranking_metrics(cat(ep_prob), cat(ep_y))                              # over the default group
+        rk_val = ranking_metrics(cat(val_prob), cat(val_y))
+        history.append(dict(epoch=epoch, train_loss=red[0] / max(int(red[1]), 1), val_loss=mean_val,
+                            f1_train=f1, f1_val=f1v, precision_val=pv, recall_val=rv,
+                            auroc_train=rk_tr["auroc"], ap_train=rk_tr["average_precision"],
+                            auroc_val=rk_val["auroc"], ap_val=rk_val["average_precision"]))
+        log.info(f"epoch {epoch}: train loss {history[-1]['train_loss']:.4f} f1 {f1:.4f} | val loss {mean_val:.4f} f1 {f1v:.4f}")
+        log.info(f"epoch {epoch}: train auroc {_fmt(rk_tr['auroc'])} ap {_fmt(rk_tr['average_precision'])} | "
+                 f"val auroc {_fmt(rk_val['auroc'])} ap {_fmt(rk_val['average_precision'])}")
+        log.debug(f"epoch {epoch}: train steps {time.perf_counter() - t_ep:.3f} s ({int(red[1])} over {world} ranks)")
+
+    # every replica tests its own identical copy of the test graphs: their metrics must not merge over the group (and
+    # rank 0's curve files must not wait for the others), so they go through a group of this rank alone
+    solo = [dist.new_group([r]) for r in range(world)][rank]
+    stats, path = save_test_and_write(args, model, dataset, test, threshold, pos_weight, write=rank == 0, group=solo)
+    dist.barrier()                                     # rank 0's files are complete when every rank returns
+    return dict(model=model, dataset=dataset, history=history, test=stats, model_path=path)

@@ -58,14 +58,20 @@ class GraphedBatchStep:
     graphs (a scheduler that replaces ``param_group['lr']`` is not seen by them).  Batches whose edge lists exceed the
     single-launch CSR build (4096 edges) fall back to the eager step.
 
+    ``reduce_grads`` (data-parallel training, ``dist.GradReducer``) runs between ``loss.backward()`` and
+    ``opt.step()`` of the eager step and of the captured graph, never in the capture's warm-up: ranks capture their
+    buckets at different times, and a collective there would put their reductions out of step.
+
         stepper = GraphedBatchStep(model, optimizer, dataset.class_balance)
         for batch in DeviceLoader(dataset.train, batch_size=32, ...):
             loss, logits = stepper(batch)
     """
 
-    def __init__(self, model, optimizer, pos_weight, node_quantum=64, edge_quantum=128, max_buckets=128):
+    def __init__(self, model, optimizer, pos_weight, node_quantum=64, edge_quantum=128, max_buckets=128,
+                 reduce_grads=None):
         from . import ops
         self.model, self.opt, self.pw = model, optimizer, float(pos_weight)
+        self.reduce_grads = reduce_grads
         self.nq, self.eq, self.max_buckets = int(node_quantum), int(edge_quantum), int(max_buckets)
         self.buckets = {}
         self.stats = {"captures": 0, "replays": 0, "eager": 0}
@@ -167,6 +173,8 @@ class GraphedBatchStep:
             self.opt.zero_grad(set_to_none=True)
             loss, logits = self._loss(g)
             loss.backward()
+            if self.reduce_grads is not None:
+                self.reduce_grads()
             self.opt.step()
         torch.cuda.current_stream().wait_stream(side)
         ops.clear_cache()
@@ -177,6 +185,8 @@ class GraphedBatchStep:
         self.opt.zero_grad(set_to_none=True)
         loss, logits = self.model.forward_loss(batch, self.pw)
         loss.backward()
+        if self.reduce_grads is not None:
+            self.reduce_grads()
         self.opt.step()
         self.stats["eager"] += 1
         return loss.detach(), logits

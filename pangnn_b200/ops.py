@@ -1171,6 +1171,54 @@ def rows_scatter_add(src, idx, dst):
     LAUNCHES["count"] += 1
 
 
+# ------------------------------------------------------------------------------------------------
+# data-parallel gradient average over peer memory (csrc/grad_reduce.cu)
+# ------------------------------------------------------------------------------------------------
+GRAD_REDUCE_MAX_TENSORS, GRAD_REDUCE_MAX_RANKS = 32, 8
+
+
+def _ptr_array(ptrs):
+    arr = (C.c_void_p * max(len(ptrs), 1))(*ptrs)
+    return arr, C.cast(arr, C.c_void_p)
+
+
+def _grad_table(grads, numels):
+    """(keep-alive, grads**, numels*) host tables: ``grads`` are fp32 dense CUDA tensors or None (NULL)."""
+    for g in grads:
+        if g is not None and (not g.is_cuda or g.dtype != torch.float32 or not g.is_contiguous()):
+            raise _abi.PangnnError("grad_push / grad_reduce need dense fp32 CUDA gradients")
+    gp = _ptr_array([g.data_ptr() if g is not None else None for g in grads])
+    nn = (C.c_int64 * max(len(numels), 1))(*[int(n) for n in numels])
+    return (gp[0], nn), gp[1], C.cast(nn, C.c_void_p)
+
+
+def grad_bucket_floats(numels):
+    """Floats one bucket half needs for tensors of ``numels`` elements (each tensor starts on a 4-float boundary)."""
+    nn = (C.c_int64 * max(len(numels), 1))(*[int(n) for n in numels])
+    return int(_abi.load().pangnn_grad_bucket_floats(C.cast(nn, C.c_void_p), len(numels)))
+
+
+def grad_push(grads, numels, bucket, half_floats, peer_signals, rank, ctrl):
+    """Pack ``grads`` into half ``ctrl[0] & 1`` of ``bucket`` (this rank's, 2 * ``half_floats`` floats) and signal
+    ``ctrl[0] + 1`` into slot ``rank`` of every ``peer_signals`` array (data pointers, one per rank, in rank order)."""
+    keep, gp, nn = _grad_table(grads, numels)
+    sig_keep, sp = _ptr_array(list(peer_signals))
+    _abi.check(_abi.load().pangnn_grad_push(gp, nn, len(grads), _p(bucket), int(half_floats), sp, len(peer_signals),
+                                            int(rank), _p(ctrl), _stream()), "grad_push")
+    LAUNCHES["count"] += 1
+
+
+def grad_reduce(grads, numels, peer_buckets, half_floats, signal, rank, ctrl, timeout_s=120.0):
+    """Wait for every rank's signal of this call, then ``grads = (b_0 + ... + b_{W-1}) * fp32(1 / W)`` in rank order
+    over half ``ctrl[0] & 1`` of the ``peer_buckets`` (data pointers, in rank order); None entries are skipped.  A wait
+    longer than ``timeout_s`` leaves ``1 + rank of the missing peer`` in ``ctrl[3]`` instead."""
+    keep, gp, nn = _grad_table(grads, numels)
+    buck_keep, bp = _ptr_array(list(peer_buckets))
+    _abi.check(_abi.load().pangnn_grad_reduce(gp, nn, len(grads), bp, int(half_floats), _p(signal), len(peer_buckets),
+                                              int(rank), _p(ctrl), int(timeout_s * 1e9), _stream()), "grad_reduce")
+    LAUNCHES["count"] += 1
+
+
 def neighbour_band(num_nodes, n, device="cuda", out=None):
     """Whole-graph neighbour band ``[2, Eb]`` int64 (``src/dataset.py:351-366``) from one closed-form
     kernel, no host sync.  ``out`` = ``(src_row, dst_row)`` writes into existing int64 storage (the tail of

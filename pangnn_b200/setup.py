@@ -55,6 +55,9 @@ def build_parser():
                         "(pangnn_b200.graphs.GraphedBatchStep; batches over 4096 edges per list stay eager)")
     p.add_argument("--whole_graph_training", action="store_true",
                    help="train on the whole graph as one batch instead of per-group sub-graphs")
+    p.add_argument("--data_parallel", action="store_true",
+                   help="(new) with --train under torchrun: replicate the model, shard the sub-graph batches, average "
+                        "gradients each step (pangnn_b200.dist_train.run_data_parallel)")
     p.add_argument("--seed", default=0, type=int)
     return p
 

@@ -62,9 +62,10 @@ def youden_threshold(prob, labels):
     return float(p[last][best]) if float(j[best]) > 0 else None
 
 
-def evaluate(model, graphs, threshold, pos_weight=None):
+def evaluate(model, graphs, threshold, pos_weight=None, group=None):
     """Whole-batch inference as ``src/predict.py:29-55``: logits, sigmoid, threshold, confusion; plus the ROC AUC, AP
-    and Youden threshold of the probabilities (``src/plot.py:103-107,131``; exact, ``metrics.ranking_metrics``)."""
+    and Youden threshold of the probabilities (``src/plot.py:103-107,131``; exact, ``metrics.ranking_metrics`` over
+    ``group``: pass a group of one rank for a replica's own graphs while a default process group exists)."""
     model.eval()
     out = []
     for g in graphs:
@@ -72,7 +73,7 @@ def evaluate(model, graphs, threshold, pos_weight=None):
         tn, fp, fn, tp = confusion(pred, g.y)
         p, r, f1 = prf(tn, fp, fn, tp, eps=0.0)
         rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=p, recall=r, f1=f1, logits=logits, prob=prob, pred=pred)
-        rk = ranking_metrics(prob, g.y)
+        rk = ranking_metrics(prob, g.y, group)
         rec.update(auroc=rk["auroc"], average_precision=rk["average_precision"],
                    youden_threshold=rk["youden_threshold"])
         if pos_weight is not None:
@@ -145,14 +146,14 @@ def write_groups(dataset, graph, stat, out_dir):
     return path
 
 
-def write_curves(graph, stat, out_dir):
+def write_curves(graph, stat, out_dir, group=None):
     """``roc_curve.csv`` (threshold,fpr,tpr) and ``precision_recall_curve.csv`` (threshold,precision,recall; the final
     (1, 0) point has no threshold) of the test probabilities, thinned as sklearn's ``drop_intermediate=True``: the
     data of the reference's ROC and PR figures (``src/plot.py:103-107,131``).  Floats are written round-trip exact."""
-    roc = roc_curve(stat["prob"], graph.y)
+    roc = roc_curve(stat["prob"], graph.y, group)
     if roc is None:
         return None
-    return write_curve_files(roc, precision_recall_curve(stat["prob"], graph.y, drop_intermediate=True), out_dir)
+    return write_curve_files(roc, precision_recall_curve(stat["prob"], graph.y, group, drop_intermediate=True), out_dir)
 
 
 def write_curve_files(roc, pr, out_dir):
@@ -192,22 +193,15 @@ def run(args, device=None):
 
     With a default process group initialised (``main`` under ``torchrun``) every rank runs the genome-partitioned
     driver, ``pangnn_b200.dist_train.run_partitioned``; in a group of one rank the reference's sub-graph training
-    (``--train`` without ``--whole_graph_training``) has nothing to partition and runs the loop below."""
+    (``--train`` without ``--whole_graph_training``) has nothing to partition and runs the loop below.  With
+    ``--train --data_parallel`` in a group, every rank runs ``dist_train.run_data_parallel`` instead."""
     from . import dist_train
+    if dist_train.data_parallel(args):
+        return dist_train.run_data_parallel(args, device)
     if dist_train.partitioned(args):
         return dist_train.run_partitioned(args, device)
     device = torch.device(device if device is not None else "cuda")
-    torch.manual_seed(args.seed)
-    t0 = time.time()
-    if args.simulate_dataset:
-        log.info("Simulating dataset.")
-        dataset = UnionGraphDataset(calculate_baseline=True, split=(0.7, 0.15, 0.01),
-                                    categorical_nodes=args.categorical_node, device=device)
-    else:
-        dataset = UnionGraphDataset(args.annotation, args.similarity, args.ribap_groups, split=(0.7, 0.15, 0.01),
-                                    categorical_nodes=args.categorical_node, calculate_baseline=True, device=device)
-    log.info(f"Dataset: {dataset.num_genes} genes, class balance {dataset.class_balance}, built in {time.time() - t0:.1f} s")
-    model = AlternateGCN(device, dataset, dataset.categorical_nodes, dims=[args.node_dim, args.hidden_dim]).to(device)
+    dataset, model = build_dataset_and_model(args, device)
     optimizer = torch.optim.Adam(model.parameters(), lr=0.001)                        # pangnn.py:88
     scheduler = torch.optim.lr_scheduler.ReduceLROnPlateau(optimizer, mode="min", patience=10, factor=0.6)
     pos_weight = float(dataset.class_balance) if dataset.class_balance else 1.0       # pangnn.py:98
@@ -297,27 +291,53 @@ def run(args, device=None):
         log.info(f"epoch {epoch}: train auroc {_fmt(rk_tr['auroc'])} ap {_fmt(rk_tr['average_precision'])} | "
                  f"val auroc {_fmt(rk_val['auroc'])} ap {_fmt(rk_val['average_precision'])}")
 
-    os.makedirs(args.output, exist_ok=True)
+    stats, path = save_test_and_write(args, model, dataset, test, threshold, pos_weight)
+    return dict(model=model, dataset=dataset, history=history, test=stats, model_path=path)
+
+
+def build_dataset_and_model(args, device):
+    """The dataset (simulated or read) and the freshly initialised model of ``run``, from ``args.seed``."""
+    torch.manual_seed(args.seed)
+    t0 = time.time()
+    if args.simulate_dataset:
+        log.info("Simulating dataset.")
+        dataset = UnionGraphDataset(calculate_baseline=True, split=(0.7, 0.15, 0.01),
+                                    categorical_nodes=args.categorical_node, device=device)
+    else:
+        dataset = UnionGraphDataset(args.annotation, args.similarity, args.ribap_groups, split=(0.7, 0.15, 0.01),
+                                    categorical_nodes=args.categorical_node, calculate_baseline=True, device=device)
+    log.info(f"Dataset: {dataset.num_genes} genes, class balance {dataset.class_balance}, built in {time.time() - t0:.1f} s")
+    model = AlternateGCN(device, dataset, dataset.categorical_nodes, dims=[args.node_dim, args.hidden_dim]).to(device)
+    return dataset, model
+
+
+def save_test_and_write(args, model, dataset, test, threshold, pos_weight, write=True, group=None):
+    """The end of a training run: save ``model.pkl``, test, and write the test outputs.  ``write=False`` (every rank
+    of a data-parallel run but the first) tests without saving or writing; ``group`` as in ``evaluate``.
+    -> (test stats, model path)."""
     path = os.path.join(args.output, os.path.basename(args.model_args))
-    torch.save(model.state_dict(), path)                                              # pangnn.py:339-341
-    log.info(f"Saved model parameters to '{path}'")
-    stats = evaluate(model, test, threshold, pos_weight)                              # pangnn.py:344-346
+    if write:
+        os.makedirs(args.output, exist_ok=True)
+        torch.save(model.state_dict(), path)                                          # pangnn.py:339-341
+        log.info(f"Saved model parameters to '{path}'")
+    stats = evaluate(model, test, threshold, pos_weight, group)                       # pangnn.py:344-346
     for s in stats:
         log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f}")
     log_ranking(stats)
     if stats:
         add_baselines(dataset, test[0], stats[0])
-        write_groups(dataset, test[0], stats[0], args.output)
-        write_curves(test[0], stats[0], args.output)                                  # src/plot.py:103-107,131
-        if args.simulate_dataset:                                                     # src/predict.py:84: not args.train or simulate
-            write_edge_table(dataset, test[0], stats[0], args.output)
-    return dict(model=model, dataset=dataset, history=history, test=stats, model_path=path)
+        if write:
+            write_groups(dataset, test[0], stats[0], args.output)
+            write_curves(test[0], stats[0], args.output, group)                       # src/plot.py:103-107,131
+            if args.simulate_dataset:                                                 # src/predict.py:84: not args.train or simulate
+                write_edge_table(dataset, test[0], stats[0], args.output)
+    return stats, path
 
 
 def main(argv=None):
     """``pangnn.py``.  Under ``torchrun --nproc-per-node N`` (``WORLD_SIZE`` > 1) each process joins an NCCL group
-    from the environment on the GPU ``LOCAL_RANK`` and runs the genome-partitioned driver; the group is destroyed on
-    exit, also on an error."""
+    from the environment on the GPU ``LOCAL_RANK`` and runs the genome-partitioned driver (the data-parallel one with
+    ``--train --data_parallel``); the group is destroyed on exit, also on an error."""
     args = setup.parse(argv)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world <= 1:
