@@ -89,7 +89,8 @@ class UnionGraphDataset:
         # ---- device: sort / dedupe / trivial filter / softmax + Q-score / labels  (a1-a7)
         src, dst, w, y = pp.normalize_sim_scores(*self.raw_hits, self.genome_of, self.group_of,
                                                  num_nodes=self.num_genes, device=self.device)
-        self.sim_edges = (src, dst, w, y)
+        # without a RIBAP table the normalisation writes zeros for y: they are not labels and go no further
+        self.sim_edges = (src, dst, w, y if has_labels else None)
         self.has_labels = has_labels
 
         if args.train:
@@ -104,15 +105,15 @@ class UnionGraphDataset:
     def generate_graphs(self):
         """Whole graph (``src/dataset.py:325-395``): sim edges + Q-score weights + labels, the
         +-n neighbour band (self loops, crossing genome seams), optional union assembly
-        ``[sim ; nb]`` with weights ``[w ; 1...]``."""
+        ``[sim ; nb]`` with weights ``[w ; 1...]``.  Without labels (no RIBAP table; the reference crashes at
+        ``src/dataset.py:345``) the graph is the same with ``y = None`` and ``class_balance`` stays None."""
         src, dst, w, y = self.sim_edges
         dev = self.device
         N, n = self.num_genes, args.neighbours
         edge_index = torch.stack((src.long(), dst.long()))
-        if not self.has_labels:
-            raise ValueError("the reference's whole-graph path requires labels (src/dataset.py:345)")
-        pos = y.sum()
-        self.class_balance = ((y == 0).sum() / pos).item()                       # src/dataset.py:346
+        if y is not None:
+            pos = y.sum()
+            self.class_balance = ((y == 0).sum() / pos).item()                   # src/dataset.py:346
         x = torch.ones(N, device=dev) if self.categorical_nodes else torch.ones(N, 1, device=dev)
         if args.union_edge_weights:
             union = ops.union_index(edge_index, N, n)                            # band written into the tail
@@ -156,6 +157,8 @@ class UnionGraphDataset:
         ``get_neighbour_graph`` of ``src/helper.py:327-417``), all groups at once on the device
         (``pangnn_b200.subgraphs.extract``).  -> (list-of-graphs view over the packed arena, class balance)."""
         src, dst, w, y = self.sim_edges
+        if y is None:
+            raise ValueError("training sub-graphs need labels: name the RIBAP groups table with -r")
         arena = subgraphs.extract(src, dst, w, y, self.num_genes, args.neighbours, groups,
                                   union=bool(args.union_edge_weights), gff_is_subset=self.gff_is_subset,
                                   chunks=args.cpus)

@@ -474,7 +474,8 @@ class LocalGraph:
 
 class PartitionedGraph:
     """What ``DistModel`` consumes: the local pieces of the whole-graph ``Data`` object.
-    All edge lists are in GLOBAL ids and may be supersets of what the rank needs."""
+    All edge lists are in GLOBAL ids and may be supersets of what the rank needs.  ``y`` may be None (a graph without
+    labels, for inference only): ``self.y`` and ``class_balance`` are then None."""
 
     def __init__(self, bounds, rank, world, x_own, conv_ei, conv_w, nb_ei, scored_ei, scored_w, y,
                  group=None):
@@ -486,15 +487,15 @@ class PartitionedGraph:
         self.nb = LocalGraph(nb_ei, *b, anchor="dst", group=group) if nb_ei is not None else None
         self.scored = LocalGraph(scored_ei, *b, anchor="src", group=group)
         m = self.scored.edge_mask
-        self.y = self.pick(y)
+        self.y = self.pick(y) if y is not None else None
         self.skip = self.pick(scored_w).float() if args.skip_connections else None
         self.scored_edge_ids = self.pick(torch.arange(m.numel(), device=m.device))
-        cnt = torch.tensor([float(self.y.numel()), float(self.y.sum().item())], dtype=torch.float64,
-                           device=self.y.device)
+        pos = float(self.y.sum().item()) if self.y is not None else 0.0
+        cnt = torch.tensor([float(self.scored_edge_ids.numel()), pos], dtype=torch.float64, device=m.device)
         if world > 1:
             dist.all_reduce(cnt, group=group)
         self.num_edges_total = int(cnt[0].item())
-        self.class_balance = float((cnt[0] - cnt[1]) / cnt[1])                    # src/dataset.py:346
+        self.class_balance = float((cnt[0] - cnt[1]) / cnt[1]) if self.y is not None else None   # src/dataset.py:346
 
     def pick(self, t):
         """Per-edge tensor of the scored list given to the constructor -> the rows of this rank's scored edges, in
@@ -558,7 +559,7 @@ class PartitionedGraph:
             setattr(pg, name, new)
         for ev in ready.values():
             main.wait_event(ev)
-        pg.x, pg.y, pg.skip = d["x"], d["y"], d.get("skip")
+        pg.x, pg.y, pg.skip = d["x"], d.get("y"), d.get("skip")
         return pg
 
     def prefetch_from(self, host, device, consumer=None):
@@ -767,7 +768,7 @@ class DistModel:
             # A.6: one embedding row per gene, indexed by GLOBAL position (rows of other ranks get
             # zero gradient here; the flat all-reduce sums the disjoint row blocks)
             lo = pg.bounds[pg.rank]
-            x = m.embedding(torch.arange(lo, lo + pg.n_own, device=pg.y.device))
+            x = m.embedding(torch.arange(lo, lo + pg.n_own, device=pg.x.device))
         elif (pg.x.dim() == 2 and pg.x.size(1) == 1 and getattr(m, "fuse_embedding", True)
               and m.conv_in.out_channels % 4 == 0 and m.conv_in.out_channels <= 256):
             x = None                                                   # Linear(1, D) + conv_in folded (rank1.cu)
@@ -823,18 +824,31 @@ class DistModel:
                                           1.0 / max(pg.num_edges_total, 1), dpq_out, unit_grad)
 
     @torch.no_grad()
+    def predict(self, pg, threshold):
+        """This rank's ``(logits, prob, pred)`` of the edges ``pg.scored_edge_ids``: sigmoid and threshold fused into
+        the scorer kernel, as ``AlternateGCN.predict``.  Reads no labels."""
+        next_step()
+        pq_ext, weights, _ = self._scorer_inputs(pg, self.embed(pg))
+        return ops.edge_score_predict(pq_ext, *weights, pg.scored.gs, pg.skip, threshold)
+
+    @torch.no_grad()
     def evaluate(self, pg, threshold, pos_weight=None):
         """Test statistics of the whole partitioned graph, identical on every rank (``train.evaluate`` of the global
         graph, ``src/predict.py:29-55``): global confusion matrix (one all-reduce of four counts), precision /
         recall / F1 with ``eps=0``, the global mean BCE loss when ``pos_weight`` is given, and the exact global
         ranking metrics of the probabilities (``metrics.ranking_metrics`` over the group).  Also returns this
-        rank's ``logits`` / ``prob`` / ``pred`` (edges ``pg.scored_edge_ids``)."""
+        rank's ``logits`` / ``prob`` / ``pred`` (edges ``pg.scored_edge_ids``).  A graph without labels (``pg.y``
+        None) gets those and ``predicted_positive``, the global number of edges predicted positive, alone."""
         from .metrics import ranking_metrics
         from .train import prf
-        next_step()
-        pq_ext, weights, _ = self._scorer_inputs(pg, self.embed(pg))
-        logits, prob, pred = ops.edge_score_predict(pq_ext, *weights, pg.scored.gs, pg.skip, threshold)
+        logits, prob, pred = self.predict(pg, threshold)
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         y = pg.y
+        if y is None:
+            k = pred.sum(dtype=torch.int64)
+            if world > 1:
+                dist.all_reduce(k, group=self.group)
+            return dict(logits=logits, prob=prob, pred=pred, predicted_positive=int(k))
         p, yl = pred.long(), y.long()
         tp = (p * yl).sum()
         fp = (p * (1 - yl)).sum()
@@ -844,7 +858,6 @@ class DistModel:
         if pos_weight is not None:
             loss_sum = torch.nn.functional.binary_cross_entropy_with_logits(
                 logits, y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device), reduction="sum")
-        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         if world > 1:
             dist.all_reduce(cnt, group=self.group)
             if loss_sum is not None:

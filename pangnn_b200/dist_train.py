@@ -25,13 +25,14 @@ from . import preprocessing as pp
 from .dataset import UnionGraphDataset
 from .gnn import AlternateGCN
 from .metrics import precision_recall_curve, ranking_metrics, roc_curve
-from .setup import log
-from .train import _fmt, log_ranking, prf, write_curve_files
+from .setup import check_label_flags, log
+from .train import _fmt, log_test, prf, write_curve_files
 
 
 def check_partition_flags(args, world):
     """Raise ``ValueError`` when the flags ask for something the partitioned driver at ``world`` ranks cannot do.
     Depends on the flags and ``world`` alone, so every rank refuses alike, before any device work."""
+    check_label_flags(args)
     bad = []
     if getattr(args, "data_parallel", False):
         if args.whole_graph_training:
@@ -167,8 +168,7 @@ def _run(args, device, rank, world):
             log.info(f"Found model file '{args.model_args}' with trained parameters, restoring model state for inference..")
             model.load_state_dict(torch.load(args.model_args, map_location=device))
         stat = _test(dm, pg, threshold, pos_weight, tables)
-        log.info(f"test: f1 {stat['f1']:.4f} precision {stat['precision']:.4f} recall {stat['recall']:.4f} loss {stat['loss']:.4f}")
-        log_ranking([stat])
+        log_test([stat], loss=True)
         timings["outputs_s"] = _outputs(args, pg, stat, tables, N, rank, world, edge_table=True)
         return dict(model=model, dataset=dataset, history=history, test=[stat], graph=pg, timings=timings)
 
@@ -214,8 +214,7 @@ def _run(args, device, rank, world):
         torch.save(sd, path)                                                          # pangnn.py:339-341
     log.info(f"Saved model parameters to '{path}'")
     stat = _test(dm, pg, threshold, pos_weight, tables)                               # pangnn.py:344-346
-    log.info(f"test: f1 {stat['f1']:.4f} precision {stat['precision']:.4f} recall {stat['recall']:.4f}")
-    log_ranking([stat])
+    log_test([stat])
     timings["outputs_s"] = _outputs(args, pg, stat, tables, N, rank, world, edge_table=bool(args.simulate_dataset))
     return dict(model=model, dataset=dataset, history=history, test=[stat], model_path=path, graph=pg, timings=timings)
 
@@ -228,12 +227,14 @@ def _test(dm, pg, threshold, pos_weight, tables):
 
 def _outputs(args, pg, stat, t, N, rank, world, edge_table):
     """The one-GPU CLI's test outputs (``train.add_baselines``, ``write_groups``, ``write_curves``,
-    ``write_edge_table``) for the whole partitioned graph.  -> seconds spent."""
+    ``write_edge_table``) for the whole partitioned graph.  Without labels (``pg.y`` None) the baselines are not scored,
+    no curves are written and the table's ``homolog`` column is -1.  -> seconds spent."""
     t0 = time.perf_counter()
-    dev = pg.y.device
+    dev = stat["logits"].device
     genome_d = torch.as_tensor(t["genome_of"], device=dev)
     order = torch.argsort(t["gid"])                           # the rank's rows in global (src, dst) order
-    src, dst, y = t["src"][order], t["dst"][order], pg.y[order]
+    src, dst = t["src"][order], t["dst"][order]
+    y = pg.y[order] if pg.y is not None else None
     logits = stat["logits"][order]
     q_base = (t["q_base"][order] if t["q_base"] is not None else pp.baseline_labels(src, dst, t["w"][order], genome_d))
     raw_base = (t["raw_base"][order] if t["raw_base"] is not None else
@@ -242,14 +243,15 @@ def _outputs(args, pg, stat, t, N, rank, world, edge_table):
     stat["logit_baseline"] = torch.empty_like(logit_base).index_copy_(0, order, logit_base)
 
     # baselines line: precision / recall / F1 from the all-reduced confusion counts (src/predict.py:77-89)
-    cand = {"base_labels": q_base, "base_labels_raw": raw_base, "logit_baseline": logit_base}
-    cnt = torch.stack([_counts(v, y) for v in cand.values()])
-    if world > 1:
-        dist.all_reduce(cnt)
-    out = {k: prf(*c, eps=0.0) for k, c in zip(cand, cnt.tolist())} if pg.num_edges_total else {}
-    stat["baselines"] = out
-    log.info("baselines (precision / recall / f1): " +
-             "; ".join(f"{k} {p:.4f} / {r:.4f} / {f:.4f}" for k, (p, r, f) in out.items()))
+    if y is not None:
+        cand = {"base_labels": q_base, "base_labels_raw": raw_base, "logit_baseline": logit_base}
+        cnt = torch.stack([_counts(v, y) for v in cand.values()])
+        if world > 1:
+            dist.all_reduce(cnt)
+        out = {k: prf(*c, eps=0.0) for k, c in zip(cand, cnt.tolist())} if pg.num_edges_total else {}
+        stat["baselines"] = out
+        log.info("baselines (precision / recall / f1): " +
+                 "; ".join(f"{k} {p:.4f} / {r:.4f} / {f:.4f}" for k, (p, r, f) in out.items()))
 
     # ortholog groups: the predicted-positive edges in global ids, gathered on rank 0 (counts, then one padded
     # gather), and the one-GPU connected components there
@@ -275,7 +277,7 @@ def _outputs(args, pg, stat, t, N, rank, world, edge_table):
         log.info(f"Wrote {len(groups)} ortholog groups to '{path}'")
 
     # ROC and precision-recall curves over the group, written by rank 0 (src/plot.py:103-107,131)
-    roc = roc_curve(stat["prob"], pg.y)
+    roc = roc_curve(stat["prob"], pg.y) if pg.y is not None else None
     if roc is not None:
         pr = precision_recall_curve(stat["prob"], pg.y, drop_intermediate=True)
         if rank == 0:

@@ -47,7 +47,8 @@ def write_q_score_vs_logit(edge_index, edge_attr, logits, labels, gene_lst=None,
     one row per SCORED edge, keyed by (source, target), with the input Q-score (``edge_attr[:E]`` — the literal
     slice of ``src/plot.py:456``), the output logit, the label and the three max-candidate baselines.  Same
     columns, order, dtypes (score / logit float64, homolog int64) and text format as ``DataFrame.to_csv(index=False)``.
-    Tensors may live on the device; one D2H copy per column, rows formatted by pandas' C writer.
+    Tensors may live on the device; one D2H copy per column, rows formatted by pandas' C writer.  A column passed as
+    None is written as -1 on every row: an absent baseline, or ``labels`` of a run without labels (``-r ''``).
 
     A table can be written in consecutive pieces: the first call with ``header=True``, the others with
     ``header=False, append=True``; the file is byte for byte the one a single call on the whole table writes."""
@@ -70,7 +71,8 @@ def write_q_score_vs_logit(edge_index, edge_attr, logits, labels, gene_lst=None,
         cols["source_str_id"], cols["target_str_id"] = src.astype(str), dst.astype(str)
     cols["score"] = host(edge_attr, np.float32)[:E].astype(np.float64)     # float32 values widened, as .tolist() does
     cols["logit"] = host(logits, np.float32).astype(np.float64)
-    cols["homolog"] = host(labels, np.float32)[:E].astype(np.int64)
+    cols["homolog"] = (host(labels, np.float32)[:E].astype(np.int64) if labels is not None
+                       else np.full(E, -1, dtype=np.int64))
     for name, v in (("q_score_baseline", base_labels), ("raw_baseline", base_labels_raw), ("logit_baseline", logit_baseline)):
         cols[name] = host(v, np.int64) if v is not None else np.full(E, -1, dtype=np.int64)
     os.makedirs(os.path.dirname(path) or ".", exist_ok=True)

@@ -84,6 +84,19 @@ def inert_flags(ns):
     return [k for k, default in _INERT.items() if getattr(ns, k, default) != default]
 
 
+def has_labels(ns):
+    """Whether the run's edges have labels: simulated data always has them; with input files ``-r ''`` names no RIBAP
+    table, for inference on genomes whose ortholog groups are not known yet."""
+    return bool(ns.simulate_dataset) or bool(ns.ribap_groups)
+
+
+def check_label_flags(ns):
+    """Raise ``ValueError`` when the flags ask for training without labels.  Depends on the flags alone, so every rank
+    of a multi-GPU run refuses alike, before any device work."""
+    if ns.train and not has_labels(ns):
+        raise ValueError("--train needs labels: name the RIBAP groups table with -r (-r '' runs inference only)")
+
+
 def parse(argv=None):
     """Parse ``argv`` INTO the module-global ``args`` (so every importer sees the same object)."""
     ns = _post(parser.parse_args(argv))

@@ -65,11 +65,16 @@ def youden_threshold(prob, labels):
 def evaluate(model, graphs, threshold, pos_weight=None, group=None):
     """Whole-batch inference as ``src/predict.py:29-55``: logits, sigmoid, threshold, confusion; plus the ROC AUC, AP
     and Youden threshold of the probabilities (``src/plot.py:103-107,131``; exact, ``metrics.ranking_metrics`` over
-    ``group``: pass a group of one rank for a replica's own graphs while a default process group exists)."""
+    ``group``: pass a group of one rank for a replica's own graphs while a default process group exists).  A graph
+    without labels (``y`` None) gets its ``logits`` / ``prob`` / ``pred`` and ``predicted_positive``, the number of
+    edges predicted positive, alone."""
     model.eval()
     out = []
     for g in graphs:
         logits, prob, pred = model.predict(g, threshold)
+        if g.y is None:
+            out.append(dict(logits=logits, prob=prob, pred=pred, predicted_positive=int(pred.sum())))
+            continue
         tn, fp, fn, tp = confusion(pred, g.y)
         p, r, f1 = prf(tn, fp, fn, tp, eps=0.0)
         rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=p, recall=r, f1=f1, logits=logits, prob=prob, pred=pred)
@@ -93,6 +98,19 @@ def log_ranking(stats):
                  f"youden threshold {_fmt(s['youden_threshold'])}")
 
 
+def log_test(stats, loss=False):
+    """The test lines of the log: F1, precision, recall (and the loss), then the ranking metrics.  A graph without
+    labels has one line instead, with its predicted-positive count."""
+    for s in stats:
+        if "f1" not in s:
+            log.info(f"test: {s['predicted_positive']} scored edges predicted positive; no labels given (-r ''), so "
+                     f"the confusion matrix, loss, ranking metrics and curves are skipped")
+            continue
+        log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f}" +
+                 (f" loss {s.get('loss', float('nan')):.4f}" if loss else ""))
+    log_ranking([s for s in stats if "f1" in s])
+
+
 def _whole_graph(dataset, graph):
     return getattr(graph, "node_id", None) is None or graph.node_id.numel() == dataset.num_genes
 
@@ -109,11 +127,15 @@ def _logit_baseline(dataset, graph, stat):
 
 def add_baselines(dataset, graph, stat):
     """Precision / recall / F1 of the max-candidate baselines next to the model's (``src/predict.py:77-89``):
-    ``stat["baselines"] = {name: (p, r, f1)}`` for the whole test graph (a sub-graph batch has no baseline)."""
+    ``stat["baselines"] = {name: (p, r, f1)}`` for the whole test graph (a sub-graph batch has no baseline).  Without
+    labels only the logit baseline is computed, for the per-edge table, and nothing is scored."""
     if not _whole_graph(dataset, graph):
         return None
+    logit_base = _logit_baseline(dataset, graph, stat)
+    if graph.y is None:
+        return None
     cand = {"base_labels": dataset.base_labels, "base_labels_raw": dataset.base_labels_raw,
-            "logit_baseline": _logit_baseline(dataset, graph, stat)}
+            "logit_baseline": logit_base}
     out = {}
     for name, lab in cand.items():
         if lab is None or len(lab) == 0:
@@ -149,7 +171,10 @@ def write_groups(dataset, graph, stat, out_dir):
 def write_curves(graph, stat, out_dir, group=None):
     """``roc_curve.csv`` (threshold,fpr,tpr) and ``precision_recall_curve.csv`` (threshold,precision,recall; the final
     (1, 0) point has no threshold) of the test probabilities, thinned as sklearn's ``drop_intermediate=True``: the
-    data of the reference's ROC and PR figures (``src/plot.py:103-107,131``).  Floats are written round-trip exact."""
+    data of the reference's ROC and PR figures (``src/plot.py:103-107,131``).  Floats are written round-trip exact.
+    A graph without labels has no curves: nothing is written."""
+    if graph.y is None:
+        return None
     roc = roc_curve(stat["prob"], graph.y, group)
     if roc is None:
         return None
@@ -194,8 +219,12 @@ def run(args, device=None):
     With a default process group initialised (``main`` under ``torchrun``) every rank runs the genome-partitioned
     driver, ``pangnn_b200.dist_train.run_partitioned``; in a group of one rank the reference's sub-graph training
     (``--train`` without ``--whole_graph_training``) has nothing to partition and runs the loop below.  With
-    ``--train --data_parallel`` in a group, every rank runs ``dist_train.run_data_parallel`` instead."""
+    ``--train --data_parallel`` in a group, every rank runs ``dist_train.run_data_parallel`` instead.
+
+    With input files and ``-r ''`` the graph has no labels: the inference branch writes the groups and the per-edge
+    table (``homolog`` -1), and ``--train`` is refused."""
     from . import dist_train
+    setup.check_label_flags(args)
     if dist_train.data_parallel(args):
         return dist_train.run_data_parallel(args, device)
     if dist_train.partitioned(args):
@@ -214,9 +243,7 @@ def run(args, device=None):
             log.info(f"Found model file '{args.model_args}' with trained parameters, restoring model state for inference..")
             model.load_state_dict(torch.load(args.model_args, map_location=device))
         stats = evaluate(model, test, threshold, pos_weight)
-        for s in stats:
-            log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f} loss {s.get('loss', float('nan')):.4f}")
-        log_ranking(stats)
+        log_test(stats, loss=True)
         if stats:
             add_baselines(dataset, test[0], stats[0])
             write_groups(dataset, test[0], stats[0], args.output)
@@ -321,9 +348,7 @@ def save_test_and_write(args, model, dataset, test, threshold, pos_weight, write
         torch.save(model.state_dict(), path)                                          # pangnn.py:339-341
         log.info(f"Saved model parameters to '{path}'")
     stats = evaluate(model, test, threshold, pos_weight, group)                       # pangnn.py:344-346
-    for s in stats:
-        log.info(f"test: f1 {s['f1']:.4f} precision {s['precision']:.4f} recall {s['recall']:.4f}")
-    log_ranking(stats)
+    log_test(stats)
     if stats:
         add_baselines(dataset, test[0], stats[0])
         if write:
