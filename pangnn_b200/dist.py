@@ -701,7 +701,7 @@ def _layer(x_own, conv, lg, weighted, act, site):
     W, b = conv.lin.weight, conv.bias
     val_dst, val_src = lg.norm(weighted)
     plan = lg.plan
-    if W.size(1) < W.size(0):                                   # widening: aggregate first
+    if ops.aggregate_first(W):
         _, dx_out = _fwd_buf(plan, site, W.size(1), x_own.device)
         x_ext = HaloGather.apply(x_own, plan, site)
         ax = ops.AggregateFn.apply(x_ext, None, lg.gs.dst, val_dst, lg.gs.src, val_src, lg.n_own, ops.ACT_NONE, dx_out)
@@ -744,18 +744,6 @@ def _embed_conv(m, pg, act, consumer=None):
                                m.conv_in.bias, act)
 
 
-def _layer_ext(x_ext, conv, lg, weighted, act):
-    """One GCNConv (+ELU) whose input already holds the graph's own + halo rows (ghost rows recomputed locally,
-    see ``_embed_conv``): no exchange; the gradient of every extended row stays on this rank."""
-    W, b = conv.lin.weight, conv.bias
-    val_dst, val_src = lg.norm(weighted)
-    if W.size(1) < W.size(0):                                   # widening: aggregate first
-        ax = ops.AggregateFn.apply(x_ext, None, lg.gs.dst, val_dst, lg.gs.src, val_src, lg.n_own, ops.ACT_NONE, None)
-        return ops.linear(ax, W, b, act)
-    t_ext = ops.linear(x_ext, W, None, ops.ACT_NONE)
-    return ops.AggregateFn.apply(t_ext, b, lg.gs.dst, val_dst, lg.gs.src, val_src, lg.n_own, act, None)
-
-
 class DistModel:
     """Runs an ``AlternateGCN``'s parameters on a ``PartitionedGraph`` (mlp decoder, node_dim 64)."""
 
@@ -763,37 +751,31 @@ class DistModel:
         self.model, self.group = model, group
 
     def embed(self, pg):
+        """``AlternateGCN.embed`` on the partition: the same embedding and ``conv_schedule``.  Each layer exchanges its
+        halo (``_layer``; the exchange site is named by the layer's position), except a fused embedding and the layer
+        that consumes its ghost rows (``_embed_conv``)."""
         m, ELU = self.model, ops.ACT_ELU
-        if getattr(m, "_categorical", False):
+        schedule, done = m.conv_schedule(), 0
+        if m._categorical:
             # A.6: one embedding row per gene, indexed by GLOBAL position (rows of other ranks get
             # zero gradient here; the flat all-reduce sums the disjoint row blocks)
             lo = pg.bounds[pg.rank]
-            x = m.embedding(torch.arange(lo, lo + pg.n_own, device=pg.x.device))
-        elif (pg.x.dim() == 2 and pg.x.size(1) == 1 and getattr(m, "fuse_embedding", True)
-              and m.conv_in.out_channels % 4 == 0 and m.conv_in.out_channels <= 256):
-            x = None                                                   # Linear(1, D) + conv_in folded (rank1.cu)
+            h = m.embedding(torch.arange(lo, lo + pg.n_own, device=pg.x.device))
+        elif m.fuses_embedding(pg.x):
+            mod, on, weighted = schedule[1]
+            consumer = getattr(pg, on) if on is not None else None
+            h, done = _embed_conv(m, pg, ELU, consumer), 1
+            if consumer is not None:
+                val_dst, val_src = consumer.norm(weighted)
+                h = ops.gcn_layer_csr(h, mod.lin.weight, mod.bias, consumer.gs.dst, val_dst, consumer.gs.src, val_src,
+                                      consumer.n_own, ELU)
+                done = 2
         else:
-            x = (torch.addcmul(m.embedding.bias, pg.x, m.embedding.weight.t())
+            h = (torch.addcmul(m.embedding.bias, pg.x, m.embedding.weight.t())
                  if pg.x.dim() == 2 and pg.x.size(1) == 1 else m.embedding(pg.x))
-        if x is None:
-            if args.union_edge_weights:
-                h = _layer_ext(_embed_conv(m, pg, ELU, pg.conv), m.conv_hidden, pg.conv, True, ELU)
-                for i in range(1, max(args.neighbours - 2, 1)):
-                    h = _layer(h, m.conv_hidden, pg.conv, True, ELU, f"hid{i}")
-                return _layer(h, m.conv_out, pg.conv, False, ELU, "out")
-            if args.base_model:
-                return m.activation_fct(m.linear_out(_embed_conv(m, pg, ELU)))
-            return _layer_ext(_embed_conv(m, pg, ELU, pg.nb), m.conv_out, pg.nb, False, ELU)
-        if args.union_edge_weights:
-            h = _layer(x, m.conv_in, pg.conv, True, ELU, "in")
-            for i in range(max(args.neighbours - 2, 1)):
-                h = _layer(h, m.conv_hidden, pg.conv, True, ELU, f"hid{i}")
-            return _layer(h, m.conv_out, pg.conv, False, ELU, "out")
-        if args.base_model:
-            h = _layer(x, m.conv_in, pg.conv, True, ELU, "in")
-            return m.activation_fct(m.linear_out(h))
-        h = _layer(x, m.conv_in, pg.conv, True, ELU, "in")
-        return _layer(h, m.conv_out, pg.nb, False, ELU, "nb")
+        for i, (mod, on, weighted) in enumerate(schedule[done:], done):
+            h = m.activation_fct(mod(h)) if on is None else _layer(h, mod, getattr(pg, on), weighted, ELU, f"conv{i}")
+        return h
 
     def _scorer_inputs(self, pg, h):
         """-> (endpoint rows pq_ext [n_ext, 2D], the scorer's weights (w1c, b1, w2, b2, w3, b3), dpq_out)."""

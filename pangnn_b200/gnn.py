@@ -91,42 +91,56 @@ class AlternateGCN(nn.Module):
         self.fuse_embedding = True        # Linear(1, D) + conv_in as one rank-2 update when x is [N, 1]
 
     # -- node embeddings after the convolutions (src/gnn.py:125-166) ------------------------------
-    def embed(self, graph):
-        ELU = ops.ACT_ELU
-        if (not self._categorical and graph.x.dim() == 2 and graph.x.size(1) == 1 and self.fuse_embedding
-                and OPERATOR_LAYER["kind"] == "function"
-                and self.conv_in.out_channels % 4 == 0 and self.conv_in.out_channels <= 256):
-            # scalar node features: Linear(1, D) + conv_in collapse into one rank-2 update (ops.RankOneFn)
+    def conv_schedule(self):
+        """The layers that follow the embedding under the current flags (``src/gnn.py:129-166``), one GPU and partition
+        alike: ``[(module, graph, weighted), ...]`` with ``graph`` "conv" (the union graph with ``--union_edge_weights``,
+        else the scored edges), "nb" (the neighbour band) or None (``linear_out`` + ELU, ``--base_model``) and
+        ``weighted`` whether the layer takes the edge weights."""
+        first = (self.conv_in, "conv", True)
+        if args.union_edge_weights:
+            hidden = [(self.conv_hidden, "conv", True)] * max(args.neighbours - 2, 1)
+            return [first] + hidden + [(self.conv_out, "conv", False)]
+        if args.base_model:
+            return [first, (self.linear_out, None, False)]
+        return [first, (self.conv_out, "nb", False)]
+
+    def fuses_embedding(self, x):
+        """Whether ``Linear(1, D)`` + ``conv_in`` run as one rank-2 update (``ops.RankOneFn``) for node features ``x``."""
+        return (not self._categorical and self.fuse_embedding and x.dim() == 2 and x.size(1) == 1
+                and self.conv_in.out_channels % 4 == 0 and self.conv_in.out_channels <= 256)
+
+    @staticmethod
+    def _edges(graph, on, weighted):
+        """(edge_index, edge_weight) of a schedule entry on a whole graph."""
+        if on == "nb":
+            ei = graph.neighbour_edge_index
+        else:
             ei = graph.union_edge_index if args.union_edge_weights else graph.edge_index
-            emb, cin = self.embedding, self.conv_in
-            nodes = ops.embed_conv(graph.x, emb.weight, emb.bias, cin.lin.weight, cin.bias, ei, graph.edge_attr, ELU)
-            return self._embed_tail(graph, nodes)
-        if self._categorical:
+        return ei, (graph.edge_attr if weighted else None)
+
+    def embed(self, graph):
+        schedule = self.conv_schedule()
+        if self.fuses_embedding(graph.x) and OPERATOR_LAYER["kind"] == "function":
+            cin, on, weighted = schedule.pop(0)
+            emb = self.embedding
+            nodes = ops.embed_conv(graph.x, emb.weight, emb.bias, cin.lin.weight, cin.bias,
+                                   *self._edges(graph, on, weighted), ops.ACT_ELU)
+        elif self._categorical:
             idx = graph.x if graph.x.dtype == torch.long else (
                 graph.node_id if hasattr(graph, "node_id") else
                 torch.arange(graph.x.size(0), device=graph.x.device))
-            node_embeddings = self.embedding(idx)
+            nodes = self.embedding(idx)
         elif graph.x.dim() == 2 and graph.x.size(1) == 1:
             # Linear(1, D) (src/gnn.py:97,125) is an outer product: x w^T + b as ONE broadcast elementwise pass
             # instead of a K = 1 library GEMM (0.18 ms at N = 1e6) — same values, same parameters
-            node_embeddings = torch.addcmul(self.embedding.bias, graph.x, self.embedding.weight.t())
+            nodes = torch.addcmul(self.embedding.bias, graph.x, self.embedding.weight.t())
         else:
-            node_embeddings = self.embedding(graph.x)
-        ei = graph.union_edge_index if args.union_edge_weights else graph.edge_index
-        nodes = self.conv_in(node_embeddings, ei, graph.edge_attr, _act=ELU)
-        return self._embed_tail(graph, nodes)
-
-    def _embed_tail(self, graph, nodes):
-        """The layers after ``conv_in`` + ELU (``src/gnn.py:131-166``)."""
-        ELU = ops.ACT_ELU
-        if args.union_edge_weights:
-            for _ in range(max(args.neighbours - 2, 1)):
-                nodes = self.conv_hidden(nodes, graph.union_edge_index, graph.edge_attr, _act=ELU)
-            nodes = self.conv_out(nodes, graph.union_edge_index, None, _act=ELU)
-        elif args.base_model:
-            nodes = self.activation_fct(self.linear_out(nodes))
-        else:
-            nodes = self.conv_out(nodes, graph.neighbour_edge_index, None, _act=ELU)
+            nodes = self.embedding(graph.x)
+        for mod, on, weighted in schedule:
+            if on is None:
+                nodes = self.activation_fct(mod(nodes))
+            else:
+                nodes = mod(nodes, *self._edges(graph, on, weighted), _act=ops.ACT_ELU)
         return nodes
 
     def _skip(self, graph):

@@ -215,13 +215,6 @@ def gcn_aggregate(rowptr, col, val, x, num_rows, bias=None, act=ACT_NONE, out=No
     return out
 
 
-def aggregate(gs, ent, x, by_dst, bias=None, act=ACT_NONE, out=None):
-    """``A_hat x`` (``by_dst``) or ``A_hat^T x`` over the structure ``gs`` with the normalisation ``ent`` (=
-    ``gs.norm(weight, need_src=not by_dst)``)."""
-    csr = gs.dst if by_dst else gs.src
-    return gcn_aggregate(csr.rowptr, csr.col, ent["dst" if by_dst else "src"], x, gs.num_nodes, bias, act, out)
-
-
 def segment_sum_edges(csr, rows, num_rows, out):
     """``out[i] = sum of the per-edge ``rows`` of CSR row i`` (the scorer's per-edge gradients back to the nodes).
     A list that arrived in this CSR's order needs no gather: its rows are consecutive (identity columns)."""
@@ -337,14 +330,11 @@ def node_linear(x, w, bias=None, act=ACT_NONE, w_is_kn=False, out=None, push=Non
     if not _tc_shape(x, n, k) or x.size(1) != k or w.stride(1) != 1 or (bias is not None and bias.data_ptr() % 16):
         if push is not None:
             raise _abi.PangnnError("the fused halo push needs the tensor-core shapes (n, k in {64, 128})")
-        y = torch.mm(x, w if w_is_kn else w.t())
+        y = torch.mm(x, w if w_is_kn else w.t(), out=out)
         if bias is not None:
             y += bias
         if act == ACT_ELU:
             torch.nn.functional.elu_(y)
-        if out is not None:
-            out.copy_(y)
-            return out
         return y
     lib = _abi.load()
     M = x.size(0)
@@ -521,59 +511,22 @@ def drop_structs(graph):
 # ------------------------------------------------------------------------------------------------
 # autograd: one GCN layer  y = act( A_hat (x W^T) + b )
 # ------------------------------------------------------------------------------------------------
-class GCNLayerFn(torch.autograd.Function):
-    """Transform-then-aggregate (the reference's order): y = act(A_hat (x W^T) + b).  Used when the
-    layer does not widen (out <= in), so the gather runs at the narrower width."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, gs, edge_weight, act):
-        ent = gs.norm(edge_weight, need_src=False)
-        h = node_linear(x, weight)                                      # K3: tcgen05 3xTF32
-        y = aggregate(gs, ent, h, True, bias, act)
-        ctx.gs, ctx.edge_weight, ctx.act = gs, edge_weight, act
-        ctx.has_bias = bias is not None
-        ctx.save_for_backward(x, weight, y if act != ACT_NONE else None)
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, weight, y = ctx.saved_tensors
-        gs = ctx.gs
-        ent = gs.norm(ctx.edge_weight, need_src=True)
-        g, dbias = act_bwd_bias(dy, y, ctx.act)
-        dh = aggregate(gs, ent, g, False)                                            # A_hat^T g
-        dW = gemm_tn(dh, x) if ctx.needs_input_grad[1] else None
-        dx = node_linear(dh, weight, w_is_kn=True) if ctx.needs_input_grad[0] else None
-        return dx, dW, (dbias if ctx.has_bias and ctx.needs_input_grad[2] else None), None, None, None
+def aggregate_first(weight):
+    """The order of a GCN layer with ``weight`` [out, in]: aggregate, then transform, when the layer widens, so that
+    the HBM/L2-bound gather moves rows of width ``in`` instead of ``out`` (half the bytes for conv_in, 64 -> 128).
+    A_hat (x W^T) = (A_hat x) W^T, so both orders compute the same map; ``gcn_aggregate`` needs ``in % 4 == 0``."""
+    return weight.size(1) < weight.size(0) and weight.size(1) % 4 == 0
 
 
-class GCNLayerAggFirstFn(torch.autograd.Function):
-    """Aggregate-then-transform: y = act((A_hat x) W^T + b) — the same linear map (A_hat (x W^T) =
-    (A_hat x) W^T), chosen when the layer widens (in < out) so that the HBM/L2-bound gather moves
-    rows of width `in` instead of `out` (half the bytes for conv_in, 64 -> 128)."""
-
-    @staticmethod
-    def forward(ctx, x, weight, bias, gs, edge_weight, act):
-        ent = gs.norm(edge_weight, need_src=False)
-        ax = aggregate(gs, ent, x, True)
-        y = node_linear(ax, weight, bias, act)                          # bias + ELU in the GEMM epilogue
-        ctx.gs, ctx.edge_weight, ctx.act = gs, edge_weight, act
-        ctx.has_bias = bias is not None
-        ctx.save_for_backward(ax, weight, y if act != ACT_NONE else None)
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        ax, weight, y = ctx.saved_tensors
-        gs = ctx.gs
-        g, dbias = act_bwd_bias(dy, y, ctx.act)
-        dW = gemm_tn(g, ax) if ctx.needs_input_grad[1] else None
-        dx = None
-        if ctx.needs_input_grad[0]:
-            ent = gs.norm(ctx.edge_weight, need_src=True)
-            dax = node_linear(g, weight, w_is_kn=True)
-            dx = aggregate(gs, ent, dax, False)
-        return dx, dW, (dbias if ctx.has_bias and ctx.needs_input_grad[2] else None), None, None, None
+def gcn_layer_csr(x, weight, bias, csr_dst, val_dst, csr_src, val_src, n_out, act=ACT_NONE):
+    """``act(A_hat (x W^T) + b)[:n_out]`` from ``linear`` and ``AggregateFn``, in the order of ``aggregate_first``.
+    ``x`` holds every source row of the graph (own + halo or ghost rows on a partition, all rows on one GPU);
+    ``csr_src`` / ``val_src`` serve the backward alone.  Saved for the backward: ``x`` (``A_hat x`` when aggregating
+    first), ``W`` and, with an activation, ``y``."""
+    if aggregate_first(weight):
+        ax = AggregateFn.apply(x, None, csr_dst, val_dst, csr_src, val_src, n_out, ACT_NONE)
+        return linear(ax, weight, bias, act)
+    return AggregateFn.apply(linear(x, weight), bias, csr_dst, val_dst, csr_src, val_src, n_out, act)
 
 
 def rank1_vectors(csr_dst, val_dst, x, num_rows=None):
@@ -652,8 +605,13 @@ def gcn_layer(x, weight, bias, edge_index, edge_weight=None, act=ACT_NONE):
     """GCNConv(add_self_loops=False) forward (+ optional fused ELU) — ``src/gnn.py:129-165``."""
     _need_cuda(x, weight, edge_index)
     gs = graph_struct(edge_index, x.size(0))
-    fn = GCNLayerAggFirstFn if (weight.size(1) < weight.size(0) and weight.size(1) % 4 == 0) else GCNLayerFn
-    return fn.apply(x.contiguous(), weight, bias, gs, edge_weight, act)
+    # the by-source CSR and its normalisation are built only for an aggregation whose backward will run
+    # (inference builds neither); in training they are cached with the structure and the weights
+    grad_from = (x,) if aggregate_first(weight) else (x, weight, bias)
+    need_src = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in grad_from)
+    ent = gs.norm(edge_weight, need_src)
+    src, val_src = (gs.src, ent["src"]) if need_src else (None, None)
+    return gcn_layer_csr(x, weight, bias, gs.dst, ent["dst"], src, val_src, gs.num_nodes, act)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -880,7 +838,9 @@ class LinearFn(torch.autograd.Function):
             # a fresh tensor object over the caller's memory (never the caller's own tensor: returning
             # an input would need mark_dirty and tie this node's history to a reused buffer)
             y_full = _alias(out_full, out_full.shape, out_full.stride())
-        y = node_linear(x, weight, bias, act, out=y_full[:M], push=push)
+        # without extra rows, the output itself and not a view of it: a view made here and written by torch ops (the
+        # library GEMM of shapes outside {64, 128}) cannot be saved for the backward
+        y = node_linear(x, weight, bias, act, out=y_full if y_full.size(0) == M else y_full[:M], push=push)
         ctx.act, ctx.has_bias, ctx.M = act, bias is not None, M
         ctx.save_for_backward(x, weight, y if act != ACT_NONE else None)
         return y_full
@@ -903,12 +863,12 @@ def linear(x, weight, bias=None, act=ACT_NONE, extra_rows=0, out_full=None, push
 
 
 # ------------------------------------------------------------------------------------------------
-# building blocks of the genome-partitioned (multi-GPU) path: see pangnn_b200/dist.py
+# the aggregation of a GCN layer (gcn_layer_csr), on one GPU and on a partition (pangnn_b200/dist.py)
 # ------------------------------------------------------------------------------------------------
 class AggregateFn(torch.autograd.Function):
-    """y[:n_out] = act(A_hat x_ext + b) on a LOCAL graph whose sources live in "own + halo"
-    numbering: forward walks the by-destination CSR (rows = owned nodes), backward walks the
-    by-source CSR (rows = own + halo) and returns gradients for every extended row — into
+    """y[:n_out] = act(A_hat x_ext + b) on a graph whose sources live in "own + halo" numbering (a LOCAL graph of
+    a partition; on one GPU every row is owned): forward walks the by-destination CSR (rows = owned nodes), backward
+    walks the by-source CSR (rows = own + halo) and returns gradients for every extended row — into
     ``dx_out`` when given (a symmetric-memory buffer whose halo part the owners read over NVLink)."""
 
     @staticmethod

@@ -201,14 +201,14 @@ edge_score_bce.register_autograd(_score_bce_backward, setup_context=_score_bce_s
 # ------------------------------------------------------------------------------------------------
 def gcn_conv(x, weight, bias, edge_index, edge_weight=None, act=ops.ACT_NONE):
     """``GCNConv(add_self_loops=False).forward`` (+ optional fused ELU), ``src/gnn.py:129-165``: gcn_norm once per
-    (structure, weights) from the structure cache, then ``node_linear`` and ``gcn_propagate`` in the order that
-    moves the narrower rows through the gather (``ops.gcn_layer`` makes the same choice)."""
+    (structure, weights) from the structure cache, then ``node_linear`` and ``gcn_propagate`` in the order of
+    ``ops.aggregate_first``, as ``ops.gcn_layer``."""
     gs = ops.graph_struct(edge_index, x.size(0))
     ent = gs.norm(edge_weight, need_src=True)
     d, s = gs.dst, gs.src
     csr = (d.rowptr, d.col, ent["dst"], s.rowptr, s.col, ent["src"], gs.num_nodes)
     P = torch.ops.pangnn
-    if weight.size(1) < weight.size(0) and weight.size(1) % 4 == 0:          # widening layer: aggregate first
+    if ops.aggregate_first(weight):
         return P.node_linear(P.gcn_propagate(x, None, *csr, ops.ACT_NONE), weight, bias, act, False)
     return P.gcn_propagate(P.node_linear(x, weight, None, ops.ACT_NONE, False), bias, *csr, act)
 

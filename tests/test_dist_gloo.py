@@ -111,7 +111,7 @@ def _patch(ops):
 
 
 # ------------------------------------------------------------------------------------------------
-def _worker(rank, world, init_file, case, variant, out_dir):
+def _worker(rank, world, init_file, case, variant, fuse_embedding, out_dir):
     dist.init_process_group("gloo", init_method=f"file://{init_file}", rank=rank, world_size=world)
     try:
         from pangnn_b200 import dist as pd, ops, setup
@@ -127,6 +127,7 @@ def _worker(rank, world, init_file, case, variant, out_dir):
         N = graph.x.size(0)
         model = AlternateGCN("cpu", None, False, dims=[fl.node_dim, fl.hidden_dim])
         model.load_state_dict(make_state_dict(fl.node_dim, fl.hidden_dim, fl.skip_connections, seed=1234))
+        model.fuse_embedding = fuse_embedding
         pgraph = pd.PartitionedGraph.from_global(graph, N, rank, world)
         dm = pd.DistModel(model)
         pw = float(g[f"model/{variant}/pos_weight"])
@@ -145,13 +146,15 @@ def _worker(rank, world, init_file, case, variant, out_dir):
 
 
 @pytest.mark.parametrize("world", [2, 3])
-@pytest.mark.parametrize("case,variant", [("sim5", "default"), ("sim5", "union_skip"), ("c1", "base"),
-                                          ("c1", "union_n4")])
-def test_partitioned_model_equals_whole_graph(case, variant, world):
+@pytest.mark.parametrize("case,variant,fuse_embedding", [
+    pytest.param(case, variant, fuse, id=f"{case}-{variant}" + ("" if fuse else "-unfused"))
+    for fuse in (True, False)
+    for case, variant in [("sim5", "default"), ("sim5", "union_skip"), ("c1", "base"), ("c1", "union_n4")]])
+def test_partitioned_model_equals_whole_graph(case, variant, fuse_embedding, world):
     g = load_golden(case)
     with tempfile.TemporaryDirectory() as tmp:
         init_file = os.path.join(tmp, "rendezvous")
-        mp.spawn(_worker, args=(world, init_file, case, variant, tmp), nprocs=world, join=True)
+        mp.spawn(_worker, args=(world, init_file, case, variant, fuse_embedding, tmp), nprocs=world, join=True)
         outs = [np.load(os.path.join(tmp, f"r{r}.npz")) for r in range(world)]
     key = f"model/{variant}"
     ref_logits, ref_loss = g[f"{key}/logits"], float(g[f"{key}/loss"])
