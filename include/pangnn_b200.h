@@ -313,6 +313,11 @@ int pangnn_segment_max_labels(const int32_t *q, const int32_t *t, const void *sc
  *     da1[E,D] (per-edge gradient wrt a1, to be segment-reduced to the nodes),
  *     grads[] = { dW2[D*D], db2[D], dw3[D], db3[1], db1[D], dw1c[D] }  (overwritten).
  * dz comes from dlogits[E] when given, else from the fused BCE:  dz = scale*((1-y)s - pw*y*(1-s)).
+ * Label contract of bwd's fused BCE (dlogits == NULL): y[e] in {0, 1} is a label; y[e] < 0 means "no label"
+ * (an edge held out of training, --edge_split): its loss term and its dz are 0, so it adds nothing to da1 (its row
+ * is written as 0), grads or loss_sum, while its logit is still written.  scale stays the caller's: 1 / (number
+ * of labelled edges) for a mean.  Labels in {0, 1} give bit-identical results to a call without this rule.
+ * fwd's optional loss (y != NULL) requires labels in {0, 1}; no split path calls it.
  * ---------------------------------------------------------------------------------------------- */
 #define PANGNN_SCORER_D 64
 #define PANGNN_SCORER_NGRADS (64 * 64 + 64 + 64 + 1 + 64 + 64)
@@ -335,6 +340,20 @@ int pangnn_edge_score_bwd(const float *pq, const int32_t *src, const int32_t *ds
                           const float *w3, const float *b3, int64_t num_edges, const float *dlogits,
                           const float *y, float pos_weight, float scale, float *da1, float *grads,
                           float *logits, double *loss_sum, void *ws, size_t ws_bytes, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Held-out edges of whole-graph training (--edge_split VAL TEST): split[e] of the scored edge (src[e], dst[e])
+ * (global node ids >= 0) by its unordered pair a = min, b = max: x = first word of Philox4x32-10 keyed by
+ * (seed, purpose 5) at counter (0, a, b, 0); PANGNN_SPLIT_VAL if x < t_val, PANGNN_SPLIT_TEST if
+ * x < t_val + t_test (as a 64-bit sum, at most 2^32), else PANGNN_SPLIT_TRAIN.  t_val = floor(VAL * 2^32),
+ * t_test = floor(TEST * 2^32), computed by the caller.  Both directions of a pair get the same code; the codes
+ * depend on (seed, a, b) alone, not on the edge order or the rank that holds the edge.
+ * ---------------------------------------------------------------------------------------------- */
+#define PANGNN_SPLIT_TRAIN 0
+#define PANGNN_SPLIT_VAL 1
+#define PANGNN_SPLIT_TEST 2
+int pangnn_edge_split(const int32_t *src, const int32_t *dst, int64_t num_edges, uint64_t seed, uint32_t t_val,
+                      uint32_t t_test, int8_t *split, void *stream);
 
 /* Cosine decoder of src/gnn.py:179,206-207 (F.cosine_similarity, eps 1e-8) and the row-wise dot
  * of src/gnn.py:77-79 (mode 0 = cosine, 1 = dot), forward only. */

@@ -64,6 +64,7 @@ SIGNATURES = {
     "pangnn_edge_score_bwd": (_int, [_c_p] * 10 + [_i64, _c_p, _c_p, _f32, _f32, _c_p, _c_p, _c_p,
                                                    _c_p, _c_p, _sz, _c_p]),
     "pangnn_edge_score_predict": (_int, [_c_p] * 10 + [_i64, _f32, _c_p, _c_p, _c_p, _c_p]),
+    "pangnn_edge_split": (_int, [_c_p, _c_p, _i64, C.c_uint64, C.c_uint32, C.c_uint32, _c_p, _c_p]),
     "pangnn_edge_pair_score": (_int, [_c_p, _i64, _i32, _c_p, _c_p, _i64, _int, _c_p, _c_p]),
     "pangnn_edge_pair_score_bwd_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "pangnn_edge_pair_score_bwd": (_int, [_c_p, _i64, _i32, _i32, _i64, _c_p, _c_p, _c_p, _c_p, _c_p, _c_p,

@@ -12,7 +12,8 @@
 //            dr1 = da2 W2 = dz (.) (m2 W2') row by row, so G2 needs neither dz nor a hi / lo split of its A operand
 //            (a 0 / 1 matrix is exact in TF32: 2 products per k-step instead of 3) and is issued BEFORE the logit
 //            reduction, the loss and the sigmoid — it runs underneath them.
-//   epi-1b   z = r2 . w3 + b3 (one CTA barrier: partial sums of the 4 column slices); logit, loss, dz;
+//   epi-1b   z = r2 . w3 + b3 (one CTA barrier: partial sums of the 4 column slices); logit, loss, dz (an edge
+//            without a label, y < 0, gets no loss term and dz = 0, so every gradient contribution vanishes);
 //            dz m2 (hi / lo of the ROW scalar dz, selected by the mask) row-major -> smem over X (operand A of G3)
 //   G3       [P_hi ; P_lo] += [dz m2 hi | dz m2 lo]^T (r1_hi + r1_lo)   D3 [128 x 64], both operands MN-major (the
 //            row-major tiles themselves in the 128B / 32-byte-atom swizzle, umma.cuh); accumulates across the CTA's
@@ -320,6 +321,10 @@ edge_score_train_kernel(const ScorerArgs p) {
                 asm volatile("prefetch.global.L2 [%0];" :: "l"(pd + 128));
             }
             PROF_T(2);
+            // this edge slot's label, loaded before the G1 wait so that its latency hides under the contraction
+            const int64_t e = e0 + row;
+            const bool ok = e < p.E;
+            const float yy = (ok && p.y) ? __ldg(p.y + e) : 0.f;
             umma::mbar_wait(&bar1, par);
             umma::fence_after_sync();
             PROF_T(3);
@@ -359,10 +364,9 @@ edge_score_train_kernel(const ScorerArgs p) {
             load_indices(tile + 2 * (int64_t)gridDim.x);
             PROF_T(5);
             // ---- epilogue 1b: logit, loss, dz
-            const int64_t e = e0 + row;
-            const bool ok = e < p.E;
             const float zz = sZp[row] + sZp[BM + row] + sZp[2 * BM + row] + sZp[3 * BM + row] + b3;
-            const float yy = (ok && p.y) ? p.y[e] : 0.f;
+            // y < 0: no label (held out): no loss term, dz = 0.  Selects, not branches: the loss branch stays uniform
+            const bool labelled = yy >= 0.f;
             if (h == 0 && ok) {
                 if (p.logits) p.logits[e] = zz;
                 if (p.prob || p.pred) {
@@ -373,7 +377,8 @@ edge_score_train_kernel(const ScorerArgs p) {
                 if (p.y && p.loss_partial) {
                     // torch BCEWithLogits(pos_weight): (1-y) z + (1+(pw-1)y) (log1p(exp(-|z|)) + max(-z,0))
                     const float lw = fmaf(p.pos_weight - 1.f, yy, 1.f);
-                    loss_acc += (1.f - yy) * zz + lw * (log1pf(expf(-fabsf(zz))) + fmaxf(-zz, 0.f));
+                    const float term = (1.f - yy) * zz + lw * (log1pf(expf(-fabsf(zz))) + fmaxf(-zz, 0.f));
+                    loss_acc += labelled ? term : 0.f;
                 }
             }
             float dz = 0.f;
@@ -384,7 +389,8 @@ edge_score_train_kernel(const ScorerArgs p) {
                     // torch's backward: ((pw*y + 1 - y) * sigmoid(z) - pw*y) * grad
                     const float sg = 1.f / (1.f + expf(-zz));
                     const float t = p.pos_weight * yy;
-                    dz = ((t + 1.f - yy) * sg - t) * p.scale;
+                    const float g = ((t + 1.f - yy) * sg - t) * p.scale;
+                    dz = labelled ? g : 0.f;
                 }
             }
             if (h == 0) gb3 += dz;

@@ -479,7 +479,7 @@ class PartitionedGraph:
 
     def __init__(self, bounds, rank, world, x_own, conv_ei, conv_w, nb_ei, scored_ei, scored_w, y,
                  group=None):
-        self.rank, self.world, self.bounds = rank, world, bounds
+        self.rank, self.world, self.bounds, self.group = rank, world, bounds, group
         b = (bounds, rank, world)
         self.n_own = bounds[rank + 1] - bounds[rank]
         self.x = x_own
@@ -502,6 +502,20 @@ class PartitionedGraph:
         their local order (the order of ``y``, ``skip`` and the logits)."""
         m, o = self.scored.edge_mask, self.scored.edge_order
         return t[m][o].contiguous() if o is not None else t[m].contiguous()
+
+    def scored_endpoints(self):
+        """GLOBAL ``(src, dst)`` of this rank's scored edges, in their local order."""
+        lg, lo = self.scored, self.bounds[self.rank]
+        ext = torch.cat((torch.arange(lo, lo + lg.n_own, device=lg.edge_index.device), lg.halo_ids.long()))
+        return ext[lg.edge_index[0]], ext[lg.edge_index[1]]
+
+    def build_edge_split(self, seed, fractions):
+        """``--edge_split``: ``self.split``, the ``edge_split.EdgeSplit`` of this rank's scored edges from their global
+        endpoints (no communication) with the counts and the train class balance over the group (one all-reduce).
+        -> the split."""
+        from .edge_split import EdgeSplit
+        self.split = EdgeSplit.build(*self.scored_endpoints(), self.y, seed, fractions, self.group)
+        return self.split
 
     # -- host round trip of the rank's local batch (bench.py's end-to-end leg) ----------------------
     _LOCALS = ("conv", "nb", "scored")
@@ -797,13 +811,16 @@ class DistModel:
 
     __call__ = forward
 
-    def forward_loss(self, pg, pos_weight, unit_grad=True):
+    def forward_loss(self, pg, pos_weight, unit_grad=True, y=None, num_labelled=None):
         """-> (this rank's share of the global mean loss, logits of the locally scored edges).  ``unit_grad``: the
-        loss is back-propagated as is (``loss.backward()``, checked on the device) — pass False to scale it first."""
+        loss is back-propagated as is (``loss.backward()``, checked on the device) — pass False to scale it first.
+        ``y``: this rank's selected labels in place of ``pg.y`` (``-1`` = held out, ``--edge_split``), the mean then
+        taken over ``num_labelled``, the GLOBAL number of edges with a label."""
         next_step()                                            # exchange buffers of the other parity (see _sym)
         pq_ext, weights, dpq_out = self._scorer_inputs(pg, self.embed(pg))
-        return ops.EdgeScoreBCEPQFn.apply(pq_ext, *weights, pg.scored.gs, pg.skip, pg.y, float(pos_weight),
-                                          1.0 / max(pg.num_edges_total, 1), dpq_out, unit_grad)
+        n = pg.num_edges_total if num_labelled is None else int(num_labelled)
+        return ops.EdgeScoreBCEPQFn.apply(pq_ext, *weights, pg.scored.gs, pg.skip, pg.y if y is None else y,
+                                          float(pos_weight), 1.0 / max(n, 1), dpq_out, unit_grad)
 
     @torch.no_grad()
     def predict(self, pg, threshold):
@@ -814,13 +831,16 @@ class DistModel:
         return ops.edge_score_predict(pq_ext, *weights, pg.scored.gs, pg.skip, threshold)
 
     @torch.no_grad()
-    def evaluate(self, pg, threshold, pos_weight=None):
+    def evaluate(self, pg, threshold, pos_weight=None, labels=None):
         """Test statistics of the whole partitioned graph, identical on every rank (``train.evaluate`` of the global
         graph, ``src/predict.py:29-55``): global confusion matrix (one all-reduce of four counts), precision /
         recall / F1 with ``eps=0``, the global mean BCE loss when ``pos_weight`` is given, and the exact global
         ranking metrics of the probabilities (``metrics.ranking_metrics`` over the group).  Also returns this
         rank's ``logits`` / ``prob`` / ``pred`` (edges ``pg.scored_edge_ids``).  A graph without labels (``pg.y``
-        None) gets those and ``predicted_positive``, the global number of edges predicted positive, alone."""
+        None) gets those and ``predicted_positive``, the global number of edges predicted positive, alone.
+        ``labels``: this rank's selected labels (``-1`` outside the selection, ``--edge_split``): the counts, the loss
+        and the ranking metrics are then over the selected edges of every rank alone, and ``sel`` is this rank's
+        mask of them; ``logits`` / ``prob`` / ``pred`` stay those of every edge."""
         from .metrics import ranking_metrics
         from .train import prf
         logits, prob, pred = self.predict(pg, threshold)
@@ -831,6 +851,10 @@ class DistModel:
             if world > 1:
                 dist.all_reduce(k, group=self.group)
             return dict(logits=logits, prob=prob, pred=pred, predicted_positive=int(k))
+        out = dict(logits=logits, prob=prob, pred=pred)
+        if labels is not None:
+            out["sel"] = labels >= 0
+            y, logits, prob, pred = labels[out["sel"]], logits[out["sel"]], prob[out["sel"]], pred[out["sel"]]
         p, yl = pred.long(), y.long()
         tp = (p * yl).sum()
         fp = (p * (1 - yl)).sum()
@@ -847,9 +871,10 @@ class DistModel:
                 dist.all_reduce(loss_sum, group=self.group)
         tn, fp, fn, tp = (int(v) for v in cnt.tolist())
         pr, rc, f1 = prf(tn, fp, fn, tp, eps=0.0)
-        rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=pr, recall=rc, f1=f1, logits=logits, prob=prob, pred=pred)
+        rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=pr, recall=rc, f1=f1, **out)
         if loss_sum is not None:
-            rec["loss"] = float(loss_sum) / max(pg.num_edges_total, 1)
+            n = pg.num_edges_total if labels is None else tn + fp + fn + tp           # the global selected count
+            rec["loss"] = float(loss_sum) / max(n, 1)
         rk = ranking_metrics(prob, y, self.group)
         rec.update(auroc=rk["auroc"], average_precision=rk["average_precision"],
                    youden_threshold=rk["youden_threshold"], num_runs=rk["num_runs"])

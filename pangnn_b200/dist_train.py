@@ -19,6 +19,7 @@ import torch
 import torch.distributed as dist
 
 from . import dist as pdist
+from . import edge_split as es
 from . import ops
 from . import postprocessing as post
 from . import preprocessing as pp
@@ -33,6 +34,7 @@ def check_partition_flags(args, world):
     """Raise ``ValueError`` when the flags ask for something the partitioned driver at ``world`` ranks cannot do.
     Depends on the flags and ``world`` alone, so every rank refuses alike, before any device work."""
     check_label_flags(args)
+    es.check_flags(args)
     bad = []
     if getattr(args, "data_parallel", False):
         if args.whole_graph_training:
@@ -129,9 +131,8 @@ def _partition(args, device, rank, world):
         lab = lambda v: pg.pick(torch.as_tensor(v, dtype=torch.int64, device=device))
         t = dict(w=pg.pick(graph.edge_attr[:graph.edge_index.size(1)]), q_base=lab(dataset.base_labels),
                  raw_base=lab(dataset.base_labels_raw), names=dataset.gene_str_ids_lst, genome_of=dataset.genome_of)
-    lg, lo = pg.scored, pg.bounds[rank]
-    ext = torch.cat((torch.arange(lo, lo + lg.n_own, device=device), lg.halo_ids.long()))   # local id -> global id
-    t.update(gid=gid, src=ext[lg.edge_index[0]], dst=ext[lg.edge_index[1]])
+    src, dst = pg.scored_endpoints()
+    t.update(gid=gid, src=src, dst=dst)
     return pg, dataset, N, t
 
 
@@ -151,6 +152,14 @@ def _run(args, device, rank, world):
     pg, dataset, N, tables = _partition(args, device, rank, world)
     pos_weight = pg.class_balance                                                    # src/dataset.py:346, global
     log.info(f"Dataset: {N} genes, class balance {pos_weight}, built in {time.time() - t0:.1f} s")
+    fit, val_labels, test_labels = {}, None, None
+    if args.edge_split is not None:
+        # --edge_split: the split of the rank's own scored edges; counts and the train class balance are global
+        split = pg.build_edge_split(args.seed, args.edge_split)
+        log.info(split.describe())
+        pos_weight = split.class_balance
+        fit = dict(y=split.labels(pg.y, es.TRAIN), num_labelled=split.count(es.TRAIN))
+        val_labels, test_labels = split.labels(pg.y, es.VAL), split.labels(pg.y, es.TEST)
     torch.manual_seed(args.seed)                                                     # the one-GPU CLI's parameters
     model = AlternateGCN(device, N if args.categorical_node else dataset, args.categorical_node,
                          dims=[args.node_dim, args.hidden_dim]).to(device)
@@ -167,7 +176,7 @@ def _run(args, device, rank, world):
         if os.path.exists(args.model_args):
             log.info(f"Found model file '{args.model_args}' with trained parameters, restoring model state for inference..")
             model.load_state_dict(torch.load(args.model_args, map_location=device))
-        stat = _test(dm, pg, threshold, pos_weight, tables)
+        stat = _test(dm, pg, threshold, pos_weight, tables, test_labels)
         log_test([stat], loss=True)
         timings["outputs_s"] = _outputs(args, pg, stat, tables, N, rank, world, edge_table=True)
         return dict(model=model, dataset=dataset, history=history, test=[stat], graph=pg, timings=timings)
@@ -175,22 +184,26 @@ def _run(args, device, rank, world):
     for epoch in range(args.epochs):                                                  # pangnn.py:167-238
         t_ep = time.perf_counter()
         optimizer.zero_grad()
-        loss, logits = dm.forward_loss(pg, pos_weight)
+        loss, logits = dm.forward_loss(pg, pos_weight, **fit)
         loss.backward()
         dm.allreduce_grads()
         optimizer.step()
         prob = torch.sigmoid(logits.detach())
+        y = pg.y
+        if fit:                                               # the train edges alone
+            y, prob = es.select(fit["y"], prob)
         # the loss is this rank's share of the global mean: the sum over ranks is the one-GPU value
-        red = torch.cat((loss.detach().double().view(1), _counts(prob >= threshold, pg.y).double()))
+        red = torch.cat((loss.detach().double().view(1), _counts(prob >= threshold, y).double()))
         if world > 1:
             dist.all_reduce(red)
         red = red.tolist()
         train_loss, cm = red[0], [int(v) for v in red[1:]]
-        rk_tr = ranking_metrics(prob, pg.y)                   # over the default group: global, the same on every rank
+        rk_tr = ranking_metrics(prob, y)                      # over the default group: global, the same on every rank
         if args.dynamic_binary_threshold:                     # pangnn.py:229-233; == train.youden_threshold
             threshold = rk_tr["youden_threshold"] if rk_tr["youden_threshold"] is not None else threshold
         t_val = time.perf_counter()
-        val = dm.evaluate(pg, threshold, pos_weight)          # validation on the same whole graph, global
+        # validation: the same whole graph (its validation edges with --edge_split), global
+        val = dm.evaluate(pg, threshold, pos_weight, val_labels)
         t_end = time.perf_counter()
         timings["train_s"].append(t_val - t_ep)
         timings["val_s"].append(t_end - t_val)
@@ -202,6 +215,8 @@ def _run(args, device, rank, world):
                             f1_train=f1, f1_val=f1v, precision_val=pv, recall_val=rv,
                             auroc_train=rk_tr["auroc"], ap_train=rk_tr["average_precision"],
                             auroc_val=val["auroc"], ap_val=val["average_precision"]))
+        if val_labels is not None:                            # --edge_split: the validation edges' (tn, fp, fn, tp)
+            history[-1]["val_confusion"] = (val["tn"], val["fp"], val["fn"], val["tp"])
         log.info(f"epoch {epoch}: train loss {train_loss:.4f} f1 {f1:.4f} | val loss {mean_val:.4f} f1 {f1v:.4f}")
         log.info(f"epoch {epoch}: train auroc {_fmt(rk_tr['auroc'])} ap {_fmt(rk_tr['average_precision'])} | "
                  f"val auroc {_fmt(val['auroc'])} ap {_fmt(val['average_precision'])}")
@@ -213,14 +228,14 @@ def _run(args, device, rank, world):
         os.makedirs(args.output, exist_ok=True)
         torch.save(sd, path)                                                          # pangnn.py:339-341
     log.info(f"Saved model parameters to '{path}'")
-    stat = _test(dm, pg, threshold, pos_weight, tables)                               # pangnn.py:344-346
+    stat = _test(dm, pg, threshold, pos_weight, tables, test_labels)                  # pangnn.py:344-346
     log_test([stat])
     timings["outputs_s"] = _outputs(args, pg, stat, tables, N, rank, world, edge_table=bool(args.simulate_dataset))
     return dict(model=model, dataset=dataset, history=history, test=[stat], model_path=path, graph=pg, timings=timings)
 
 
-def _test(dm, pg, threshold, pos_weight, tables):
-    stat = dm.evaluate(pg, threshold, pos_weight)
+def _test(dm, pg, threshold, pos_weight, tables, labels=None):
+    stat = dm.evaluate(pg, threshold, pos_weight, labels)
     stat["edge_ids"] = tables["gid"]
     return stat
 
@@ -228,7 +243,8 @@ def _test(dm, pg, threshold, pos_weight, tables):
 def _outputs(args, pg, stat, t, N, rank, world, edge_table):
     """The one-GPU CLI's test outputs (``train.add_baselines``, ``write_groups``, ``write_curves``,
     ``write_edge_table``) for the whole partitioned graph.  Without labels (``pg.y`` None) the baselines are not scored,
-    no curves are written and the table's ``homolog`` column is -1.  -> seconds spent."""
+    no curves are written and the table's ``homolog`` column is -1.  With ``stat["sel"]`` (``--edge_split``) the
+    baselines and curves are those of the test edges; the groups and the table cover every edge.  -> seconds spent."""
     t0 = time.perf_counter()
     dev = stat["logits"].device
     genome_d = torch.as_tensor(t["genome_of"], device=dev)
@@ -245,7 +261,8 @@ def _outputs(args, pg, stat, t, N, rank, world, edge_table):
     # baselines line: precision / recall / F1 from the all-reduced confusion counts (src/predict.py:77-89)
     if y is not None:
         cand = {"base_labels": q_base, "base_labels_raw": raw_base, "logit_baseline": logit_base}
-        cnt = torch.stack([_counts(v, y) for v in cand.values()])
+        keep = stat["sel"][order] if "sel" in stat else None
+        cnt = torch.stack([_counts(v, y) if keep is None else _counts(v[keep], y[keep]) for v in cand.values()])
         if world > 1:
             dist.all_reduce(cnt)
         out = {k: prf(*c, eps=0.0) for k, c in zip(cand, cnt.tolist())} if pg.num_edges_total else {}
@@ -277,9 +294,12 @@ def _outputs(args, pg, stat, t, N, rank, world, edge_table):
         log.info(f"Wrote {len(groups)} ortholog groups to '{path}'")
 
     # ROC and precision-recall curves over the group, written by rank 0 (src/plot.py:103-107,131)
-    roc = roc_curve(stat["prob"], pg.y) if pg.y is not None else None
+    prob, yc = stat["prob"], pg.y
+    if yc is not None and "sel" in stat:
+        prob, yc = prob[stat["sel"]], yc[stat["sel"]]
+    roc = roc_curve(prob, yc) if yc is not None else None
     if roc is not None:
-        pr = precision_recall_curve(stat["prob"], pg.y, drop_intermediate=True)
+        pr = precision_recall_curve(prob, yc, drop_intermediate=True)
         if rank == 0:
             write_curve_files(roc, pr, args.output)
 

@@ -251,13 +251,24 @@ class AlternateGCN(nn.Module):
         wait()
         return graph
 
-    def forward_loss(self, graph, pos_weight):
+    def forward_loss(self, graph, pos_weight, y=None, num_labelled=None):
         """Fused training form of ``criterion(model(batch), batch.y)`` (``pangnn.py:200-203``):
-        returns ``(loss, logits)`` with logits detached; one kernel for scorer + loss + gradients."""
+        returns ``(loss, logits)`` with logits detached; one kernel for scorer + loss + gradients.
+
+        ``y``: labels in place of ``graph.y`` where ``-1`` marks an edge held out of training (``--edge_split``,
+        ``edge_split.EdgeSplit.labels``); the loss is then the mean over the ``num_labelled`` edges with ``y >= 0``.
+        Held-out edges stay in the graph: only their loss terms are dropped."""
+        if y is None:
+            y = graph.y
         if not self._use_fused_mlp_flag():
             logits = self.forward(graph)
-            loss = torch.nn.functional.binary_cross_entropy_with_logits(
-                logits, graph.y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device))
+            pw = torch.as_tensor(float(pos_weight), device=logits.device)
+            if num_labelled is None:
+                loss = torch.nn.functional.binary_cross_entropy_with_logits(logits, y, pos_weight=pw)
+            else:
+                sel = y >= 0
+                loss = torch.nn.functional.binary_cross_entropy_with_logits(
+                    logits[sel], y[sel], pos_weight=pw, reduction="sum") / max(int(num_labelled), 1)
             return loss, logits.detach()
         nodes = self.embed(graph)
         gs = ops.graph_struct(graph.edge_index, nodes.size(0))
@@ -265,10 +276,11 @@ class AlternateGCN(nn.Module):
         if OPERATOR_LAYER["kind"] == "library":
             from . import torch_ops
             return torch_ops.score_edges_bce(nodes, m[0].weight, m[0].bias, m[2].weight, m[2].bias, m[4].weight,
-                                             m[4].bias, graph.edge_index, self._skip(graph), graph.y, float(pos_weight))
+                                             m[4].bias, graph.edge_index, self._skip(graph), y, float(pos_weight),
+                                             num_labelled)
         return ops.EdgeScoreBCEFn.apply(
             nodes, m[0].weight, m[0].bias, m[2].weight, m[2].bias, m[4].weight, m[4].bias,
-            gs, self._skip(graph), graph.y, float(pos_weight))
+            gs, self._skip(graph), y, float(pos_weight), num_labelled)
 
     def _use_fused_mlp_flag(self):
         return args.decoder == "mlp" and self.mlp[2].weight.size(0) == ops.SCORER_D

@@ -746,21 +746,23 @@ class EdgeScoreFn(torch.autograd.Function):
 class EdgeScoreBCEFn(torch.autograd.Function):
     """Fused training form: (loss, logits) = BCEWithLogits(pos_weight)(MLP(...), y), mean reduction
     (``pangnn.py:98,203``).  ONE kernel produces logits, loss and all gradients; backward only
-    rescales by the incoming scalar."""
+    rescales by the incoming scalar.  ``num_labelled``: the number of edges with a label (``y >= 0``; an edge with
+    ``y < 0`` is held out, ``edge_split``), the divisor of the mean; None = every edge."""
 
     @staticmethod
-    def forward(ctx, h, w1, b1, w2, b2, w3, b3, gs, skip, y, pos_weight):
+    def forward(ctx, h, w1, b1, w2, b2, w3, b3, gs, skip, y, pos_weight, num_labelled=None):
         wcat, w1c = _scorer_common(h, w1, skip)
         E = gs.num_edges
+        n = max(E if num_labelled is None else int(num_labelled), 1)
         pq = node_linear(h, wcat)
         logits = torch.empty(E, dtype=torch.float32, device=h.device)
         loss_sum = torch.zeros(1, dtype=torch.float64, device=h.device)
         da1, grads = edge_score_train(pq, w1c, b1, w2, b2, w3, b3, gs, skip, y=y, pos_weight=pos_weight,
-                                      scale=1.0 / max(E, 1), logits=logits, loss_sum=loss_sum)
+                                      scale=1.0 / n, logits=logits, loss_sum=loss_sum)
         ctx.gs, ctx.skip = gs, skip
         ctx.save_for_backward(h, wcat, da1, grads)
         ctx.mark_non_differentiable(logits)
-        loss = (loss_sum / max(E, 1)).float().squeeze(0)
+        loss = (loss_sum / n).float().squeeze(0)
         return loss, logits
 
     @staticmethod
@@ -768,7 +770,7 @@ class EdgeScoreBCEFn(torch.autograd.Function):
         h, wcat, da1, grads = ctx.saved_tensors
         out = _unpack_scorer_grads(grads, da1, ctx.gs, h, wcat, ctx.skip, ctx.needs_input_grad[0],
                                    scale=dloss)
-        return out + (None, None, None, None)
+        return out + (None, None, None, None, None)
 
 
 class EdgePairScoreFn(torch.autograd.Function):
@@ -894,7 +896,8 @@ class AggregateFn(torch.autograd.Function):
 class EdgeScoreBCEPQFn(torch.autograd.Function):
     """Fused scorer + BCE on pre-transformed endpoint rows ``pq_ext`` [n_ext, 2D] (layer 1 hoisted by
     the caller).  Returns (sum of the per-edge losses * scale, logits).  Backward yields ``dpq_ext``
-    (P half reduced by source, Q half by destination — both sorted-segment) and the small grads."""
+    (P half reduced by source, Q half by destination — both sorted-segment) and the small grads.  An edge with
+    ``y < 0`` (held out, ``edge_split``) adds no loss and no gradient; ``scale`` is then 1 / the labelled count."""
 
     @staticmethod
     def forward(ctx, pq, w1c, b1, w2, b2, w3, b3, gs, skip, y, pos_weight, scale, dpq_out=None, unit_grad=False):

@@ -58,6 +58,10 @@ def build_parser():
     p.add_argument("--data_parallel", action="store_true",
                    help="(new) with --train under torchrun: replicate the model, shard the sub-graph batches, average "
                         "gradients each step (pangnn_b200.dist_train.run_data_parallel)")
+    p.add_argument("--edge_split", nargs=2, type=float, default=None, metavar=("VAL", "TEST"),
+                   help="(new) with --whole_graph_training: hold out these fractions of the scored edges (by unordered "
+                        "gene pair, from --seed) as validation and test edges; they stay in message passing, only "
+                        "their labels are hidden from training (pangnn_b200.edge_split)")
     p.add_argument("--seed", default=0, type=int)
     return p
 

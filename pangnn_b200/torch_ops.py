@@ -213,15 +213,17 @@ def gcn_conv(x, weight, bias, edge_index, edge_weight=None, act=ops.ACT_NONE):
     return P.gcn_propagate(P.node_linear(x, weight, None, ops.ACT_NONE, False), bias, *csr, act)
 
 
-def score_edges_bce(h, w1, b1, w2, b2, w3, b3, edge_index, skip, y, pos_weight):
+def score_edges_bce(h, w1, b1, w2, b2, w3, b3, edge_index, skip, y, pos_weight, num_labelled=None):
     """``criterion(mlp(cat(h[src], h[dst] (, skip))), y)`` (``src/gnn.py:171-177``, ``pangnn.py:98,203``), mean
-    reduction: -> (loss, logits).  Layer 1 of the MLP is hoisted to the nodes (``pq = h [W1a ; W1b]^T``)."""
+    reduction: -> (loss, logits).  Layer 1 of the MLP is hoisted to the nodes (``pq = h [W1a ; W1b]^T``).
+    ``num_labelled``: the number of edges with ``y >= 0`` (held-out edges carry ``y = -1``, ``edge_split``), the
+    divisor of the mean and the kernel's ``scale``; None = every edge."""
     gs = ops.graph_struct(edge_index, h.size(0))
     src, dst = gs.endpoints32
     wcat, w1c = ops.split_w1(w1, skip is not None)
     P = torch.ops.pangnn
     pq = P.node_linear(h, wcat, None, ops.ACT_NONE, False)
-    E = gs.num_edges
+    n = max(gs.num_edges if num_labelled is None else int(num_labelled), 1)
     loss, logits, _, _ = P.edge_score_bce(pq, src, dst, skip, w1c, b1, w2, b2, w3, b3, y, float(pos_weight),
-                                          1.0 / max(E, 1), gs.src.rowptr, gs.src.perm, gs.dst.rowptr, gs.dst.perm)
+                                          1.0 / n, gs.src.rowptr, gs.src.perm, gs.dst.rowptr, gs.dst.perm)
     return loss, logits.detach()

@@ -13,6 +13,7 @@ import time
 import numpy as np
 import torch
 
+from . import edge_split as es
 from . import postprocessing as post
 from . import setup
 from .metrics import precision_recall_curve, ranking_metrics, roc_curve
@@ -62,28 +63,39 @@ def youden_threshold(prob, labels):
     return float(p[last][best]) if float(j[best]) > 0 else None
 
 
-def evaluate(model, graphs, threshold, pos_weight=None, group=None):
+def evaluate(model, graphs, threshold, pos_weight=None, group=None, labels=None):
     """Whole-batch inference as ``src/predict.py:29-55``: logits, sigmoid, threshold, confusion; plus the ROC AUC, AP
     and Youden threshold of the probabilities (``src/plot.py:103-107,131``; exact, ``metrics.ranking_metrics`` over
     ``group``: pass a group of one rank for a replica's own graphs while a default process group exists).  A graph
     without labels (``y`` None) gets its ``logits`` / ``prob`` / ``pred`` and ``predicted_positive``, the number of
-    edges predicted positive, alone."""
+    edges predicted positive, alone.
+
+    ``labels``: per graph, selected labels (``-1`` outside the selection, ``edge_split.EdgeSplit.labels``): the
+    statistics are then over the edges with a label >= 0 alone, whose mask is kept as ``sel``; ``logits`` / ``prob``
+    / ``pred`` stay those of every edge (the groups file and the per-edge table cover all edges)."""
     model.eval()
     out = []
-    for g in graphs:
+    for i, g in enumerate(graphs):
         logits, prob, pred = model.predict(g, threshold)
         if g.y is None:
             out.append(dict(logits=logits, prob=prob, pred=pred, predicted_positive=int(pred.sum())))
             continue
-        tn, fp, fn, tp = confusion(pred, g.y)
+        y, lg, pr, pd = g.y, logits, prob, pred
+        sel = None
+        if labels is not None:
+            sel = labels[i] >= 0
+            y, lg, pr, pd = labels[i][sel], logits[sel], prob[sel], pred[sel]
+        tn, fp, fn, tp = confusion(pd, y)
         p, r, f1 = prf(tn, fp, fn, tp, eps=0.0)
         rec = dict(tn=tn, fp=fp, fn=fn, tp=tp, precision=p, recall=r, f1=f1, logits=logits, prob=prob, pred=pred)
-        rk = ranking_metrics(prob, g.y, group)
+        if sel is not None:
+            rec["sel"] = sel
+        rk = ranking_metrics(pr, y, group)
         rec.update(auroc=rk["auroc"], average_precision=rk["average_precision"],
                    youden_threshold=rk["youden_threshold"])
         if pos_weight is not None:
             rec["loss"] = float(torch.nn.functional.binary_cross_entropy_with_logits(
-                logits, g.y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device)))
+                lg, y, pos_weight=torch.as_tensor(float(pos_weight), device=logits.device)))
         out.append(rec)
     return out
 
@@ -137,11 +149,13 @@ def add_baselines(dataset, graph, stat):
     cand = {"base_labels": dataset.base_labels, "base_labels_raw": dataset.base_labels_raw,
             "logit_baseline": logit_base}
     out = {}
+    sel = stat.get("sel")                                     # --edge_split: the test edges alone
+    y = graph.y if sel is None else graph.y[sel]
     for name, lab in cand.items():
         if lab is None or len(lab) == 0:
             continue
         pred = torch.as_tensor(lab, device=graph.y.device)
-        out[name] = prf(*confusion(pred, graph.y), eps=0.0)
+        out[name] = prf(*confusion(pred if sel is None else pred[sel], y), eps=0.0)
     stat["baselines"] = out
     log.info("baselines (precision / recall / f1): " +
              "; ".join(f"{k} {p:.4f} / {r:.4f} / {f:.4f}" for k, (p, r, f) in out.items()))
@@ -172,13 +186,17 @@ def write_curves(graph, stat, out_dir, group=None):
     """``roc_curve.csv`` (threshold,fpr,tpr) and ``precision_recall_curve.csv`` (threshold,precision,recall; the final
     (1, 0) point has no threshold) of the test probabilities, thinned as sklearn's ``drop_intermediate=True``: the
     data of the reference's ROC and PR figures (``src/plot.py:103-107,131``).  Floats are written round-trip exact.
-    A graph without labels has no curves: nothing is written."""
+    A graph without labels has no curves: nothing is written.  With ``stat["sel"]`` (``--edge_split``) the curves are
+    those of the selected (test) edges."""
     if graph.y is None:
         return None
-    roc = roc_curve(stat["prob"], graph.y, group)
+    prob, y = stat["prob"], graph.y
+    if stat.get("sel") is not None:
+        prob, y = prob[stat["sel"]], y[stat["sel"]]
+    roc = roc_curve(prob, y, group)
     if roc is None:
         return None
-    return write_curve_files(roc, precision_recall_curve(stat["prob"], graph.y, group, drop_intermediate=True), out_dir)
+    return write_curve_files(roc, precision_recall_curve(prob, y, group, drop_intermediate=True), out_dir)
 
 
 def write_curve_files(roc, pr, out_dir):
@@ -222,9 +240,15 @@ def run(args, device=None):
     ``--train --data_parallel`` in a group, every rank runs ``dist_train.run_data_parallel`` instead.
 
     With input files and ``-r ''`` the graph has no labels: the inference branch writes the groups and the per-edge
-    table (``homolog`` -1), and ``--train`` is refused."""
+    table (``homolog`` -1), and ``--train`` is refused.
+
+    With ``--edge_split VAL TEST`` the whole graph's scored edges are split (``edge_split``): training sees the labels
+    of the train edges alone (loss, ``pos_weight``, train statistics, dynamic threshold), validation and the scheduler
+    the validation edges, and the test statistics and curves are the whole graph's test edges, also in the inference
+    branch.  The groups file and the per-edge table still cover every edge."""
     from . import dist_train
     setup.check_label_flags(args)
+    es.check_flags(args)
     if dist_train.data_parallel(args):
         return dist_train.run_data_parallel(args, device)
     if dist_train.partitioned(args):
@@ -237,12 +261,19 @@ def run(args, device=None):
     threshold = args.binary_threshold
     history = []
     test = [g.to(device) for g in dataset.test]
+    split = test_labels = None
+    if args.edge_split is not None:
+        # the whole graph's test edges are what the test statistics cover, in training and inference alike
+        whole = _whole_graph_of(args, dataset, test, device)
+        split = es.EdgeSplit.build(*whole.edge_index, whole.y, args.seed, args.edge_split)
+        log.info(split.describe())
+        test, test_labels, pos_weight = [whole], [split.labels(whole.y, es.TEST)], split.class_balance
 
     if not args.train or os.path.exists(args.model_args):                             # pangnn.py:125-144
         if os.path.exists(args.model_args):
             log.info(f"Found model file '{args.model_args}' with trained parameters, restoring model state for inference..")
             model.load_state_dict(torch.load(args.model_args, map_location=device))
-        stats = evaluate(model, test, threshold, pos_weight)
+        stats = evaluate(model, test, threshold, pos_weight, labels=test_labels)
         log_test(stats, loss=True)
         if stats:
             add_baselines(dataset, test[0], stats[0])
@@ -255,12 +286,17 @@ def run(args, device=None):
     def loader(graphs, seed):
         return DeviceLoader(graphs, batch_size=args.batch_size, shuffle=True, device=device, seed=seed) if graphs else []
     train_loader, val_loader = loader(dataset.train, args.seed), loader(dataset.val, args.seed + 1)
+    fit, val_labels = {}, None            # --edge_split: forward_loss's train labels, the validation labels
     if args.whole_graph_training:
         # one batch = the whole graph (what the genome-partitioned multi-GPU path and bench.py train on; the
         # reference's per-group sub-graph regime cannot scale past ~1e5 genes, SURVEY F7/F8)
-        whole = test[0] if (args.simulate_dataset and test) else dataset.generate_graphs().to(device)
+        whole = test[0] if split is not None else _whole_graph_of(args, dataset, test, device)
         train_loader, val_loader = [whole], [whole]
         pos_weight = float(dataset.class_balance)                                     # src/dataset.py:346
+        if split is not None:
+            pos_weight = split.class_balance
+            fit = dict(y=split.labels(whole.y, es.TRAIN), num_labelled=split.count(es.TRAIN))
+            val_labels = split.labels(whole.y, es.VAL)
     stepper = None
     if getattr(args, "cuda_graphs", False) and isinstance(train_loader, DeviceLoader):
         # the loop body below as ONE CUDA graph per batch-size bucket; the learning rate lives in device memory so
@@ -280,12 +316,14 @@ def run(args, device=None):
                 labels = stepper.last_y
             else:
                 optimizer.zero_grad()
-                loss, logits = model.forward_loss(batch, pos_weight)                  # criterion(model(batch), labels), fused
+                loss, logits = model.forward_loss(batch, pos_weight, **fit)           # criterion(model(batch), labels), fused
                 loss.backward()
                 optimizer.step()
                 labels = batch.y
             train_loss += loss.item()
             prob = torch.sigmoid(logits)
+            if fit:                                                                   # the train edges alone
+                labels, prob = es.select(fit["y"], prob)
             ep_prob.append(prob.detach())
             ep_y.append(labels.clone() if stepper is not None else labels)   # the stepper's labels are static buffers
             pred = (prob >= threshold).int()
@@ -299,11 +337,14 @@ def run(args, device=None):
         with torch.no_grad():                                                         # pangnn.py:241-275
             for batch in val_loader:
                 logits, prob, pred = model.predict(batch, threshold)
+                y = batch.y
+                if val_labels is not None:                                            # the validation edges alone
+                    y, logits, prob, pred = es.select(val_labels, logits, prob, pred)
                 val_prob.append(prob)
-                val_y.append(batch.y)
+                val_y.append(y)
                 val_loss += float(torch.nn.functional.binary_cross_entropy_with_logits(
-                    logits, batch.y, pos_weight=torch.as_tensor(pos_weight, device=logits.device)))
-                cmv = [a + b for a, b in zip(cmv, confusion(pred, batch.y))]
+                    logits, y, pos_weight=torch.as_tensor(pos_weight, device=logits.device)))
+                cmv = [a + b for a, b in zip(cmv, confusion(pred, y))]
         p, r, f1 = prf(*cm)
         pv, rv, f1v = prf(*cmv)
         mean_val = val_loss / max(len(val_loader), 1)
@@ -314,12 +355,19 @@ def run(args, device=None):
                             f1_train=f1, f1_val=f1v, precision_val=pv, recall_val=rv,
                             auroc_train=rk_tr["auroc"], ap_train=rk_tr["average_precision"],
                             auroc_val=rk_val["auroc"], ap_val=rk_val["average_precision"]))
+        if val_labels is not None:                            # --edge_split: the validation edges' (tn, fp, fn, tp)
+            history[-1]["val_confusion"] = tuple(cmv)
         log.info(f"epoch {epoch}: train loss {history[-1]['train_loss']:.4f} f1 {f1:.4f} | val loss {mean_val:.4f} f1 {f1v:.4f}")
         log.info(f"epoch {epoch}: train auroc {_fmt(rk_tr['auroc'])} ap {_fmt(rk_tr['average_precision'])} | "
                  f"val auroc {_fmt(rk_val['auroc'])} ap {_fmt(rk_val['average_precision'])}")
 
-    stats, path = save_test_and_write(args, model, dataset, test, threshold, pos_weight)
+    stats, path = save_test_and_write(args, model, dataset, test, threshold, pos_weight, labels=test_labels)
     return dict(model=model, dataset=dataset, history=history, test=stats, model_path=path)
+
+
+def _whole_graph_of(args, dataset, test, device):
+    """The whole graph on the device: the simulated dataset's test graph, else ``generate_graphs()`` of the files."""
+    return test[0] if (args.simulate_dataset and test) else dataset.generate_graphs().to(device)
 
 
 def build_dataset_and_model(args, device):
@@ -338,16 +386,16 @@ def build_dataset_and_model(args, device):
     return dataset, model
 
 
-def save_test_and_write(args, model, dataset, test, threshold, pos_weight, write=True, group=None):
+def save_test_and_write(args, model, dataset, test, threshold, pos_weight, write=True, group=None, labels=None):
     """The end of a training run: save ``model.pkl``, test, and write the test outputs.  ``write=False`` (every rank
-    of a data-parallel run but the first) tests without saving or writing; ``group`` as in ``evaluate``.
-    -> (test stats, model path)."""
+    of a data-parallel run but the first) tests without saving or writing; ``group`` and ``labels`` as in
+    ``evaluate``.  -> (test stats, model path)."""
     path = os.path.join(args.output, os.path.basename(args.model_args))
     if write:
         os.makedirs(args.output, exist_ok=True)
         torch.save(model.state_dict(), path)                                          # pangnn.py:339-341
         log.info(f"Saved model parameters to '{path}'")
-    stats = evaluate(model, test, threshold, pos_weight, group)                       # pangnn.py:344-346
+    stats = evaluate(model, test, threshold, pos_weight, group, labels)               # pangnn.py:344-346
     log_test(stats)
     if stats:
         add_baselines(dataset, test[0], stats[0])
