@@ -48,11 +48,12 @@ edge_pair_score_kernel(const float *__restrict__ h, int64_t ldh, int32_t feat,
 }
 
 // ---- backward of the cosine / dot decoders (src/gnn.py:202-207 under autograd, pangnn.py:207) -------------
-// With c_e the forward value, na = max(|h_s|, eps), nb = max(|h_d|, eps):
-//   d/dh_s = dz_e (h_d / (na nb) - c_e h_s / na^2),   d/dh_d = dz_e (h_s / (na nb) - c_e h_d / nb^2)
+// With c_e the forward value, na = max(|h_s|, eps), nb = max(|h_d|, eps), and the norm differentiated as torch's
+// F.cosine_similarity does (clamped value, unclamped derivative h / |h|; 0 for an all-zero row):
+//   d/dh_s = dz_e (h_d / (na nb) - c_e h_s / (na |h_s|)),   d/dh_d = dz_e (h_s / (na nb) - c_e h_d / (nb |h_d|))
 // so the node gradient is TWO weighted aggregations over the scored-edge graph plus a diagonal term,
 //   dh = A_src(alpha) h + A_dst(alpha) h - diag(beta) h,   alpha_e = dz_e / (na nb),
-//   beta_n = sum_{e: src = n} dz_e c_e / na^2 + sum_{e: dst = n} dz_e c_e / nb^2
+//   beta_n = sum_{e: src = n} dz_e c_e / (na |h_s|) + sum_{e: dst = n} dz_e c_e / (nb |h_d|)
 // (dot: alpha_e = dz_e, beta = 0) — no per-edge [E, F] gradient rows are ever materialised; the aggregations
 // run on the streaming gather kernel of the convolutions (gcn.cu), the reduction order is the CSR order.
 __global__ void __launch_bounds__(256)
@@ -64,7 +65,7 @@ row_norm_kernel(const float *__restrict__ h, int64_t ldh, int32_t feat, int32_t 
     float s = 0.f;
     for (int f = lane; f < feat; f += 32) s = fmaf(a[f], a[f], s);
     s = warp_sum(s);
-    if (lane == 0) nrm[r] = fmaxf(sqrtf(s), 1e-8f);
+    if (lane == 0) nrm[r] = sqrtf(s);                    // unclamped: the eps clamp is applied by the user
 }
 
 // warp per CSR row r: val[p] = alpha of slot p, diag[r] (+)= the row's beta sum (fixed lane-strided order)
@@ -76,14 +77,16 @@ pair_coef_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__
     const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (r >= N) return;
     const int64_t b = rowptr[r], e = rowptr[r + 1];
-    const float nr = mode == 0 ? nrm[r] : 1.f;
+    const float eps = 1e-8f;
+    const float rr = mode == 0 ? nrm[r] : 1.f;           // |h_r|
+    const float nr = fmaxf(rr, eps);
     float beta = 0.f;
     for (int64_t p = b + lane; p < e; p += 32) {
         const uint32_t ed = perm[p];
         const float g = dz[ed];
         if (mode == 0) {
-            val[p] = g / (nr * nrm[col[p]]);
-            beta += g * out[ed] / (nr * nr);
+            val[p] = g / (nr * fmaxf(nrm[col[p]], eps));
+            if (rr > 0.f) beta += g * out[ed] / (nr * rr);
         } else {
             val[p] = g;
         }

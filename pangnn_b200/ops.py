@@ -804,10 +804,12 @@ class EdgePairScoreFn(torch.autograd.Function):
             if ctx.mode == 1:
                 ga, gb = g * b, g * a
             else:
-                na = a.norm(dim=1, keepdim=True).clamp_min(1e-8)
-                nb = b.norm(dim=1, keepdim=True).clamp_min(1e-8)
+                # F.cosine_similarity: clamped norms, whose derivative is taken unclamped (h / |h|, 0 at h = 0)
+                ra, rb = a.norm(dim=1, keepdim=True), b.norm(dim=1, keepdim=True)
+                na, nb = ra.clamp_min(1e-8), rb.clamp_min(1e-8)
+                ra, rb = torch.where(ra > 0, ra, 1.0), torch.where(rb > 0, rb, 1.0)
                 c = out.unsqueeze(1)
-                ga, gb = g * (b / (na * nb) - c * a / (na * na)), g * (a / (na * nb) - c * b / (nb * nb))
+                ga, gb = g * (b / (na * nb) - c * a / (na * ra)), g * (a / (na * nb) - c * b / (nb * rb))
             return torch.zeros_like(h).index_add_(0, src, ga).index_add_(0, dst, gb), None, None
         dh = torch.empty(N, F, dtype=torch.float32, device=h.device)
         ws = _ws(lib.pangnn_edge_pair_score_bwd_workspace_bytes(gs.num_edges, N, F), h.device)
